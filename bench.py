@@ -4,10 +4,12 @@ part-step images/sec, forward + backward, and fraction of the HBM roofline).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cub|deepfashion|pennaction]
     python bench.py --impl reference ...      # the CPU restatement of the reference path, host cores
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's outputs to DIR/<name>.npy
 
 One "step" = forward + backward of the path (TPS warp of the views, part softmax, masks and
 labels, mask_parts + pooling, unpool + inject, and the backward of all of it) on one batch of
-synthetic inputs.  Prints ONE JSON line on rank 0.
+synthetic inputs.  Prints ONE JSON line on rank 0.  Writes nothing into the source tree (the
+tree may be read-only): no bytecode caches either.
 """
 import argparse
 import json
@@ -82,10 +84,8 @@ def run_reference(args):
     if rank != 0:
         return
     wl = WORKLOADS[args.workload]
-    # --steps / --warmup are honoured as given; one step = one fwd+bwd of a bounded sample (batch 8, ~0.7 s on 16 cores),
-    # so the driver's 20 + 5 take ~20 s; only a request that would run for more than ~4 minutes is cut short
-    steps = max(1, min(args.steps, 300))
-    warm = max(0, min(args.warmup, 50))
+    # one step = one fwd+bwd of a bounded sample (batch 8, ~0.7 s on 16 cores)
+    steps, warm = args.steps, args.warmup
     rate, med, cores, sample = cpu_port_rate(wl, steps, warm)
     line = {
         "impl": "reference", "metric": "part-step images/sec (fwd+bwd)", "value": rate, "unit": "images/s",
@@ -233,9 +233,33 @@ def make_workload_tensors(torch, ups_b200, wl, name, B, dev, rank, seed, tps_bwd
     return t
 
 
-def measure_workload(args, torch, dist, ups_b200, name, B, dev, rank, world, reducer, steps, warmup, detailed):
+DUMP_BYTES = 60_000_000    # --dump-outputs: data budget of all arrays together, under 64 MB with the .npy headers
+
+
+def dump_outputs(out_dir, outputs):
+    """Write the arrays of `outputs` (name -> tensor) as out_dir/<name>.npy: float32, or float64 for integer arrays
+    (the labels).  An array with more elements than its share of DUMP_BYTES is written as a 1-D sample of its flat
+    entries, at positions drawn by a generator seeded with 0: they depend on the array's size only, so two runs or
+    two builds sample the same entries."""
+    import numpy as np
+    import torch
+    arrays = {k: v for k, v in outputs.items() if v is not None}
+    cap = DUMP_BYTES // (8 * max(1, len(arrays)))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in sorted(arrays.items()):
+        if t.numel() > cap:
+            idx = np.unique(np.random.default_rng(0).integers(0, t.numel(), size=cap))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        a = t.cpu().numpy()
+        a = a.astype(np.float64 if np.issubdtype(a.dtype, np.integer) else np.float32)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def measure_workload(args, torch, dist, ups_b200, name, B, dev, rank, world, reducer, steps, warmup, detailed,
+                     dump_dir=None):
     """K timed steps of the data-parallel part step on workload `name` with inputs resident in HBM.
-    Returns (record, dp, tensors); `detailed` adds per-call CUDA events and the launch count."""
+    Returns (record, dp, tensors); `detailed` adds per-call CUDA events and the launch count.  `dump_dir`: rank 0
+    writes what forward and backward returned in the last timed step there (dump_outputs)."""
     from ups_b200 import _cabi as C
     from ups_b200.dp import DataParallelPartStep
     wl = dict(WORKLOADS[name])
@@ -248,10 +272,12 @@ def measure_workload(args, torch, dist, ups_b200, name, B, dev, rank, world, red
                               decode_bwd=args.decode_bwd, reducer=reducer)
     step = dp.step
     t = make_workload_tensors(torch, ups_b200, wl, name, B, dev, rank, args.seed, args.tps_bwd)
+    last = {}    # what the last step's forward and backward returned (views of the step's output buffers)
 
     def one_step():
-        dp.forward(t["views"], t["coord"], t["tv"], t["l0"], t["l1"], t["feat"])
-        dp.backward(t["g_inj"], t["g_parts"], t["g_pooled"], t["g_m0"], t["g_m1"], t["g_warped"], g_recon=t["g_recon"])
+        last.update(dp.forward(t["views"], t["coord"], t["tv"], t["l0"], t["l1"], t["feat"]))
+        last.update(dp.backward(t["g_inj"], t["g_parts"], t["g_pooled"], t["g_m0"], t["g_m1"], t["g_warped"],
+                                g_recon=t["g_recon"]))
 
     def barrier():
         if world > 1:
@@ -292,6 +318,8 @@ def measure_workload(args, torch, dist, ups_b200, name, B, dev, rank, world, red
     C.call = raw_call
     launches = C.launch_count()
     clocks = sampler.stop() if sampler else None
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, last)
     ms = t0.elapsed_time(t1)
     if world > 1:
         tt = torch.tensor([ms], device=dev)
@@ -354,7 +382,7 @@ def run_gpu(args):
                              n_ctas=args.allreduce_ctas or default_allreduce_ctas(world))
     warm = max(args.warmup, 3)
     rec, dp, t = measure_workload(args, torch, dist, ups_b200, args.workload, B, dev, rank, world, reducer, args.steps, warm,
-                                  detailed=True)
+                                  detailed=True, dump_dir=args.dump_outputs)
     step = dp.step
     line = {
         "metric": "part-step images/sec (fwd+bwd)", "value": rec["value"], "unit": "images/s", "n_gpus": world,
@@ -549,6 +577,7 @@ def main():
     # stdout carries exactly one JSON line: everything else that writes to file descriptor 1 (NCCL prints its
     # version banner there when the box sets NCCL_DEBUG) is sent to stderr; the line goes out through the saved descriptor
     global _JSON_OUT
+    sys.dont_write_bytecode = True      # the modules imported from here on leave no __pycache__ in the tree
     sys.stdout.flush()
     _JSON_OUT = os.fdopen(os.dup(1), "w")
     os.dup2(2, 1)
@@ -575,7 +604,15 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-n4", action="store_true", help="skip the N4 first-convolution microbenchmark leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what forward and backward returned in the last one as DIR/<name>.npy "
+                         "(float32; integer outputs as float64; arrays too large for 64 MB in all as a fixed seeded "
+                         "sample of their entries; rank 0's shard when N>1)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

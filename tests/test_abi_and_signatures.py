@@ -232,6 +232,6 @@ def test_bench_reference_arm_prints_one_json_line():
     lines = [ln for ln in r.stdout.splitlines() if ln.strip()]
     assert len(lines) == 1, r.stdout[:2000]
     d = json.loads(lines[0])
-    assert d["impl"] == "reference" and d["unit"] == "images/s" and d["value"] > 0
+    assert d["impl"] == "reference" and d["unit"] == "images/s" and d["value"] > 0 and d["steps"] == 1
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0

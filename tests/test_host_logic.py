@@ -110,3 +110,32 @@ def test_bench_knows_the_bytes_of_every_call_of_the_fused_step(ups):
     for n in ("ups_step_warp_decode_fwd_rows", "ups_step_encode_fwd_rows", "ups_step_decode_bwd_tc_rows", "ups_step_encode_bwd_rows"):
         traffic, source = bench.ncu_traffic(n, "cub", 256)
         assert traffic and traffic > 0.9 * bench.call_bytes(n, 16, 64, 3, 256, 16384) * 0.5 and source, n
+
+
+def test_bench_dump_outputs_fits_64_mb_and_samples_the_same_entries(tmp_path):
+    """bench.py --dump-outputs: small arrays are written whole, integer ones as float64; arrays too large for 64 MB in
+    all are written as a 1-D sample taken at the same positions on every call, so two runs compare entry for entry."""
+    import importlib.util
+    import os
+
+    import numpy as np
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    spec = importlib.util.spec_from_file_location("bench_under_test", os.path.join(root, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    g = torch.Generator().manual_seed(0)
+    base = torch.arange(16_000_000, dtype=torch.float32)          # 64 MB: each entry holds its own flat position
+    out = {f"big{i}": base for i in range(12)}
+    out.update(small=torch.randn(4, 5, generator=g), labels=torch.randint(0, 16, (2, 8, 8), generator=g), absent=None)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), out)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == sorted([f"big{i}.npy" for i in range(12)] + ["labels.npy", "small.npy"])
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 64_000_000
+    load = lambda d, n: np.load(tmp_path / d / f"{n}.npy")  # noqa: E731
+    assert load("a", "small").dtype == np.float32 and np.array_equal(load("a", "small"), out["small"].numpy())
+    assert load("a", "labels").dtype == np.float64 and np.array_equal(load("a", "labels"), out["labels"].numpy())
+    s = load("a", "big0")
+    assert s.dtype == np.float32 and s.ndim == 1 and 0 < s.size < base.numel()
+    assert np.all(np.diff(s) > 0) and s[-1] < base.numel()                  # distinct positions, in order
+    assert np.array_equal(s, load("b", "big0")) and np.array_equal(s, load("a", "big11"))
