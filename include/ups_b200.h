@@ -343,6 +343,35 @@ int ups_step_warp_decode_fwd_rows(const float* U, const float* U2, const float* 
                                   int N, int N2, int S, const float* l0, int l0_row, const float* feat, float* m0,
                                   long long* labels0, float* inj, int B, int K, int F, void* stream);
 
+/* ---- the mean-field logit noise drawn on the device (MeanFieldDistribution.sample, cub/code/nn.py:1421-1427) ----
+ * The training step samples its logits as l = mean + noise_level * N(0,1) (model.py:420-421).  The N(0,1) draw here is a
+ * pure function of (seed, draw, global pixel, part), defined in csrc/canon_math.cuh: Philox4x32-10 with key = seed and
+ * counter = (global pixel lo, hi, part / 4, draw), 24-bit uniforms in (0, 1], Box-Muller with the canonical log / sin /
+ * cos.  It does not depend on K, the launch geometry or the batch split.  draw = 0 for l0, 1 for l1; global pixel =
+ * (sample_offset + b) * P + p.  The sampled logit is fl(mean + fl(noise_level * z)); -inf (a padded part) stays -inf. */
+/* eps [n_pix, K] for global pixels pix_offset .. pix_offset + n_pix - 1: what the kernels below draw. */
+int ups_normal_philox_fwd(unsigned long long seed, int draw, long long pix_offset, long long n_pix, int K, float* out,
+                          void* stream);
+/* ups_part_softmax_sampled_fwd with eps drawn in registers (pixel i of `mean` is global pixel pix_offset + i);
+ * logits_out, labels and hard may be NULL. */
+int ups_part_softmax_sampled_philox_fwd(const float* mean, unsigned long long seed, int draw, long long pix_offset,
+                                        float noise_level, float* logits_out, float* probs, int64_t* labels, float* hard,
+                                        long long n_pix, int K, void* stream);
+/* The fused forward kernels on means: the arguments of the _rows forms, then (seed, sample_offset, noise_level).  l0 / l1
+ * are the means; the noise is added right after the load (decode side draw 0, encode side draw 1).  The sampled logits
+ * are not written: ups_normal_philox_fwd + ups_mean_field_sample_fwd regenerate them bit for bit.  The backward entry
+ * points are unchanged: d l / d mean is the identity, so dl0 / dl1 are the gradients of the means. */
+int ups_step_decode_fwd_noise(const float* l0, int l0_row, const float* feat, float* m0, long long* labels0, float* inj,
+                              int B, int P, int K, int F, unsigned long long seed, long long sample_offset, float noise_level,
+                              void* stream);
+int ups_step_encode_fwd_noise(const float* l1, int l1_row, const float* img1, float* m1, float* parts_pm, float* pooled,
+                              int B, int P, int K, int Kpl, void* ws, size_t ws_bytes, unsigned long long seed,
+                              long long sample_offset, float noise_level, void* stream);
+int ups_step_warp_decode_fwd_noise(const float* U, const float* U2, const float* coord, const float* T, float* out,
+                                   float* out2, int N, int N2, int S, const float* l0, int l0_row, const float* feat, float* m0,
+                                   long long* labels0, float* inj, int B, int K, int F, unsigned long long seed,
+                                   long long sample_offset, float noise_level, void* stream);
+
 /* K1 + K3 of the fused step in ONE launch (csrc/step_fwd_fused.cu): the TPS warp of the views (ups_tps_warp_pair_fwd's
  * arguments: U [N,S,S,3], optional second image set U2 [N2,S,S,3] sharing the first N2 warps, coord, T -> out, out2) and
  * the decode-side forward (ups_step_decode_fwd's arguments) are independent (model.py:282-311 vs :426-447,482-484);

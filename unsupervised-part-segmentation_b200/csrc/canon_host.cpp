@@ -9,6 +9,30 @@ extern "C" {
 void ups_host_exp(const float* x, float* y, long long n) { for (long long i = 0; i < n; ++i) y[i] = ups::exp_canon(x[i]); }
 void ups_host_log(const float* x, float* y, long long n) { for (long long i = 0; i < n; ++i) y[i] = ups::log_canon(x[i]); }
 
+// the mean-field logit noise (canon_math.cuh::normal4_philox)
+void ups_host_philox(const uint32_t* ctr, const uint32_t* key, uint32_t* out, long long n) {
+    for (long long i = 0; i < n; ++i) {
+        uint32_t c[4] = {ctr[4 * i], ctr[4 * i + 1], ctr[4 * i + 2], ctr[4 * i + 3]};
+        ups::philox4x32_10(c[0], c[1], c[2], c[3], key[2 * i], key[2 * i + 1]);
+        for (int j = 0; j < 4; ++j) out[4 * i + j] = c[j];
+    }
+}
+void ups_host_box_muller(const uint32_t* xa, const uint32_t* xb, float* za, float* zb, long long n) {
+    for (long long i = 0; i < n; ++i) ups::box_muller_canon(xa[i], xb[i], za[i], zb[i]);
+}
+void ups_host_sincos2pi(const float* u, float* s, float* c, long long n) {
+    for (long long i = 0; i < n; ++i) ups::sincos2pi_canon(u[i], s[i], c[i]);
+}
+// eps [n_pix, K] for global pixels pix_offset .. pix_offset + n_pix - 1 (ups_normal_philox_fwd on the host)
+void ups_host_normal_philox(unsigned long long seed, int draw, long long pix_offset, long long n_pix, int K, float* out) {
+    for (long long i = 0; i < n_pix; ++i)
+        for (int j = 0; 4 * j < K; ++j) {
+            float z[4];
+            ups::normal4_philox(seed, (uint32_t)draw, (unsigned long long)(pix_offset + i), (uint32_t)j, z[0], z[1], z[2], z[3]);
+            for (int l = 0; l < 4 && 4 * j + l < K; ++l) out[i * K + 4 * j + l] = z[l];
+        }
+}
+
 void ups_host_softmax(const float* x, float* p, long long* labels, float* hard, long long n_pix, int K) {
     std::vector<float> e(ups::KMAX * 2);
     for (long long i = 0; i < n_pix; ++i) {

@@ -26,6 +26,8 @@
 #define UPS_DDIV(a, b) __ddiv_rn((a), (b))
 #define UPS_F2I(x) __float_as_int(x)
 #define UPS_I2F(x) __int_as_float(x)
+#define UPS_FSQRT(a) __fsqrt_rn(a)
+#define UPS_UMULHI(a, b) __umulhi((a), (b))
 #else
 #define UPS_FMUL(a, b) ((a) * (b))
 #define UPS_FADD(a, b) ((a) + (b))
@@ -39,6 +41,8 @@ static inline int ups_f2i_host(float x) { int i; memcpy(&i, &x, 4); return i; }
 static inline float ups_i2f_host(int i) { float x; memcpy(&x, &i, 4); return x; }
 #define UPS_F2I(x) ups_f2i_host(x)
 #define UPS_I2F(x) ups_i2f_host(x)
+#define UPS_FSQRT(a) sqrtf(a)
+#define UPS_UMULHI(a, b) ((uint32_t)(((uint64_t)(a) * (uint64_t)(b)) >> 32))
 #include <math.h>
 #endif
 
@@ -245,5 +249,78 @@ UPS_HD float softmax_row_canon(const float* x, float* p, float* e, int K) {
     for (int k = 0; k < K; ++k) { p[k] = UPS_FMUL(p[k], rs); pmax = p[k] > pmax ? p[k] : pmax; }
     return pmax;
 }
+
+// ---------------------------------------------------------------- the mean-field logit noise (oracle/noise.py::normal_philox)
+// MeanFieldDistribution.sample (cub/code/nn.py:1421-1427) draws l = mean + noise_level * N(0,1).  The draw here is a pure
+// function of (seed, draw, global pixel, part), so a kernel can generate it in registers wherever it reads the mean:
+//   x[0..3] = Philox4x32-10(counter = (gpix lo, gpix hi, k / 4, draw), key = (seed lo, seed hi))
+//             gpix = (sample_offset + b) * P + p;  draw = 0 for l0, 1 for l1
+//   u(x)    = ((x >> 8) + 1) * 2^-24                       in (0, 1], exact in fp32
+//   parts 4j, 4j+1 from (x0, x1), parts 4j+2, 4j+3 from (x2, x3), Box-Muller on (u_a, u_b):
+//   r = sqrt(-2 * log_canon(u_a));  z = r * cos_canon(2 pi u_b),  r * sin_canon(2 pi u_b)      |z| <= 5.77, finite
+//   sampled logit = fl(mean + fl(noise_level * z))  (-inf + finite = -inf: padded parts stay -inf)
+// The value does not depend on K, the launch geometry or the batch split.
+constexpr uint32_t PHILOX_M0 = 0xD2511F53u, PHILOX_M1 = 0xCD9E8D57u;
+constexpr uint32_t PHILOX_W0 = 0x9E3779B9u, PHILOX_W1 = 0xBB67AE85u;
+
+// Philox4x32-10 (Salmon et al., SC'11; the Random123 constants): c <- philox(c, key)
+UPS_HD void philox4x32_10(uint32_t& c0, uint32_t& c1, uint32_t& c2, uint32_t& c3, uint32_t k0, uint32_t k1) {
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        const uint32_t hi0 = UPS_UMULHI(PHILOX_M0, c0), lo0 = PHILOX_M0 * c0;
+        const uint32_t hi1 = UPS_UMULHI(PHILOX_M1, c2), lo1 = PHILOX_M1 * c2;
+        c0 = hi1 ^ c1 ^ k0; c1 = lo1; c2 = hi0 ^ c3 ^ k1; c3 = lo0;
+        k0 += PHILOX_W0; k1 += PHILOX_W1;
+    }
+}
+
+// (0, 1]: the top 24 bits of x plus one, times 2^-24 (integer -> float is exact below 2^24 + 1)
+UPS_HD float uniform24(uint32_t x) { return UPS_FMUL((float)((x >> 8) + 1u), 5.9604644775390625e-8f); }
+
+// sin and cos of 2 pi u for u in [0, 1], canonical order.  t = 4u and its fraction f are exact; f > 1/2 is folded to
+// 1 - f (exact) so that the polynomial argument x = fl(g * pi/2) lies in [0, pi/4]; Cephes sinf / cosf polynomials,
+// every operation rounded separately; the quadrant floor(t) mod 4 picks signs and the sin/cos swap.
+UPS_HD void sincos2pi_canon(float u, float& s_out, float& c_out) {
+    const float t = UPS_FMUL(u, 4.0f);
+    const float q = floorf(t);
+    const float f = UPS_FSUB(t, q);
+    const bool fold = f > 0.5f;
+    const float g = fold ? UPS_FSUB(1.0f, f) : f;
+    const float x = UPS_FMUL(g, 1.57079632679489662f);
+    const float z = UPS_FMUL(x, x);
+    float sn = UPS_FADD(UPS_FMUL(-1.9515295891e-4f, z), 8.3321608736e-3f);
+    sn = UPS_FADD(UPS_FMUL(sn, z), -1.6666654611e-1f);
+    sn = UPS_FMUL(UPS_FMUL(sn, z), x);
+    sn = UPS_FADD(sn, x);
+    float cs = UPS_FADD(UPS_FMUL(2.443315711809948e-5f, z), -1.388731625493765e-3f);
+    cs = UPS_FADD(UPS_FMUL(cs, z), 4.166664568298827e-2f);
+    cs = UPS_FMUL(UPS_FMUL(cs, z), z);
+    cs = UPS_FSUB(cs, UPS_FMUL(0.5f, z));
+    cs = UPS_FADD(cs, 1.0f);
+    const float s = fold ? cs : sn, c = fold ? sn : cs;   // sin, cos of (pi/2) f
+    const int quad = ((int)q) & 3;
+    s_out = quad == 0 ? s : quad == 1 ? c : quad == 2 ? -s : -c;
+    c_out = quad == 0 ? c : quad == 1 ? -s : quad == 2 ? -c : s;
+}
+
+// two N(0,1) values from one pair of Philox words: (r cos, r sin)
+UPS_HD void box_muller_canon(uint32_t xa, uint32_t xb, float& za, float& zb) {
+    const float r = UPS_FSQRT(UPS_FMUL(-2.0f, log_canon(uniform24(xa))));
+    float s, c;
+    sincos2pi_canon(uniform24(xb), s, c);
+    za = UPS_FMUL(r, c);
+    zb = UPS_FMUL(r, s);
+}
+
+// the normals of parts 4j .. 4j+3 of global pixel `gpix`
+UPS_HD void normal4_philox(unsigned long long seed, uint32_t draw, unsigned long long gpix, uint32_t j, float& z0,
+                           float& z1, float& z2, float& z3) {
+    uint32_t c0 = (uint32_t)gpix, c1 = (uint32_t)(gpix >> 32), c2 = j, c3 = draw;
+    philox4x32_10(c0, c1, c2, c3, (uint32_t)seed, (uint32_t)(seed >> 32));
+    box_muller_canon(c0, c1, z0, z1);
+    box_muller_canon(c2, c3, z2, z3);
+}
+
+UPS_HD float sampled_logit(float mean, float noise_level, float z) { return UPS_FADD(mean, UPS_FMUL(noise_level, z)); }
 
 }  // namespace ups

@@ -56,6 +56,14 @@ inline void prefer_max_shared_carveout(Kern kern) {
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 inline long long cdiv(long long a, long long b) { return (a + b - 1) / b; }
 
+// the mean-field logit noise of one side of the step (canon_math.cuh::normal4_philox)
+struct NoiseArgs {
+    unsigned long long seed;
+    long long sample_offset;   // global index of the launch's first sample
+    float level;
+    int draw;                  // 0: l0, 1: l1
+};
+
 #if defined(__CUDACC__)
 __device__ __forceinline__ float4 ld4(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
 // streaming variants: read-once inputs / write-once outputs should not displace reusable lines
@@ -77,6 +85,15 @@ __device__ __forceinline__ float4 ld_row4(const float* __restrict__ base, size_t
     v.z = k0 + 2 < row ? __ldcs(p + 2) : pad;
     v.w = k0 + 3 < row ? __ldcs(p + 3) : pad;
     return v;
+}
+
+// parts 4c .. 4c+3 of pixel p of sample b (of P pixels) sampled in registers: v + noise_level * z
+__device__ __forceinline__ float4 add_noise4(float4 v, const NoiseArgs& n, int b, int P, int p, int c) {
+    const unsigned long long g = (unsigned long long)(n.sample_offset + b) * (unsigned long long)P + (unsigned)p;
+    float z0, z1, z2, z3;
+    normal4_philox(n.seed, (uint32_t)n.draw, g, (uint32_t)c, z0, z1, z2, z3);
+    return make_float4(sampled_logit(v.x, n.level, z0), sampled_logit(v.y, n.level, z1), sampled_logit(v.z, n.level, z2),
+                       sampled_logit(v.w, n.level, z3));
 }
 
 template <int W>

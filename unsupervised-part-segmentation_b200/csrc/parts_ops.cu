@@ -9,14 +9,17 @@ constexpr int TPB = 256;
 
 // =================================================================== softmax over parts
 // Fast path: K = 4*LPP, LPP lanes per pixel, one float4 per lane, fully coalesced.
-// SAMPLED: logits = mean + noise*eps first (MeanFieldDistribution.sample, cub/code/nn.py:1421-1427), one rounding per step.
-template <int LPP, int UNROLL, bool SAMPLED>
+// MODE: SM_PLAIN softmax(logits); SM_EPS logits = mean + noise*eps first (MeanFieldDistribution.sample,
+// cub/code/nn.py:1421-1427), one rounding per step; SM_PHILOX the same with eps drawn in registers (canon_math.cuh, the
+// mean-field logit noise; pixel i is global pixel nz.sample_offset + i).
+constexpr int SM_PLAIN = 0, SM_EPS = 1, SM_PHILOX = 2;
+template <int LPP, int UNROLL, int MODE>
 __global__ void __launch_bounds__(TPB) part_softmax_fwd_kernel(const float* __restrict__ logits,
                                                                const float* __restrict__ eps, float noise,
                                                                float* __restrict__ logits_out,
                                                                float* __restrict__ probs,
                                                                long long* __restrict__ labels,
-                                                               float* __restrict__ hard, long long n4) {
+                                                               float* __restrict__ hard, long long n4, NoiseArgs nz) {
     // n4 = n_pix * LPP float4s in total; every lane stays alive for the shuffles
     const long long base = ((long long)blockIdx.x * UNROLL) * TPB + threadIdx.x;
     float4 v[UNROLL];
@@ -25,12 +28,19 @@ __global__ void __launch_bounds__(TPB) part_softmax_fwd_kernel(const float* __re
         const long long i = base + (long long)u * TPB;
         const long long ii = i < n4 ? i : n4 - 1;
         v[u] = ld4_stream(logits + 4 * ii);
-        if (SAMPLED) {
+        if (MODE == SM_EPS) {
             const float4 e = ld4_stream(eps + 4 * ii);
             v[u] = make_float4(__fadd_rn(v[u].x, __fmul_rn(noise, e.x)), __fadd_rn(v[u].y, __fmul_rn(noise, e.y)),
                                __fadd_rn(v[u].z, __fmul_rn(noise, e.z)), __fadd_rn(v[u].w, __fmul_rn(noise, e.w)));
-            if (logits_out && i < n4) st4(logits_out + 4 * i, v[u]);
         }
+        if (MODE == SM_PHILOX) {
+            float z0, z1, z2, z3;
+            normal4_philox(nz.seed, (uint32_t)nz.draw, (unsigned long long)(nz.sample_offset + ii / LPP),
+                           (uint32_t)(ii & (LPP - 1)), z0, z1, z2, z3);
+            v[u] = make_float4(sampled_logit(v[u].x, nz.level, z0), sampled_logit(v[u].y, nz.level, z1),
+                               sampled_logit(v[u].z, nz.level, z2), sampled_logit(v[u].w, nz.level, z3));
+        }
+        if (MODE != SM_PLAIN && logits_out && i < n4) st4(logits_out + 4 * i, v[u]);
     }
 #pragma unroll
     for (int u = 0; u < UNROLL; ++u) {
@@ -46,23 +56,35 @@ __global__ void __launch_bounds__(TPB) part_softmax_fwd_kernel(const float* __re
     }
 }
 
-// Generic K (e.g. the reference's shipped n_parts = 25): one thread per pixel.
+// Generic K (e.g. the reference's shipped n_parts = 25): one thread per pixel.  MODE as part_softmax_fwd_kernel's
+// (SM_PLAIN and SM_EPS share one instantiation: the eps mode is the run-time `eps != nullptr`).
+template <int MODE>
 __global__ void __launch_bounds__(128) part_softmax_fwd_generic_kernel(const float* __restrict__ logits,
                                                                        const float* __restrict__ eps, float noise,
                                                                        float* __restrict__ logits_out,
                                                                        float* __restrict__ probs,
                                                                        long long* __restrict__ labels,
                                                                        float* __restrict__ hard, long long n_pix,
-                                                                       int K) {
+                                                                       int K, NoiseArgs nz) {
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_pix) return;
     float x[KMAX], p[KMAX], e[KMAX];
     for (int k = 0; k < K; ++k) x[k] = logits[i * K + k];
-    if (eps) {
+    if (MODE != SM_PHILOX && eps) {
         for (int k = 0; k < K; ++k) {
             x[k] = __fadd_rn(x[k], __fmul_rn(noise, eps[i * K + k]));
             if (logits_out) logits_out[i * K + k] = x[k];
         }
+    }
+    if (MODE == SM_PHILOX) {
+        for (int j = 0; 4 * j < K; ++j) {
+            float z[4];
+            normal4_philox(nz.seed, (uint32_t)nz.draw, (unsigned long long)(nz.sample_offset + i), (uint32_t)j, z[0], z[1],
+                           z[2], z[3]);
+            for (int l = 0; l < 4 && 4 * j + l < K; ++l) x[4 * j + l] = sampled_logit(x[4 * j + l], nz.level, z[l]);
+        }
+        if (logits_out)
+            for (int k = 0; k < K; ++k) logits_out[i * K + k] = x[k];
     }
     const float pmax = softmax_row_canon(x, p, e, K);
     int arg = -1;
@@ -105,6 +127,22 @@ __global__ void part_softmax_bwd_generic_kernel(const float* __restrict__ probs,
     float dot = 0.f;
     for (int k = 0; k < K; ++k) dot += probs[i * K + k] * gsum(i * K + k);
     for (int k = 0; k < K; ++k) dlogits[i * K + k] = probs[i * K + k] * (gsum(i * K + k) - dot);
+}
+
+// eps [n_pix, K] of global pixels pix_offset + i: one thread per (pixel, group of 4 parts)
+__global__ void __launch_bounds__(TPB) normal_philox_kernel(float* __restrict__ out, long long n, int J, int K, NoiseArgs nz) {
+    const long long t = (long long)blockIdx.x * TPB + threadIdx.x;   // over n_pix * J
+    if (t >= n) return;
+    const long long i = t / J;
+    const int j = (int)(t - i * J);
+    float z[4];
+    normal4_philox(nz.seed, (uint32_t)nz.draw, (unsigned long long)(nz.sample_offset + i), (uint32_t)j, z[0], z[1], z[2], z[3]);
+    float* o = out + i * K + 4 * j;
+    if (4 * j + 4 <= K && (K & 3) == 0) {
+        st4_stream(o, make_float4(z[0], z[1], z[2], z[3]));
+    } else {
+        for (int l = 0; l < 4 && 4 * j + l < K; ++l) __stcs(o + l, z[l]);
+    }
 }
 
 // y += a*x  and  out[v] = g[v] (or 0) + (v == idx ? extra : 0): the two elementwise sums of the unfused step
@@ -402,9 +440,10 @@ using namespace ups;
 static inline unsigned nblk(long long n, int tpb) { return (unsigned)cdiv(n, tpb); }
 #define UPS_GRID_OK(n, tpb) UPS_REQUIRE(cdiv((n), (tpb)) < (1ll << 31), "problem too large for one launch")
 
+// nz != nullptr: the philox mode (eps == nullptr); eps != nullptr: the eps mode; neither: plain softmax
 static int part_softmax_fwd_impl(const char* what, const float* logits, const float* eps, float noise,
                                  float* logits_out, float* probs, long long* labels, float* hard_st, long long n_pix,
-                                 int K, void* stream) {
+                                 int K, void* stream, const NoiseArgs* nz = nullptr) {
     UPS_REQUIRE(logits && probs, "%s: null pointer", what);
     UPS_REQUIRE(n_pix >= 0 && K >= 1 && K <= KMAX, "%s: n_pix=%lld K=%d (1..%d)", what, n_pix, K, KMAX);
     if (n_pix == 0) return UPS_OK;
@@ -416,12 +455,16 @@ static int part_softmax_fwd_impl(const char* what, const float* logits, const fl
     {                                                                                                                \
         const long long n4 = n_pix * LPP;                                                                            \
         UPS_GRID_OK(n4, TPB * U);                                                                                    \
-        if (eps)                                                                                                     \
-            part_softmax_fwd_kernel<LPP, U, true><<<nblk(n4, TPB * U), TPB, 0, s>>>(logits, eps, noise, logits_out,  \
-                                                                                    probs, labels, hard_st, n4);     \
+        if (nz)                                                                                                      \
+            part_softmax_fwd_kernel<LPP, U, SM_PHILOX><<<nblk(n4, TPB * U), TPB, 0, s>>>(                            \
+                logits, nullptr, 0.f, logits_out, probs, labels, hard_st, n4, *nz);                                  \
+        else if (eps)                                                                                                \
+            part_softmax_fwd_kernel<LPP, U, SM_EPS><<<nblk(n4, TPB * U), TPB, 0, s>>>(logits, eps, noise, logits_out, \
+                                                                                      probs, labels, hard_st, n4,    \
+                                                                                      NoiseArgs{});                  \
         else                                                                                                         \
-            part_softmax_fwd_kernel<LPP, U, false><<<nblk(n4, TPB * U), TPB, 0, s>>>(logits, nullptr, 0.f, nullptr,  \
-                                                                                     probs, labels, hard_st, n4);    \
+            part_softmax_fwd_kernel<LPP, U, SM_PLAIN><<<nblk(n4, TPB * U), TPB, 0, s>>>(                             \
+                logits, nullptr, 0.f, nullptr, probs, labels, hard_st, n4, NoiseArgs{});                             \
         return after_launch("part_softmax_fwd_kernel");                                                              \
     }
     if (vec && K == 4) UPS_SM_FWD(1)
@@ -430,8 +473,12 @@ static int part_softmax_fwd_impl(const char* what, const float* logits, const fl
     if (vec && K == 32) UPS_SM_FWD(8)
 #undef UPS_SM_FWD
     UPS_GRID_OK(n_pix, 128);
-    part_softmax_fwd_generic_kernel<<<nblk(n_pix, 128), 128, 0, s>>>(logits, eps, noise, logits_out, probs, labels,
-                                                                     hard_st, n_pix, K);
+    if (nz)
+        part_softmax_fwd_generic_kernel<SM_PHILOX><<<nblk(n_pix, 128), 128, 0, s>>>(logits, nullptr, 0.f, logits_out, probs,
+                                                                                labels, hard_st, n_pix, K, *nz);
+    else
+        part_softmax_fwd_generic_kernel<SM_PLAIN><<<nblk(n_pix, 128), 128, 0, s>>>(logits, eps, noise, logits_out, probs,
+                                                                               labels, hard_st, n_pix, K, NoiseArgs{});
     return after_launch("part_softmax_fwd_generic_kernel");
 }
 
@@ -447,6 +494,29 @@ extern "C" int ups_part_softmax_sampled_fwd(const float* mean, const float* eps,
     UPS_REQUIRE(eps, "part_softmax_sampled_fwd: null pointer");
     return part_softmax_fwd_impl("part_softmax_sampled_fwd", mean, eps, noise_level, logits_out, probs,
                                  reinterpret_cast<long long*>(labels), hard_st, n_pix, K, stream);
+}
+
+extern "C" int ups_part_softmax_sampled_philox_fwd(const float* mean, unsigned long long seed, int draw, long long pix_offset,
+                                                   float noise_level, float* logits_out, float* probs, int64_t* labels,
+                                                   float* hard_st, long long n_pix, int K, void* stream) {
+    UPS_REQUIRE(draw >= 0 && pix_offset >= 0, "part_softmax_sampled_philox_fwd: draw=%d pix_offset=%lld", draw, pix_offset);
+    const NoiseArgs nz{seed, pix_offset, noise_level, draw};
+    return part_softmax_fwd_impl("part_softmax_sampled_philox_fwd", mean, nullptr, 0.f, logits_out, probs,
+                                 reinterpret_cast<long long*>(labels), hard_st, n_pix, K, stream, &nz);
+}
+
+extern "C" int ups_normal_philox_fwd(unsigned long long seed, int draw, long long pix_offset, long long n_pix, int K, float* out,
+                                     void* stream) {
+    UPS_REQUIRE(out, "normal_philox_fwd: null pointer");
+    UPS_REQUIRE(n_pix >= 0 && K >= 1 && draw >= 0 && pix_offset >= 0, "normal_philox_fwd: n_pix=%lld K=%d draw=%d pix_offset=%lld",
+                n_pix, K, draw, pix_offset);
+    UPS_REQUIRE((K & 3) != 0 || aligned16(out), "normal_philox_fwd: 16-byte alignment");
+    if (n_pix == 0) return UPS_OK;
+    const int J = (K + 3) / 4;
+    const long long n = n_pix * J;
+    UPS_GRID_OK(n, TPB);
+    normal_philox_kernel<<<nblk(n, TPB), TPB, 0, as_stream(stream)>>>(out, n, J, K, NoiseArgs{seed, pix_offset, 1.0f, draw});
+    return after_launch("normal_philox_kernel");
 }
 
 extern "C" int ups_part_softmax_bwd(const float* probs, const float* g, float* dlogits, long long n_pix, int K,

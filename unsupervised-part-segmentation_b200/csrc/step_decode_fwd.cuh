@@ -38,11 +38,13 @@ __device__ __noinline__ void inject_rows_general(float4 mh, const float4* fs4, f
 
 // FT = compile-time F (0: run-time F) so that the row/column split of the inject store is shifts.
 // (split, b): the CTA's pixel range of sample b; fs4: K*F floats of shared memory (feat[b] as [K][F/4] float4)
-template <int LPP, int FT>
+// NOISE: l0 holds the means and the logits are sampled in registers right after the load (canon_math.cuh, the mean-field
+// logit noise); the noise-free instantiation is the plain kernel.
+template <int LPP, int FT, bool NOISE = false>
 __device__ __forceinline__ void step_decode_fwd_body(const float* __restrict__ l0, const float* __restrict__ feat,
                                                      float* __restrict__ m0, long long* __restrict__ labels0,
                                                      float* __restrict__ inj, int P, int Frt, int pix_per_cta, int split,
-                                                     int b, float4* fs4, int l0_row) {
+                                                     int b, float4* fs4, int l0_row, const NoiseArgs& nz = NoiseArgs{}) {
     // l0_row: row length of l0 in floats (K, or the real part count when the logits of a padded K are read in place)
     constexpr int K = 4 * LPP, PW = 32 / LPP;
     const int F = FT > 0 ? FT : Frt;
@@ -58,6 +60,10 @@ __device__ __forceinline__ void step_decode_fwd_body(const float* __restrict__ l
 #pragma unroll
         for (int s = 0; s < LPP; ++s)
             v[s] = ld_row4<LPP>(l0, (size_t)b * P + pg + s * PW + plq, c, l0_row, -INFINITY);
+        if (NOISE) {
+#pragma unroll
+            for (int s = 0; s < LPP; ++s) v[s] = add_noise4(v[s], nz, b, P, pg + s * PW + plq, c);
+        }
 #pragma unroll
         for (int s = 0; s < LPP; ++s) {
             const size_t pix = (size_t)b * P + pg + s * PW + plq;

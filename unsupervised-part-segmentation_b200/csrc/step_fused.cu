@@ -30,15 +30,16 @@ template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N)); }
 
 // ============================================================================ K3 decode fwd (body: step_decode_fwd.cuh)
-template <int LPP, int FT>
+template <int LPP, int FT, bool NOISE>
 __global__ void __launch_bounds__(FTPB) step_decode_fwd_kernel(const float* __restrict__ l0,
                                                                const float* __restrict__ feat,
                                                                float* __restrict__ m0,
                                                                long long* __restrict__ labels0,
                                                                float* __restrict__ inj, int P, int Frt,
-                                                               int pix_per_cta, int l0_row) {
+                                                               int pix_per_cta, int l0_row, NoiseArgs nz) {
     extern __shared__ float4 fs4[];  // feat[b] as [K][F/4] float4
-    step_decode_fwd_body<LPP, FT>(l0, feat, m0, labels0, inj, P, Frt, pix_per_cta, blockIdx.x, blockIdx.y, fs4, l0_row);
+    step_decode_fwd_body<LPP, FT, NOISE>(l0, feat, m0, labels0, inj, P, Frt, pix_per_cta, blockIdx.x, blockIdx.y, fs4, l0_row,
+                                         nz);
 }
 
 // ============================================================================ K2 encode fwd
@@ -53,12 +54,13 @@ struct EncFwdSmem {
 };
 
 // MINB: resident CTAs per SM asked of ptxas (an explicit value also keeps the exp chains interleaved)
-template <int LPP, int MINB, bool PAD>
+// NOISE: l1 holds the means, sampled in registers right after the load (canon_math.cuh, the mean-field logit noise)
+template <int LPP, int MINB, bool PAD, bool NOISE>
 __global__ void __launch_bounds__(FTPB, MINB) step_encode_fwd_kernel(const float* __restrict__ l1,
                                                                const float* __restrict__ img1,
                                                                float* __restrict__ m1, float* __restrict__ parts,
                                                                float* __restrict__ partial, int B, int P,
-                                                               int pix_per_cta, int Kpl, int l1_row) {
+                                                               int pix_per_cta, int Kpl, int l1_row, NoiseArgs nz) {
     // Kpl <= K: number of part planes that exist in `parts` (planes Kpl..K-1 are padding of a K that is not a power
     // of two: their mask is identically zero and they are neither written nor allocated)
     using L = EncFwdSmem<LPP>;
@@ -81,6 +83,10 @@ __global__ void __launch_bounds__(FTPB, MINB) step_encode_fwd_kernel(const float
 #pragma unroll
         for (int s = 0; s < LPP; ++s)
             v[s] = ld_row4<LPP>(l1, (size_t)b * P + pg + s * PW + plq, c, l1_row, -INFINITY);
+        if (NOISE) {
+#pragma unroll
+            for (int s = 0; s < LPP; ++s) v[s] = add_noise4(v[s], nz, b, P, pg + s * PW + plq, c);
+        }
         if (lane < 24) st4(Iw + 4 * lane, ld4(img1 + ((size_t)b * P + pg) * 3 + 4 * lane));
 #pragma unroll
         for (int s = 0; s < LPP; ++s) {
@@ -410,8 +416,9 @@ extern "C" int ups_step_decode_fwd(const float* l0, const float* feat, float* m0
     return ups_step_decode_fwd_rows(l0, K, feat, m0, labels0, inj, B, P, K, F, stream);
 }
 
-extern "C" int ups_step_decode_fwd_rows(const float* l0, int l0_row, const float* feat, float* m0, long long* labels0,
-                                        float* inj, int B, int P, int K, int F, void* stream) {
+template <bool NOISE>
+static int decode_fwd_launch(const float* l0, int l0_row, const float* feat, float* m0, long long* labels0, float* inj, int B,
+                             int P, int K, int F, NoiseArgs nz, void* stream) {
     UPS_REQUIRE(l0 && feat && m0 && labels0 && inj, "step_decode_fwd: null pointer");
     UPS_REQUIRE(l0_row >= 1 && l0_row <= K, "step_decode_fwd: l0 rows of %d floats for K=%d", l0_row, K);
     if (int rc = fused_common_checks("step_decode_fwd", B, P, K)) return rc;
@@ -428,8 +435,8 @@ extern "C" int ups_step_decode_fwd_rows(const float* l0, int l0_row, const float
     cudaStream_t s = as_stream(stream);
 #define UPS_DEC_FWD2(LPP, FT)                                                                           \
     {                                                                                                   \
-        if (int rc = set_smem(step_decode_fwd_kernel<LPP, FT>, sm)) return rc;                          \
-        step_decode_fwd_kernel<LPP, FT><<<grid, FTPB, sm, s>>>(l0, feat, m0, labels0, inj, P, F, per, l0_row); \
+        if (int rc = set_smem(step_decode_fwd_kernel<LPP, FT, NOISE>, sm)) return rc;                   \
+        step_decode_fwd_kernel<LPP, FT, NOISE><<<grid, FTPB, sm, s>>>(l0, feat, m0, labels0, inj, P, F, per, l0_row, nz); \
     }
 #define UPS_DEC_FWD(LPP) \
     { if (F == 64) UPS_DEC_FWD2(LPP, 64) else if (F == 32) UPS_DEC_FWD2(LPP, 32) else if (F == 16) UPS_DEC_FWD2(LPP, 16) else UPS_DEC_FWD2(LPP, 0) }
@@ -437,6 +444,19 @@ extern "C" int ups_step_decode_fwd_rows(const float* l0, int l0_row, const float
 #undef UPS_DEC_FWD2
 #undef UPS_DEC_FWD
     return after_launch("step_decode_fwd_kernel");
+}
+
+extern "C" int ups_step_decode_fwd_rows(const float* l0, int l0_row, const float* feat, float* m0, long long* labels0,
+                                        float* inj, int B, int P, int K, int F, void* stream) {
+    return decode_fwd_launch<false>(l0, l0_row, feat, m0, labels0, inj, B, P, K, F, NoiseArgs{}, stream);
+}
+
+extern "C" int ups_step_decode_fwd_noise(const float* l0, int l0_row, const float* feat, float* m0, long long* labels0,
+                                         float* inj, int B, int P, int K, int F, unsigned long long seed, long long sample_offset,
+                                         float noise_level, void* stream) {
+    UPS_REQUIRE(sample_offset >= 0, "step_decode_fwd: sample_offset=%lld", sample_offset);
+    return decode_fwd_launch<true>(l0, l0_row, feat, m0, labels0, inj, B, P, K, F, NoiseArgs{seed, sample_offset, noise_level, 0},
+                                   stream);
 }
 
 extern "C" int ups_step_encode_fwd(const float* l1, const float* img1, float* m1, float* parts_pm, float* pooled,
@@ -449,9 +469,9 @@ extern "C" int ups_step_encode_fwd_planes(const float* l1, const float* img1, fl
     return ups_step_encode_fwd_rows(l1, K, img1, m1, parts_pm, pooled, B, P, K, Kpl, ws, ws_bytes, stream);
 }
 
-extern "C" int ups_step_encode_fwd_rows(const float* l1, int l1_row, const float* img1, float* m1, float* parts_pm,
-                                        float* pooled, int B, int P, int K, int Kpl, void* ws, size_t ws_bytes,
-                                        void* stream) {
+template <bool NOISE>
+static int encode_fwd_launch(const float* l1, int l1_row, const float* img1, float* m1, float* parts_pm, float* pooled, int B,
+                             int P, int K, int Kpl, void* ws, size_t ws_bytes, NoiseArgs nz, void* stream) {
     UPS_REQUIRE(l1 && img1 && m1 && parts_pm && pooled, "step_encode_fwd: null pointer");
     UPS_REQUIRE(l1_row >= 1 && l1_row <= K, "step_encode_fwd: l1 rows of %d floats for K=%d", l1_row, K);
     UPS_REQUIRE(Kpl >= 1 && Kpl <= K, "step_encode_fwd: %d part planes of K=%d", Kpl, K);
@@ -470,11 +490,11 @@ extern "C" int ups_step_encode_fwd_rows(const float* l1, int l1_row, const float
     {                                                                                                         \
         const size_t sm = (size_t)FW * EncFwdSmem<LPP>::WREG * sizeof(float);                                 \
         if (Kpl < K) {                                                                                        \
-            if (int rc = set_smem(step_encode_fwd_kernel<LPP, MB, true>, sm)) return rc;                      \
-            step_encode_fwd_kernel<LPP, MB, true><<<grid, FTPB, sm, s>>>(l1, img1, m1, parts_pm, partial, B, P, per, Kpl, l1_row); \
+            if (int rc = set_smem(step_encode_fwd_kernel<LPP, MB, true, NOISE>, sm)) return rc;               \
+            step_encode_fwd_kernel<LPP, MB, true, NOISE><<<grid, FTPB, sm, s>>>(l1, img1, m1, parts_pm, partial, B, P, per, Kpl, l1_row, nz); \
         } else {                                                                                              \
-            if (int rc = set_smem(step_encode_fwd_kernel<LPP, MB, false>, sm)) return rc;                     \
-            step_encode_fwd_kernel<LPP, MB, false><<<grid, FTPB, sm, s>>>(l1, img1, m1, parts_pm, partial, B, P, per, Kpl, l1_row); \
+            if (int rc = set_smem(step_encode_fwd_kernel<LPP, MB, false, NOISE>, sm)) return rc;              \
+            step_encode_fwd_kernel<LPP, MB, false, NOISE><<<grid, FTPB, sm, s>>>(l1, img1, m1, parts_pm, partial, B, P, per, Kpl, l1_row, nz); \
         }                                                                                                     \
     }
 #define UPS_ENC_FWD(LPP) \
@@ -486,6 +506,20 @@ extern "C" int ups_step_encode_fwd_rows(const float* l1, int l1_row, const float
     const long long n = (long long)B * K * 3;
     split_finalize_kernel<<<(unsigned)cdiv(n, 128), 128, 0, s>>>(partial, pooled, K * 3, splits, P, n);
     return after_launch("split_finalize_kernel");
+}
+
+extern "C" int ups_step_encode_fwd_rows(const float* l1, int l1_row, const float* img1, float* m1, float* parts_pm,
+                                        float* pooled, int B, int P, int K, int Kpl, void* ws, size_t ws_bytes,
+                                        void* stream) {
+    return encode_fwd_launch<false>(l1, l1_row, img1, m1, parts_pm, pooled, B, P, K, Kpl, ws, ws_bytes, NoiseArgs{}, stream);
+}
+
+extern "C" int ups_step_encode_fwd_noise(const float* l1, int l1_row, const float* img1, float* m1, float* parts_pm,
+                                         float* pooled, int B, int P, int K, int Kpl, void* ws, size_t ws_bytes,
+                                         unsigned long long seed, long long sample_offset, float noise_level, void* stream) {
+    UPS_REQUIRE(sample_offset >= 0, "step_encode_fwd: sample_offset=%lld", sample_offset);
+    return encode_fwd_launch<true>(l1, l1_row, img1, m1, parts_pm, pooled, B, P, K, Kpl, ws, ws_bytes,
+                                   NoiseArgs{seed, sample_offset, noise_level, 1}, stream);
 }
 
 extern "C" int ups_step_decode_bwd(const float* g_inj, const float* m0, const float* g_m0, const float* feat,

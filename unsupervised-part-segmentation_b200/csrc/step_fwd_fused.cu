@@ -21,11 +21,12 @@ struct WarpArgs {
 struct DecodeArgs {
     const float* l0; const float* feat; float* m0; long long* labels0; float* inj;
     int P, F, pix_per_cta, splits, l0_row;
+    NoiseArgs nz;      // NOISE instantiations only: l0 holds the means
 };
 
 static_assert(WARP_TPB == FTPB, "both roles use 128-thread CTAs");
 
-template <int LPP, int FT, int MINB>
+template <int LPP, int FT, int MINB, bool NOISE>
 __global__ void __launch_bounds__(FTPB, MINB) step_warp_decode_fwd_kernel(const WarpArgs wa, const DecodeArgs da, unsigned n3,
                                                                          unsigned total) {
     extern __shared__ float4 dyn4[];   // decode role: K*F floats; warp role: 2*128*3 staged pixels + 42 constants
@@ -34,7 +35,8 @@ __global__ void __launch_bounds__(FTPB, MINB) step_warp_decode_fwd_kernel(const 
     const unsigned c3n = (unsigned)(((unsigned long long)(i + 1) * n3) / total);
     if (c3n > c3) {
         const int b = (int)(c3 / (unsigned)da.splits), split = (int)(c3 - (unsigned)b * da.splits);
-        step_decode_fwd_body<LPP, FT>(da.l0, da.feat, da.m0, da.labels0, da.inj, da.P, da.F, da.pix_per_cta, split, b, dyn4, da.l0_row);
+        step_decode_fwd_body<LPP, FT, NOISE>(da.l0, da.feat, da.m0, da.labels0, da.inj, da.P, da.F, da.pix_per_cta, split, b, dyn4,
+                                             da.l0_row, da.nz);
     } else {
         const unsigned j = i - c3;
         const int b = (int)(j / (unsigned)wa.tiles_per_sample), tile = (int)(j - (unsigned)b * wa.tiles_per_sample);
@@ -56,9 +58,10 @@ extern "C" int ups_step_warp_decode_fwd(const float* U, const float* U2, const f
     return ups_step_warp_decode_fwd_rows(U, U2, coord, T, out, out2, N, N2, S, l0, K, feat, m0, labels0, inj, B, K, F, stream);
 }
 
-extern "C" int ups_step_warp_decode_fwd_rows(const float* U, const float* U2, const float* coord, const float* T, float* out,
-                                             float* out2, int N, int N2, int S, const float* l0, int l0_row, const float* feat,
-                                             float* m0, long long* labels0, float* inj, int B, int K, int F, void* stream) {
+template <bool NOISE>
+static int warp_decode_fwd_launch(const float* U, const float* U2, const float* coord, const float* T, float* out, float* out2,
+                                  int N, int N2, int S, const float* l0, int l0_row, const float* feat, float* m0,
+                                  long long* labels0, float* inj, int B, int K, int F, NoiseArgs nz, void* stream) {
     UPS_REQUIRE(l0_row >= 1 && l0_row <= K, "step_warp_decode_fwd: l0 rows of %d floats for K=%d", l0_row, K);
     UPS_REQUIRE(U && coord && T && out && l0 && feat && m0 && labels0 && inj, "step_warp_decode_fwd: null pointer");
     UPS_REQUIRE((U2 == nullptr) == (out2 == nullptr), "step_warp_decode_fwd: U2 and out2 must be given together");
@@ -71,7 +74,7 @@ extern "C" int ups_step_warp_decode_fwd_rows(const float* U, const float* U2, co
     UPS_REQUIRE((l0_row < K || aligned16(l0)) && aligned16(feat) && aligned16(m0) && aligned16(inj), "step_warp_decode_fwd: 16-byte alignment");
     WarpArgs wa{U, U2, coord, T, out, out2, N2, S, S, S, S, (int)cdiv((long long)P, WARP_TPB * WARP_PPT)};
     const int per = fused_pix_per_cta(B, P);
-    DecodeArgs da{l0, feat, m0, labels0, inj, P, F, per, (int)cdiv(P, per), l0_row};
+    DecodeArgs da{l0, feat, m0, labels0, inj, P, F, per, (int)cdiv(P, per), l0_row, nz};
     const unsigned long long n1 = (unsigned long long)N * wa.tiles_per_sample, n3 = (unsigned long long)B * da.splits;
     UPS_REQUIRE(n1 + n3 < (1ull << 31), "step_warp_decode_fwd: grid too large");
     const unsigned total = (unsigned)(n1 + n3);
@@ -83,9 +86,9 @@ extern "C" int ups_step_warp_decode_fwd_rows(const float* U, const float* U2, co
 #define UPS_WD3(LPP, FT, MB)                                                                                    \
     {                                                                                                           \
         if (sm > 48 * 1024)                                                                                     \
-            UPS_CUDA(cudaFuncSetAttribute(step_warp_decode_fwd_kernel<LPP, FT, MB>,                             \
+            UPS_CUDA(cudaFuncSetAttribute(step_warp_decode_fwd_kernel<LPP, FT, MB, NOISE>,                      \
                                           cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));               \
-        step_warp_decode_fwd_kernel<LPP, FT, MB><<<total, FTPB, sm, s>>>(wa, da, (unsigned)n3, total);          \
+        step_warp_decode_fwd_kernel<LPP, FT, MB, NOISE><<<total, FTPB, sm, s>>>(wa, da, (unsigned)n3, total);   \
     }
 #define UPS_WD2(LPP, FT) { if (minb == 5) UPS_WD3(LPP, FT, 5) else if (minb == 6) UPS_WD3(LPP, FT, 6) else UPS_WD3(LPP, FT, 4) }
 #define UPS_WD(LPP) { if (F == 64) UPS_WD2(LPP, 64) else if (F == 32) UPS_WD2(LPP, 32) else UPS_WD2(LPP, 16) }
@@ -94,4 +97,21 @@ extern "C" int ups_step_warp_decode_fwd_rows(const float* U, const float* U2, co
 #undef UPS_WD2
 #undef UPS_WD3
     return after_launch("step_warp_decode_fwd_kernel");
+}
+
+extern "C" int ups_step_warp_decode_fwd_rows(const float* U, const float* U2, const float* coord, const float* T, float* out,
+                                             float* out2, int N, int N2, int S, const float* l0, int l0_row, const float* feat,
+                                             float* m0, long long* labels0, float* inj, int B, int K, int F, void* stream) {
+    return warp_decode_fwd_launch<false>(U, U2, coord, T, out, out2, N, N2, S, l0, l0_row, feat, m0, labels0, inj, B, K, F,
+                                         NoiseArgs{}, stream);
+}
+
+extern "C" int ups_step_warp_decode_fwd_noise(const float* U, const float* U2, const float* coord, const float* T, float* out,
+                                              float* out2, int N, int N2, int S, const float* l0, int l0_row, const float* feat,
+                                              float* m0, long long* labels0, float* inj, int B, int K, int F,
+                                              unsigned long long seed, long long sample_offset, float noise_level,
+                                              void* stream) {
+    UPS_REQUIRE(sample_offset >= 0, "step_warp_decode_fwd: sample_offset=%lld", sample_offset);
+    return warp_decode_fwd_launch<true>(U, U2, coord, T, out, out2, N, N2, S, l0, l0_row, feat, m0, labels0, inj, B, K, F,
+                                        NoiseArgs{seed, sample_offset, noise_level, 0}, stream);
 }

@@ -304,8 +304,10 @@ class DataParallelPartStep:
         # experiment knob: UPS_DP_SPLIT=<ctas>: first half of the main bucket before K4, second half after K4 with <ctas> CTAs
         self.split_ctas = int(os.environ.get("UPS_DP_SPLIT", "0"))
         self.main_split = self.split_ctas > 0
+        # rank r holds samples [r*B, (r+1)*B) of the global batch: with the same noise seed on every rank, the N ranks draw
+        # exactly the logit noise that one GPU draws over the global batch (PartStep.forward(noise_seed=...))
         self.step = PartStep(per_gpu_batch, spatial_size, n_parts, local_app_size, n_views, use_tps, views_grad, device,
-                             decode_bwd=decode_bwd)
+                             decode_bwd=decode_bwd, sample_offset=self.rank * int(per_gpu_batch))
         dev = self.step.device
         K, F = self.step.K, self.step.F
         self.mod = StandInModules(K, F, dev, seed)
@@ -329,7 +331,8 @@ class DataParallelPartStep:
         self._ev = torch.cuda.Event()
 
     # ---------------------------------------------------------------- forward
-    def forward(self, views, coord, t_vector, l0, l1, feat, conv_V=None, conv_b=None):
+    def forward(self, views, coord, t_vector, l0, l1, feat, conv_V=None, conv_b=None, noise_seed=None, noise_level=1.0):
+        """PartStep.forward on this rank's shard; pass the same noise_seed on every rank."""
         # the parameters (hence the averaged gradients of the previous step) are needed from the first kernel that consumes
         # logits or features; the 11x11 TPS solves in front of it depend on the batch's warp parameters only
         inner = self.step._inner if self.step.Kp else self.step
@@ -337,7 +340,8 @@ class DataParallelPartStep:
             inner.before_params = self.reducer.wait
         else:
             self.reducer.wait()
-        return self.step.forward(views, coord, t_vector, l0, l1, feat, conv_V, conv_b)
+        return self.step.forward(views, coord, t_vector, l0, l1, feat, conv_V, conv_b, noise_seed=noise_seed,
+                                 noise_level=noise_level)
 
     def wait_grads(self):
         """The current stream waits until both buckets hold the mean over ranks (times 1/grad_scale for NCCL)."""

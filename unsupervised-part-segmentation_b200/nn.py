@@ -125,8 +125,13 @@ def edge_set(x, alpha, lambda_):
 
 
 class MeanFieldDistribution(object):
-    """cub/code/nn.py:1395-1457 — the distribution object on the part logits (model.py:413-421).  `sample` takes the
-    N(0,1) draw as an optional argument (a seeded torch.Generator otherwise): TF's RNG stream is not reproducible."""
+    """cub/code/nn.py:1395-1457 — the distribution object on the part logits (model.py:413-421).  TF's RNG stream is not
+    reproducible; `sample` takes its N(0,1) draw from one of three sources:
+      eps=...       the caller's tensor;
+      seed=...      the project's counter-based draw (csrc/canon_math.cuh), generated on the device: a pure function of
+                    (seed, draw, global pixel, part), so it regenerates bit for bit what PartStep.forward(noise_seed=seed)
+                    drew inside the step (draw 0 for l0, 1 for l1; sample_offset = global index of sample 0);
+      neither       torch.randn with `generator`."""
 
     def __init__(self, parameters, dim, stochastic=True):
         self.parameters = parameters
@@ -144,19 +149,30 @@ class MeanFieldDistribution(object):
     def n_parameters(dim):
         return dim
 
-    def sample(self, noise_level=1.0, eps=None, generator=None):
+    def _philox_args(self, seed, draw, sample_offset):
+        assert self.mean.dim() == 4
+        B, H, W, K = self.shape
+        return ops._seed_i64(seed), int(draw), int(sample_offset) * H * W, B * H * W, K
+
+    def sample(self, noise_level=1.0, eps=None, generator=None, seed=None, draw=0, sample_offset=0):
         if not self.stochastic:
             return self.mean
+        if eps is None and seed is not None:
+            s, d, off, n, K = self._philox_args(seed, draw, sample_offset)
+            eps = ops.normal_philox(s, d, off, n, K, self.mean.device).view(self.shape)
         if eps is None:
             eps = torch.randn(self.shape, generator=generator, device=self.mean.device, dtype=torch.float32)
         return ops.mean_field_sample(self.mean, eps, float(noise_level))
 
-    def sample_softmax(self, noise_level=1.0, eps=None, generator=None):
+    def sample_softmax(self, noise_level=1.0, eps=None, generator=None, seed=None, draw=0, sample_offset=0):
         """softmax(sample()) in one pass (cub/code/SB_model48i/model.py:420-430): -> (logits, probs, labels, hard)
-        with hard = straight_through_estimator(hard_max(probs, 3), probs)."""
+        with hard = straight_through_estimator(hard_max(probs, 3), probs).  With `seed` the draw is made in registers."""
         if not self.stochastic:
             probs, labels, hard = ops.part_softmax_full(self.mean)
             return self.mean, probs, labels, hard
+        if eps is None and seed is not None:
+            s, d, off, _, _ = self._philox_args(seed, draw, sample_offset)
+            return ops.part_softmax_sampled_philox(self.mean, s, d, off, float(noise_level))
         if eps is None:
             eps = torch.randn(self.shape, generator=generator, device=self.mean.device, dtype=torch.float32)
         return ops.part_softmax_sampled(self.mean, eps, float(noise_level))

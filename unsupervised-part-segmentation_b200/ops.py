@@ -665,6 +665,51 @@ part_softmax_sampled = _op(
     _pss_bwd, lambda ctx, inputs, output: ctx.save_for_backward(output[1]))
 
 
+# ------------------------------------------------------------------ the logit noise drawn on the device
+# The draw is a pure function of (seed, draw, global pixel, part) (csrc/canon_math.cuh): ups_normal_philox_fwd writes it,
+# ups_part_softmax_sampled_philox_fwd and the step's `_noise` kernels generate the same values in registers.  Seeds are
+# unsigned 64-bit; the op schemas carry them as the int64 with the same bits.
+def _seed_i64(seed: int) -> int:
+    seed = int(seed)
+    if not 0 <= seed < 2 ** 64:
+        raise ValueError(f"seed must be in [0, 2**64), got {seed}")
+    return seed - 2 ** 64 if seed >= 2 ** 63 else seed
+
+
+def _normal_philox(seed: int, draw: int, pix_offset: int, n_pix: int, K: int, device: torch.device) -> Tensor:
+    out = torch.empty(n_pix, K, dtype=torch.float32, device=device)
+    if not out.is_cuda:
+        raise C.UpsError("ups_b200: normal_philox needs a CUDA device (no CPU fallback exists)")
+    C.call("ups_normal_philox_fwd", seed % 2 ** 64, draw, pix_offset, n_pix, K, out.data_ptr(), _stream(out))
+    return out
+
+
+normal_philox = _op("normal_philox", _normal_philox,
+                    lambda seed, draw, off, n, K, device: torch.empty(n, K, dtype=torch.float32, device=device))
+
+
+def _part_softmax_sampled_philox(mean: Tensor, seed: int, draw: int, pix_offset: int,
+                                 noise_level: float) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+    mean = _f32(mean, "mean")
+    K = mean.shape[-1]
+    logits, probs, hard = torch.empty_like(mean), torch.empty_like(mean), torch.empty_like(mean)
+    labels = torch.empty(mean.shape[:-1], dtype=torch.int64, device=mean.device)
+    C.call("ups_part_softmax_sampled_philox_fwd", mean.data_ptr(), seed % 2 ** 64, draw, pix_offset, noise_level,
+           logits.data_ptr(), probs.data_ptr(), labels.data_ptr(), hard.data_ptr(), mean.numel() // K, K, _stream(mean))
+    return logits, probs, labels, hard
+
+
+def _pssp_bwd(ctx, g_logits, g_probs, g_labels, g_hard):
+    return _pss_bwd(ctx, g_logits, g_probs, g_labels, g_hard)[0], None, None, None, None
+
+
+part_softmax_sampled_philox = _op(
+    "part_softmax_sampled_philox", _part_softmax_sampled_philox,
+    lambda m, s, d, o, n: (torch.empty_like(m), torch.empty_like(m), m.new_empty(m.shape[:-1], dtype=torch.int64),
+                           torch.empty_like(m)),
+    _pssp_bwd, lambda ctx, inputs, output: ctx.save_for_backward(output[1]))
+
+
 def _weak_xent(logits: Tensor, mode: int) -> Tensor:
     x = _f32(logits, "logits")
     K = x.shape[-1]

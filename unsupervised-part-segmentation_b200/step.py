@@ -13,6 +13,10 @@ What the reference builds per training step in TrainModel.define_graph
     [h0             = conv2d(inj, V) + b   (first layer of `dd`)        model.py:96,485 ; nn.py:617-664
                       with first_conv=Co: computed from m0h and feat directly, `inj` is never formed (SURVEY 8f N4)]
 
+With a noise seed, l0 and l1 are the means of MeanFieldDistribution and the step samples them itself
+(model.py:420-421, cub/code/nn.py:1421-1427): m0, m1 = softmax(l0 + noise_level*eps0), softmax(l1 + noise_level*eps1)
+with eps drawn in registers from (seed, side, global pixel, part) (csrc/canon_math.cuh, ups_normal_philox_fwd).
+
 The CNNs between those pieces are not part of the path: `l0`, `l1` (mask decoder output) and
 `feat` (appearance encoder output) are inputs, and the cotangents of every output are inputs
 to `backward`.  All buffers are allocated once in __init__ (180 GB HBM: the B=256 CUB step
@@ -23,6 +27,17 @@ import os
 import torch
 
 from . import _cabi as C
+
+
+def _call_rows(name, noise, *args):
+    """Call the `_rows` entry point `name`, or, with noise = (seed, sample_offset, noise_level), its `_noise` form: the same
+    kernel reading l0 / l1 as means and adding the draw in registers (the same bytes; arguments of the `_rows` form, then
+    the three noise arguments, then the stream)."""
+    if noise is None:
+        C.call(name, *args)
+    else:
+        assert name.endswith("_rows"), name
+        C.call(name[:-len("_rows")] + "_noise", *args[:-1], *noise, args[-1])
 
 
 def _on_device(fn):
@@ -39,8 +54,13 @@ def _on_device(fn):
 
 class PartStep:
     def __init__(self, batch_size, spatial_size, n_parts, local_app_size=64, n_views=3, use_tps=True,
-                 views_grad=False, device="cuda", decode_bwd="auto", first_conv=0, encoder_conv=0, _planes=None):
+                 views_grad=False, device="cuda", decode_bwd="auto", first_conv=0, encoder_conv=0, sample_offset=0,
+                 _planes=None):
         B, S, K, F, V = int(batch_size), int(spatial_size), int(n_parts), int(local_app_size), int(n_views)
+        # sample_offset: global index of this step's first sample in the noise draw (forward(noise_seed=...)): a rank of a
+        # data-parallel run that holds samples [o, o + B) of the global batch draws exactly what one GPU draws for them
+        self.sample_offset = int(sample_offset)
+        assert self.sample_offset >= 0
         self.B, self.S, self.K, self.F, self.V = B, S, K, F, V
         self.P = S * S
         # _planes (internal): part planes that really exist when this step runs a padded part count (see below)
@@ -63,7 +83,7 @@ class PartStep:
                 and self.P % 32 == 0 and os.environ.get("UPS_PAD_K", "1") != "0"):
             self.Kp = 8 if K <= 8 else 16 if K <= 16 else 32
             self._inner = PartStep(B, S, self.Kp, F, n_views=V, use_tps=use_tps, views_grad=views_grad, device=self.device,
-                                   decode_bwd=decode_bwd, _planes=K)
+                                   decode_bwd=decode_bwd, sample_offset=sample_offset, _planes=K)
             self._init_padded()
             return
         # K4 variant: "tc" = persistent TMA + tcgen05/TMEM pipeline, "simt" = CUDA-core kernel
@@ -132,6 +152,26 @@ class PartStep:
     def _stream(self):
         return torch.cuda.current_stream(self.device).cuda_stream
 
+    def _noise(self, noise_seed, noise_level):
+        """(seed, sample_offset, noise_level) for the `_noise` entry points, or None (the noise-free step)."""
+        if noise_seed is None:
+            return None
+        seed = int(noise_seed)
+        if not 0 <= seed < 2 ** 64:
+            raise ValueError(f"noise_seed must be in [0, 2**64), got {noise_seed}")
+        return (seed, self.sample_offset, float(noise_level))
+
+    def _softmax_fwd(self, logits, draw, probs, labels, hard, nz, st):
+        """ups_part_softmax_fwd on the logits, or with noise nz on the means (the draw of side `draw` made in registers)."""
+        p = lambda t: None if t is None else t.data_ptr()  # noqa: E731
+        n = self.B * self.P
+        if nz is None:
+            C.call("ups_part_softmax_fwd", logits.data_ptr(), probs.data_ptr(), p(labels), p(hard), n, self.K, st)
+        else:
+            seed, offset, level = nz
+            C.call("ups_part_softmax_sampled_philox_fwd", logits.data_ptr(), seed, draw, offset * self.P, level, None,
+                   probs.data_ptr(), p(labels), p(hard), n, self.K, st)
+
     # ------------------------------------------------------------------ padded part count (K -> Kp)
     def _init_padded(self):
         B, S, K, F, Kp = self.B, self.S, self.K, self.F, self.Kp
@@ -180,7 +220,7 @@ class PartStep:
                buf.shape[-1] - n_cols, fill, st)
 
     @_on_device
-    def _forward_padded(self, views, coord, t_vector, l0, l1, feat):
+    def _forward_padded(self, views, coord, t_vector, l0, l1, feat, noise_seed=None, noise_level=1.0):
         B, S, K, F, P, Kp = self.B, self.S, self.K, self.F, self.P, self.Kp
         st = self._stream()
         assert feat.is_contiguous()
@@ -191,7 +231,8 @@ class PartStep:
         a1, n1 = self._arg(l1, self._l1p)
         # feat [B,K,F] -> [B,Kp,F]: per sample the first K*F floats of the padded block (the rest stays zero)
         C.call("ups_copy_rows", feat.data_ptr(), K * F, self._featp.data_ptr(), Kp * F, B, K * F, 0, 0.0, st)
-        o = self._inner.forward(views, coord, t_vector, a0, a1, self._featp, rows=dict(l0=n0, l1=n1))
+        o = self._inner.forward(views, coord, t_vector, a0, a1, self._featp, rows=dict(l0=n0, l1=n1), noise_seed=noise_seed,
+                                noise_level=noise_level)
         self._feat, self._img1 = feat, self._inner._img1
         return dict(warped=o["warped"], m0=self.m0, m1=self.m1, labels0=self.labels0, parts=self.parts, pooled=self.pooled,
                     inj=self.inj)
@@ -218,39 +259,49 @@ class PartStep:
         return out
 
     # ------------------------------------------------------------------ forward
-    def _decode_fwd(self, l0, feat, conv_V, conv_b, st, l0_row=None):
+    def _decode_fwd(self, l0, feat, conv_V, conv_b, st, l0_row=None, nz=None):
         """decode side on stream `st`: K3, or with first_conv softmax -> table -> 3x3 conv on the assignment"""
         B, S, K, F, P = self.B, self.S, self.K, self.F, self.P
         if not self.Co:
-            C.call("ups_step_decode_fwd_rows", l0.data_ptr(), l0_row or K, feat.data_ptr(), self.m0.data_ptr(),
-                   self.labels0.data_ptr(), self.inj.data_ptr(), B, P, K, F, st)
+            _call_rows("ups_step_decode_fwd_rows", nz, l0.data_ptr(), l0_row or K, feat.data_ptr(), self.m0.data_ptr(),
+                       self.labels0.data_ptr(), self.inj.data_ptr(), B, P, K, F, st)
             return
-        C.call("ups_part_softmax_fwd", l0.data_ptr(), self.m0.data_ptr(), self.labels0.data_ptr(),
-               self.mh0c.data_ptr(), B * P, K, st)
+        self._softmax_fwd(l0, 0, self.m0, self.labels0, self.mh0c, nz, st)
         C.call("ups_inject_conv_table_fwd", feat.data_ptr(), conv_V.data_ptr(), self.G.data_ptr(), B, K, F, self.Co, st)
         C.call("ups_inject_conv_fwd", self.mh0c.data_ptr(), self.G.data_ptr(), conv_b.data_ptr(), self.h0.data_ptr(),
                B, S, S, K, self.Co, st)
 
-    def forward(self, views, coord, t_vector, l0, l1, feat, conv_V=None, conv_b=None, enc_V=None, enc_b=None, rows=None):
+    def forward(self, views, coord, t_vector, l0, l1, feat, conv_V=None, conv_b=None, enc_V=None, enc_b=None, rows=None,
+                noise_seed=None, noise_level=1.0):
         """views [V,B,S,S,3] (view0, view1[, view0_target]), fp32 in [-1, 1] or the dataset's uint8
         (normalised on the device exactly as cub/code/data/data.py:134 does on the host); coord,
         t_vector [2B,8,2] from make_input_tps_param; l0, l1 [B,S,S,K]; feat [B,K,F].  Returns a dict
         of views into the step's persistent output buffers.
+
+        noise_seed (an integer in [0, 2**64)): the reference's training step, which samples its logits
+        (MeanFieldDistribution.sample, model.py:420-421): l0 and l1 are the MEANS and the kernels use
+        l = mean + noise_level * eps, eps ~ N(0,1) drawn in registers right after the load (draw 0 for l0, 1 for l1, global
+        pixel (sample_offset + b) * S*S + p; csrc/canon_math.cuh).  No extra pass and no extra launch.  The sampled logits
+        are not written (the reference keeps them as m0_logits / m1_logits): ups_normal_philox_fwd(seed, draw,
+        sample_offset * S*S, B*S*S, K) gives eps bit for bit, and ops.mean_field_sample(mean, eps, noise_level) the logits
+        (nn.MeanFieldDistribution(mean).sample(noise_level, seed=..., draw=..., sample_offset=...) does both).
+        backward is unchanged: d l / d mean is the identity, so dl0 / dl1 are the gradients of the means.
+        noise_seed=None is the noise-free step (l0, l1 are the logits), with the same launches as always.
 
         On the fused path K1 (TPS warp) and K3 (decode side) are independent and run as ONE launch with interleaved
         CTAs (ups_step_warp_decode_fwd): the warp's arithmetic hides under the decode side's memory stream.
         forward_warp / forward_parts are the same step as two calls (K1 | K2, K3) for callers that have the views
         before the logits."""
         if self.Kp:
-            return self._forward_padded(views, coord, t_vector, l0, l1, feat)
+            return self._forward_padded(views, coord, t_vector, l0, l1, feat, noise_seed, noise_level)
         # rows (internal, padded part counts): row lengths of l0 / l1 when they are read in place ({"l0": 25, "l1": 25})
         if self.fuse_fwd:
-            return self._forward_fused(views, coord, t_vector, l0, l1, feat, rows)
+            return self._forward_fused(views, coord, t_vector, l0, l1, feat, rows, self._noise(noise_seed, noise_level))
         self.forward_warp(views, coord, t_vector)
-        return self.forward_parts(l0, l1, feat, conv_V, conv_b, enc_V, enc_b, rows)
+        return self.forward_parts(l0, l1, feat, conv_V, conv_b, enc_V, enc_b, rows, noise_seed, noise_level)
 
     @_on_device
-    def _forward_fused(self, views, coord, t_vector, l0, l1, feat, rows=None):
+    def _forward_fused(self, views, coord, t_vector, l0, l1, feat, rows=None, nz=None):
         B, S, K, F, P, V = self.B, self.S, self.K, self.F, self.P, self.V
         st = self._stream()
         views = self._ingest(views, st)
@@ -261,15 +312,15 @@ class PartStep:
         C.call("ups_tps_solve", coord.data_ptr(), t_vector.data_ptr(), self.T.data_ptr(), 2 * B, st)
         if self.before_params is not None:
             self.before_params()     # data-parallel wrapper: wait for the averaged gradients (the TPS solve needs none)
-        C.call("ups_step_warp_decode_fwd_rows", views.data_ptr(), views[2].data_ptr() if V > 2 else None, coord.data_ptr(),
-               self.T.data_ptr(), self.warped.data_ptr(), self.warped[2].data_ptr() if V > 2 else None, 2 * B,
-               B if V > 2 else 0, S, l0.data_ptr(), r0, feat.data_ptr(), self.m0.data_ptr(), self.labels0.data_ptr(),
-               self.inj.data_ptr(), B, K, F, st)
+        _call_rows("ups_step_warp_decode_fwd_rows", nz, views.data_ptr(), views[2].data_ptr() if V > 2 else None,
+                   coord.data_ptr(), self.T.data_ptr(), self.warped.data_ptr(), self.warped[2].data_ptr() if V > 2 else None,
+                   2 * B, B if V > 2 else 0, S, l0.data_ptr(), r0, feat.data_ptr(), self.m0.data_ptr(),
+                   self.labels0.data_ptr(), self.inj.data_ptr(), B, K, F, st)
         self._warped, self._coord = self.warped, coord
         img1 = self.warped[1]
         self._img1, self._feat = img1, feat
-        C.call("ups_step_encode_fwd_rows", l1.data_ptr(), r1, img1.data_ptr(), self.m1.data_ptr(), self.parts.data_ptr(),
-               self.pooled.data_ptr(), B, P, K, self.Kpl, self.ws.data_ptr(), self.ws.numel(), st)
+        _call_rows("ups_step_encode_fwd_rows", nz, l1.data_ptr(), r1, img1.data_ptr(), self.m1.data_ptr(),
+                   self.parts.data_ptr(), self.pooled.data_ptr(), B, P, K, self.Kpl, self.ws.data_ptr(), self.ws.numel(), st)
         return dict(warped=self.warped, m0=self.m0, m1=self.m1, labels0=self.labels0, parts=self.parts,
                     pooled=self.pooled, inj=self.inj)
 
@@ -319,10 +370,13 @@ class PartStep:
         return self._warped
 
     @_on_device
-    def forward_parts(self, l0, l1, feat, conv_V=None, conv_b=None, enc_V=None, enc_b=None, rows=None):
-        """K2 (encode side: l1, warped view 1) and K3 (decode side: l0, feat) on the current stream."""
+    def forward_parts(self, l0, l1, feat, conv_V=None, conv_b=None, enc_V=None, enc_b=None, rows=None, noise_seed=None,
+                      noise_level=1.0):
+        """K2 (encode side: l1, warped view 1) and K3 (decode side: l0, feat) on the current stream.  noise_seed /
+        noise_level: l0, l1 are means, sampled inside the kernels (see forward)."""
         B, S, K, F, P = self.B, self.S, self.K, self.F, self.P
         st = self._stream()
+        nz = self._noise(noise_seed, noise_level)
         r0, r1 = (rows or {}).get("l0", K), (rows or {}).get("l1", K)
         assert (r0 == K and r1 == K) or (self.fused and not self.Co and not self.Ce), "in-place rows need the fused kernels"
         assert l0.is_contiguous() and l1.is_contiguous() and feat.is_contiguous()
@@ -340,22 +394,21 @@ class PartStep:
             assert tuple(enc_V.shape) == (3, 3, 3, self.Ce) and tuple(enc_b.shape) == (self.Ce,)
             assert enc_V.is_contiguous() and enc_b.is_contiguous()
             self._enc_V = enc_V
-            C.call("ups_part_softmax_fwd", l1.data_ptr(), self.m1.data_ptr(), None, self.mh1c.data_ptr(), B * P, K, st)
+            self._softmax_fwd(l1, 1, self.m1, None, self.mh1c, nz, st)
             C.call("ups_parts_conv_fwd", img1.data_ptr(), self.mh1c.data_ptr(), enc_V.data_ptr(), enc_b.data_ptr(),
                    self.e0.data_ptr(), B, S, S, K, 3, self.Ce, st)
         elif self.fused:
-            C.call("ups_step_encode_fwd_rows", l1.data_ptr(), r1, img1.data_ptr(), self.m1.data_ptr(), self.parts.data_ptr(),
-                   self.pooled.data_ptr(), B, P, K, self.Kpl, self.ws.data_ptr(), self.ws.numel(), st)
+            _call_rows("ups_step_encode_fwd_rows", nz, l1.data_ptr(), r1, img1.data_ptr(), self.m1.data_ptr(),
+                       self.parts.data_ptr(), self.pooled.data_ptr(), B, P, K, self.Kpl, self.ws.data_ptr(), self.ws.numel(), st)
         else:
-            C.call("ups_part_softmax_fwd", l1.data_ptr(), self.m1.data_ptr(), None, self.mh1.data_ptr(), B * P, K, st)
+            self._softmax_fwd(l1, 1, self.m1, None, self.mh1, nz, st)
             C.call("ups_mask_parts_fwd", img1.data_ptr(), self.mh1.data_ptr(), self.parts.data_ptr(), B, P, K, 3, 1, st)
             C.call("ups_part_pool_fwd", img1.data_ptr(), self.mh1.data_ptr(), self.pooled.data_ptr(), B, P, K, 3, 0,
                    1.0 / P, self.ws.data_ptr(), self.ws.numel(), st)
         if self.fused or self.Co:
-            self._decode_fwd(l0, feat, conv_V, conv_b, st, r0)
+            self._decode_fwd(l0, feat, conv_V, conv_b, st, r0, nz)
         else:
-            C.call("ups_part_softmax_fwd", l0.data_ptr(), self.m0.data_ptr(), self.labels0.data_ptr(),
-                   self.mh0.data_ptr(), B * P, K, st)
+            self._softmax_fwd(l0, 0, self.m0, self.labels0, self.mh0, nz, st)
             C.call("ups_part_inject_fwd", feat.data_ptr(), self.mh0.data_ptr(), self.inj.data_ptr(), B, P, K, F, st)
         out = dict(warped=warped, m0=self.m0, m1=self.m1, labels0=self.labels0)
         if self.Ce:
@@ -372,7 +425,8 @@ class PartStep:
     def backward(self, g_inj, g_parts, g_pooled=None, g_m0=None, g_m1=None, g_warped=None, rows=None):
         """Cotangents: g_inj [B,S,S,F+K] (with first_conv: g_h0 [B,S,S,Co] in its place), g_parts [K*B,S,S,3]
         (part-major), g_pooled [B,K,3], g_m0/g_m1 [B,S,S,K] (from the mask losses), g_warped [V,B,S,S,3]
-        (views_grad only).  Returns dict(dl0, dl1, dfeat[, dV, db][, dviews]).
+        (views_grad only).  Returns dict(dl0, dl1, dfeat[, dV, db][, dviews]).  After a forward with noise_seed, dl0 / dl1
+        are the gradients of the means (the sample is mean + a constant).
 
         = backward_decode (K4: dl0, dfeat — what the appearance encoder's backward needs) followed by
         backward_encode (K5 [, K6]: dl1 [, dviews])."""
