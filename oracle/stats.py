@@ -6,10 +6,10 @@ import torch
 
 def probs_to_mu_sigma(probs, scaling_factor):
     """cub/code/nn.py:1541-1587.  probs [b,h,w,k]; scaling_factor [b,k] -> mu [b,k,2] (y, x),
-    sigma [b,k,2,2]."""
+    sigma [b,k,2,2].  Evaluated in the dtype and on the device of `probs` (float64 gives the tests' exact reference)."""
     bn, h, w, nk = probs.shape
-    y_t = torch.linspace(-1.0, 1.0, h).reshape(h, 1).repeat(1, w)
-    x_t = torch.linspace(-1.0, 1.0, w).reshape(1, w).repeat(h, 1)
+    y_t = torch.linspace(-1.0, 1.0, h, dtype=probs.dtype, device=probs.device).reshape(h, 1).repeat(1, w)
+    x_t = torch.linspace(-1.0, 1.0, w, dtype=probs.dtype, device=probs.device).reshape(1, w).repeat(h, 1)
     meshgrid = torch.stack([y_t, x_t], dim=-1)                               # [h,w,2]
     mu = torch.einsum("ijl,aijk->akl", meshgrid, probs)
     mu_out_prod = torch.einsum("akm,akn->akmn", mu, mu)

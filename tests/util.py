@@ -31,14 +31,6 @@ def make_inputs(B, S, K, F, V=3, seed=0, tps=CUB_TPS, ties=False, tps_seed=1234)
     return dict(views=views, l0=l0, l1=l1, feat=feat, coord=coord, t_vector=t_vector, prm=prm, cot=cot)
 
 
-def reduce_atol(n_terms, atol=ATOL):
-    """Absolute tolerance for an fp32 reduction over `n_terms` O(1) terms (dfeat sums P/K pixels
-    per entry): two valid fp32 summation orders - the oracle's and the kernel's - differ by
-    ~eps*sqrt(n)*|term| on entries that cancel to ~0, where a relative bound is meaningless.
-    1e-5 up to 1024 terms, growing with sqrt(n) beyond."""
-    return atol * max(1.0, (n_terms / 1024.0) ** 0.5)
-
-
 def cuda(x):
     if isinstance(x, torch.Tensor):
         return x.cuda().contiguous()
