@@ -371,6 +371,21 @@ int ups_step_warp_decode_fwd_noise(const float* U, const float* U2, const float*
                                    float* out2, int N, int N2, int S, const float* l0, int l0_row, const float* feat, float* m0,
                                    long long* labels0, float* inj, int B, int K, int F, unsigned long long seed,
                                    long long sample_offset, float noise_level, void* stream);
+/* The same draws with the seed read from device memory: `seed` points to one device word (the uint64 seed, e.g. a
+ * one-element int64 tensor holding the same bits) that the kernel loads once, in its prologue.  For equal seed values the
+ * results are bit-identical to the by-value forms above.  A launch captured in a CUDA graph keeps the pointer, not the
+ * value: writing a new seed into the word before a replay gives that replay a new draw. */
+int ups_normal_philox_fwd_dseed(const unsigned long long* seed, int draw, long long pix_offset, long long n_pix, int K,
+                                float* out, void* stream);
+int ups_part_softmax_sampled_philox_fwd_dseed(const float* mean, const unsigned long long* seed, int draw,
+                                              long long pix_offset, float noise_level, float* logits_out, float* probs,
+                                              int64_t* labels, float* hard, long long n_pix, int K, void* stream);
+int ups_step_decode_fwd_noise_dseed(const float* l0, int l0_row, const float* feat, float* m0, long long* labels0,
+                                    float* inj, int B, int P, int K, int F, const unsigned long long* seed,
+                                    long long sample_offset, float noise_level, void* stream);
+int ups_step_encode_fwd_noise_dseed(const float* l1, int l1_row, const float* img1, float* m1, float* parts_pm,
+                                    float* pooled, int B, int P, int K, int Kpl, void* ws, size_t ws_bytes,
+                                    const unsigned long long* seed, long long sample_offset, float noise_level, void* stream);
 
 /* K1 + K3 of the fused step in ONE launch (csrc/step_fwd_fused.cu): the TPS warp of the views (ups_tps_warp_pair_fwd's
  * arguments: U [N,S,S,3], optional second image set U2 [N2,S,S,3] sharing the first N2 warps, coord, T -> out, out2) and

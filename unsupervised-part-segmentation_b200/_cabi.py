@@ -90,6 +90,10 @@ _SIGS = {
     "ups_step_decode_fwd_noise": [c_f, c_i] + [c_f] * 4 + [c_i] * 4 + [c_u64, c_ll, c_fl, c_f],
     "ups_step_encode_fwd_noise": [c_f, c_i] + [c_f] * 4 + [c_i] * 4 + [c_f, c_sz] + [c_u64, c_ll, c_fl, c_f],
     "ups_step_warp_decode_fwd_noise": [c_f] * 6 + [c_i] * 3 + [c_f, c_i] + [c_f] * 4 + [c_i] * 3 + [c_u64, c_ll, c_fl, c_f],
+    "ups_normal_philox_fwd_dseed": [c_f, c_i, c_ll, c_ll, c_i, c_f, c_f],
+    "ups_part_softmax_sampled_philox_fwd_dseed": [c_f, c_f, c_i, c_ll, c_fl, c_f, c_f, c_f, c_f, c_ll, c_i, c_f],
+    "ups_step_decode_fwd_noise_dseed": [c_f, c_i] + [c_f] * 4 + [c_i] * 4 + [c_f, c_ll, c_fl, c_f],
+    "ups_step_encode_fwd_noise_dseed": [c_f, c_i] + [c_f] * 4 + [c_i] * 4 + [c_f, c_sz] + [c_f, c_ll, c_fl, c_f],
 }
 
 OP_TPS_SOLVE, OP_POOL, OP_INJECT_BWD, OP_POOL_BWD, OP_STEP, OP_MOMENTS, OP_KL = 0, 1, 2, 3, 4, 5, 6

@@ -96,6 +96,15 @@ __device__ __forceinline__ float4 add_noise4(float4 v, const NoiseArgs& n, int b
                        sampled_logit(v.w, n.level, z3));
 }
 
+// DSEED (the `_dseed` entry points): NoiseArgs::seed carries the ADDRESS of the seed, one device word, and the kernel reads
+// it once, in its prologue.  A launch captured in a CUDA graph then draws with whatever the word holds when the graph is
+// replayed.  DSEED = false is the by-value seed, returned unchanged.
+template <bool DSEED>
+__device__ __forceinline__ NoiseArgs resolve_seed(NoiseArgs nz) {
+    if (DSEED) nz.seed = *reinterpret_cast<const unsigned long long*>(nz.seed);
+    return nz;
+}
+
 template <int W>
 __device__ __forceinline__ float group_max(float v) {
 #pragma unroll

@@ -11,16 +11,18 @@ constexpr int TPB = 256;
 // Fast path: K = 4*LPP, LPP lanes per pixel, one float4 per lane, fully coalesced.
 // MODE: SM_PLAIN softmax(logits); SM_EPS logits = mean + noise*eps first (MeanFieldDistribution.sample,
 // cub/code/nn.py:1421-1427), one rounding per step; SM_PHILOX the same with eps drawn in registers (canon_math.cuh, the
-// mean-field logit noise; pixel i is global pixel nz.sample_offset + i).
-constexpr int SM_PLAIN = 0, SM_EPS = 1, SM_PHILOX = 2;
+// mean-field logit noise; pixel i is global pixel nz.sample_offset + i); SM_PHILOX_DSEED that with the seed read from
+// device memory (resolve_seed).
+constexpr int SM_PLAIN = 0, SM_EPS = 1, SM_PHILOX = 2, SM_PHILOX_DSEED = 3;
 template <int LPP, int UNROLL, int MODE>
 __global__ void __launch_bounds__(TPB) part_softmax_fwd_kernel(const float* __restrict__ logits,
                                                                const float* __restrict__ eps, float noise,
                                                                float* __restrict__ logits_out,
                                                                float* __restrict__ probs,
                                                                long long* __restrict__ labels,
-                                                               float* __restrict__ hard, long long n4, NoiseArgs nz) {
+                                                               float* __restrict__ hard, long long n4, NoiseArgs nz_arg) {
     // n4 = n_pix * LPP float4s in total; every lane stays alive for the shuffles
+    const NoiseArgs nz = resolve_seed<MODE == SM_PHILOX_DSEED>(nz_arg);
     const long long base = ((long long)blockIdx.x * UNROLL) * TPB + threadIdx.x;
     float4 v[UNROLL];
 #pragma unroll
@@ -33,7 +35,7 @@ __global__ void __launch_bounds__(TPB) part_softmax_fwd_kernel(const float* __re
             v[u] = make_float4(__fadd_rn(v[u].x, __fmul_rn(noise, e.x)), __fadd_rn(v[u].y, __fmul_rn(noise, e.y)),
                                __fadd_rn(v[u].z, __fmul_rn(noise, e.z)), __fadd_rn(v[u].w, __fmul_rn(noise, e.w)));
         }
-        if (MODE == SM_PHILOX) {
+        if (MODE >= SM_PHILOX) {
             float z0, z1, z2, z3;
             normal4_philox(nz.seed, (uint32_t)nz.draw, (unsigned long long)(nz.sample_offset + ii / LPP),
                            (uint32_t)(ii & (LPP - 1)), z0, z1, z2, z3);
@@ -65,18 +67,19 @@ __global__ void __launch_bounds__(128) part_softmax_fwd_generic_kernel(const flo
                                                                        float* __restrict__ probs,
                                                                        long long* __restrict__ labels,
                                                                        float* __restrict__ hard, long long n_pix,
-                                                                       int K, NoiseArgs nz) {
+                                                                       int K, NoiseArgs nz_arg) {
+    const NoiseArgs nz = resolve_seed<MODE == SM_PHILOX_DSEED>(nz_arg);
     const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_pix) return;
     float x[KMAX], p[KMAX], e[KMAX];
     for (int k = 0; k < K; ++k) x[k] = logits[i * K + k];
-    if (MODE != SM_PHILOX && eps) {
+    if (MODE < SM_PHILOX && eps) {
         for (int k = 0; k < K; ++k) {
             x[k] = __fadd_rn(x[k], __fmul_rn(noise, eps[i * K + k]));
             if (logits_out) logits_out[i * K + k] = x[k];
         }
     }
-    if (MODE == SM_PHILOX) {
+    if (MODE >= SM_PHILOX) {
         for (int j = 0; 4 * j < K; ++j) {
             float z[4];
             normal4_philox(nz.seed, (uint32_t)nz.draw, (unsigned long long)(nz.sample_offset + i), (uint32_t)j, z[0], z[1],
@@ -129,8 +132,11 @@ __global__ void part_softmax_bwd_generic_kernel(const float* __restrict__ probs,
     for (int k = 0; k < K; ++k) dlogits[i * K + k] = probs[i * K + k] * (gsum(i * K + k) - dot);
 }
 
-// eps [n_pix, K] of global pixels pix_offset + i: one thread per (pixel, group of 4 parts)
-__global__ void __launch_bounds__(TPB) normal_philox_kernel(float* __restrict__ out, long long n, int J, int K, NoiseArgs nz) {
+// eps [n_pix, K] of global pixels pix_offset + i: one thread per (pixel, group of 4 parts); DSEED: see resolve_seed
+template <bool DSEED>
+__global__ void __launch_bounds__(TPB) normal_philox_kernel(float* __restrict__ out, long long n, int J, int K,
+                                                            NoiseArgs nz_arg) {
+    const NoiseArgs nz = resolve_seed<DSEED>(nz_arg);
     const long long t = (long long)blockIdx.x * TPB + threadIdx.x;   // over n_pix * J
     if (t >= n) return;
     const long long i = t / J;
@@ -440,10 +446,11 @@ using namespace ups;
 static inline unsigned nblk(long long n, int tpb) { return (unsigned)cdiv(n, tpb); }
 #define UPS_GRID_OK(n, tpb) UPS_REQUIRE(cdiv((n), (tpb)) < (1ll << 31), "problem too large for one launch")
 
-// nz != nullptr: the philox mode (eps == nullptr); eps != nullptr: the eps mode; neither: plain softmax
+// nz != nullptr: the philox mode (eps == nullptr; dseed: nz->seed is the seed's device address); eps != nullptr: the eps
+// mode; neither: plain softmax
 static int part_softmax_fwd_impl(const char* what, const float* logits, const float* eps, float noise,
                                  float* logits_out, float* probs, long long* labels, float* hard_st, long long n_pix,
-                                 int K, void* stream, const NoiseArgs* nz = nullptr) {
+                                 int K, void* stream, const NoiseArgs* nz = nullptr, bool dseed = false) {
     UPS_REQUIRE(logits && probs, "%s: null pointer", what);
     UPS_REQUIRE(n_pix >= 0 && K >= 1 && K <= KMAX, "%s: n_pix=%lld K=%d (1..%d)", what, n_pix, K, KMAX);
     if (n_pix == 0) return UPS_OK;
@@ -455,7 +462,10 @@ static int part_softmax_fwd_impl(const char* what, const float* logits, const fl
     {                                                                                                                \
         const long long n4 = n_pix * LPP;                                                                            \
         UPS_GRID_OK(n4, TPB * U);                                                                                    \
-        if (nz)                                                                                                      \
+        if (nz && dseed)                                                                                             \
+            part_softmax_fwd_kernel<LPP, U, SM_PHILOX_DSEED><<<nblk(n4, TPB * U), TPB, 0, s>>>(                      \
+                logits, nullptr, 0.f, logits_out, probs, labels, hard_st, n4, *nz);                                  \
+        else if (nz)                                                                                                 \
             part_softmax_fwd_kernel<LPP, U, SM_PHILOX><<<nblk(n4, TPB * U), TPB, 0, s>>>(                            \
                 logits, nullptr, 0.f, logits_out, probs, labels, hard_st, n4, *nz);                                  \
         else if (eps)                                                                                                \
@@ -473,7 +483,10 @@ static int part_softmax_fwd_impl(const char* what, const float* logits, const fl
     if (vec && K == 32) UPS_SM_FWD(8)
 #undef UPS_SM_FWD
     UPS_GRID_OK(n_pix, 128);
-    if (nz)
+    if (nz && dseed)
+        part_softmax_fwd_generic_kernel<SM_PHILOX_DSEED><<<nblk(n_pix, 128), 128, 0, s>>>(logits, nullptr, 0.f, logits_out,
+                                                                                      probs, labels, hard_st, n_pix, K, *nz);
+    else if (nz)
         part_softmax_fwd_generic_kernel<SM_PHILOX><<<nblk(n_pix, 128), 128, 0, s>>>(logits, nullptr, 0.f, logits_out, probs,
                                                                                 labels, hard_st, n_pix, K, *nz);
     else
@@ -505,8 +518,21 @@ extern "C" int ups_part_softmax_sampled_philox_fwd(const float* mean, unsigned l
                                  reinterpret_cast<long long*>(labels), hard_st, n_pix, K, stream, &nz);
 }
 
-extern "C" int ups_normal_philox_fwd(unsigned long long seed, int draw, long long pix_offset, long long n_pix, int K, float* out,
-                                     void* stream) {
+extern "C" int ups_part_softmax_sampled_philox_fwd_dseed(const float* mean, const unsigned long long* seed, int draw,
+                                                         long long pix_offset, float noise_level, float* logits_out,
+                                                         float* probs, int64_t* labels, float* hard_st, long long n_pix, int K,
+                                                         void* stream) {
+    UPS_REQUIRE(seed, "part_softmax_sampled_philox_fwd: null seed pointer");
+    UPS_REQUIRE(draw >= 0 && pix_offset >= 0, "part_softmax_sampled_philox_fwd: draw=%d pix_offset=%lld", draw, pix_offset);
+    const NoiseArgs nz{(unsigned long long)(uintptr_t)seed, pix_offset, noise_level, draw};
+    return part_softmax_fwd_impl("part_softmax_sampled_philox_fwd", mean, nullptr, 0.f, logits_out, probs,
+                                 reinterpret_cast<long long*>(labels), hard_st, n_pix, K, stream, &nz, true);
+}
+
+// seed: the value (DSEED = false) or its device address
+template <bool DSEED>
+static int normal_philox_launch(unsigned long long seed, int draw, long long pix_offset, long long n_pix, int K, float* out,
+                                void* stream) {
     UPS_REQUIRE(out, "normal_philox_fwd: null pointer");
     UPS_REQUIRE(n_pix >= 0 && K >= 1 && draw >= 0 && pix_offset >= 0, "normal_philox_fwd: n_pix=%lld K=%d draw=%d pix_offset=%lld",
                 n_pix, K, draw, pix_offset);
@@ -515,8 +541,19 @@ extern "C" int ups_normal_philox_fwd(unsigned long long seed, int draw, long lon
     const int J = (K + 3) / 4;
     const long long n = n_pix * J;
     UPS_GRID_OK(n, TPB);
-    normal_philox_kernel<<<nblk(n, TPB), TPB, 0, as_stream(stream)>>>(out, n, J, K, NoiseArgs{seed, pix_offset, 1.0f, draw});
+    normal_philox_kernel<DSEED><<<nblk(n, TPB), TPB, 0, as_stream(stream)>>>(out, n, J, K, NoiseArgs{seed, pix_offset, 1.0f, draw});
     return after_launch("normal_philox_kernel");
+}
+
+extern "C" int ups_normal_philox_fwd(unsigned long long seed, int draw, long long pix_offset, long long n_pix, int K, float* out,
+                                     void* stream) {
+    return normal_philox_launch<false>(seed, draw, pix_offset, n_pix, K, out, stream);
+}
+
+extern "C" int ups_normal_philox_fwd_dseed(const unsigned long long* seed, int draw, long long pix_offset, long long n_pix, int K,
+                                           float* out, void* stream) {
+    UPS_REQUIRE(seed, "normal_philox_fwd: null seed pointer");
+    return normal_philox_launch<true>((unsigned long long)(uintptr_t)seed, draw, pix_offset, n_pix, K, out, stream);
 }
 
 extern "C" int ups_part_softmax_bwd(const float* probs, const float* g, float* dlogits, long long n_pix, int K,

@@ -30,7 +30,7 @@ template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N)); }
 
 // ============================================================================ K3 decode fwd (body: step_decode_fwd.cuh)
-template <int LPP, int FT, bool NOISE>
+template <int LPP, int FT, bool NOISE, bool DSEED>
 __global__ void __launch_bounds__(FTPB) step_decode_fwd_kernel(const float* __restrict__ l0,
                                                                const float* __restrict__ feat,
                                                                float* __restrict__ m0,
@@ -39,7 +39,7 @@ __global__ void __launch_bounds__(FTPB) step_decode_fwd_kernel(const float* __re
                                                                int pix_per_cta, int l0_row, NoiseArgs nz) {
     extern __shared__ float4 fs4[];  // feat[b] as [K][F/4] float4
     step_decode_fwd_body<LPP, FT, NOISE>(l0, feat, m0, labels0, inj, P, Frt, pix_per_cta, blockIdx.x, blockIdx.y, fs4, l0_row,
-                                         nz);
+                                         resolve_seed<DSEED>(nz));
 }
 
 // ============================================================================ K2 encode fwd
@@ -55,14 +55,16 @@ struct EncFwdSmem {
 
 // MINB: resident CTAs per SM asked of ptxas (an explicit value also keeps the exp chains interleaved)
 // NOISE: l1 holds the means, sampled in registers right after the load (canon_math.cuh, the mean-field logit noise)
-template <int LPP, int MINB, bool PAD, bool NOISE>
+// DSEED: the seed is read from device memory (resolve_seed)
+template <int LPP, int MINB, bool PAD, bool NOISE, bool DSEED>
 __global__ void __launch_bounds__(FTPB, MINB) step_encode_fwd_kernel(const float* __restrict__ l1,
                                                                const float* __restrict__ img1,
                                                                float* __restrict__ m1, float* __restrict__ parts,
                                                                float* __restrict__ partial, int B, int P,
-                                                               int pix_per_cta, int Kpl, int l1_row, NoiseArgs nz) {
+                                                               int pix_per_cta, int Kpl, int l1_row, NoiseArgs nz_arg) {
     // Kpl <= K: number of part planes that exist in `parts` (planes Kpl..K-1 are padding of a K that is not a power
     // of two: their mask is identically zero and they are neither written nor allocated)
+    const NoiseArgs nz = resolve_seed<DSEED>(nz_arg);
     using L = EncFwdSmem<LPP>;
     constexpr int K = L::K, PW = 32 / LPP;
     extern __shared__ float4 smem4[];
@@ -416,7 +418,7 @@ extern "C" int ups_step_decode_fwd(const float* l0, const float* feat, float* m0
     return ups_step_decode_fwd_rows(l0, K, feat, m0, labels0, inj, B, P, K, F, stream);
 }
 
-template <bool NOISE>
+template <bool NOISE, bool DSEED = false>
 static int decode_fwd_launch(const float* l0, int l0_row, const float* feat, float* m0, long long* labels0, float* inj, int B,
                              int P, int K, int F, NoiseArgs nz, void* stream) {
     UPS_REQUIRE(l0 && feat && m0 && labels0 && inj, "step_decode_fwd: null pointer");
@@ -435,8 +437,8 @@ static int decode_fwd_launch(const float* l0, int l0_row, const float* feat, flo
     cudaStream_t s = as_stream(stream);
 #define UPS_DEC_FWD2(LPP, FT)                                                                           \
     {                                                                                                   \
-        if (int rc = set_smem(step_decode_fwd_kernel<LPP, FT, NOISE>, sm)) return rc;                   \
-        step_decode_fwd_kernel<LPP, FT, NOISE><<<grid, FTPB, sm, s>>>(l0, feat, m0, labels0, inj, P, F, per, l0_row, nz); \
+        if (int rc = set_smem(step_decode_fwd_kernel<LPP, FT, NOISE, DSEED>, sm)) return rc;            \
+        step_decode_fwd_kernel<LPP, FT, NOISE, DSEED><<<grid, FTPB, sm, s>>>(l0, feat, m0, labels0, inj, P, F, per, l0_row, nz); \
     }
 #define UPS_DEC_FWD(LPP) \
     { if (F == 64) UPS_DEC_FWD2(LPP, 64) else if (F == 32) UPS_DEC_FWD2(LPP, 32) else if (F == 16) UPS_DEC_FWD2(LPP, 16) else UPS_DEC_FWD2(LPP, 0) }
@@ -459,6 +461,15 @@ extern "C" int ups_step_decode_fwd_noise(const float* l0, int l0_row, const floa
                                    stream);
 }
 
+extern "C" int ups_step_decode_fwd_noise_dseed(const float* l0, int l0_row, const float* feat, float* m0, long long* labels0,
+                                               float* inj, int B, int P, int K, int F, const unsigned long long* seed,
+                                               long long sample_offset, float noise_level, void* stream) {
+    UPS_REQUIRE(seed, "step_decode_fwd: null seed pointer");
+    UPS_REQUIRE(sample_offset >= 0, "step_decode_fwd: sample_offset=%lld", sample_offset);
+    return decode_fwd_launch<true, true>(l0, l0_row, feat, m0, labels0, inj, B, P, K, F,
+                                         NoiseArgs{(unsigned long long)(uintptr_t)seed, sample_offset, noise_level, 0}, stream);
+}
+
 extern "C" int ups_step_encode_fwd(const float* l1, const float* img1, float* m1, float* parts_pm, float* pooled,
                                    int B, int P, int K, void* ws, size_t ws_bytes, void* stream) {
     return ups_step_encode_fwd_planes(l1, img1, m1, parts_pm, pooled, B, P, K, K, ws, ws_bytes, stream);
@@ -469,7 +480,7 @@ extern "C" int ups_step_encode_fwd_planes(const float* l1, const float* img1, fl
     return ups_step_encode_fwd_rows(l1, K, img1, m1, parts_pm, pooled, B, P, K, Kpl, ws, ws_bytes, stream);
 }
 
-template <bool NOISE>
+template <bool NOISE, bool DSEED = false>
 static int encode_fwd_launch(const float* l1, int l1_row, const float* img1, float* m1, float* parts_pm, float* pooled, int B,
                              int P, int K, int Kpl, void* ws, size_t ws_bytes, NoiseArgs nz, void* stream) {
     UPS_REQUIRE(l1 && img1 && m1 && parts_pm && pooled, "step_encode_fwd: null pointer");
@@ -490,11 +501,11 @@ static int encode_fwd_launch(const float* l1, int l1_row, const float* img1, flo
     {                                                                                                         \
         const size_t sm = (size_t)FW * EncFwdSmem<LPP>::WREG * sizeof(float);                                 \
         if (Kpl < K) {                                                                                        \
-            if (int rc = set_smem(step_encode_fwd_kernel<LPP, MB, true, NOISE>, sm)) return rc;               \
-            step_encode_fwd_kernel<LPP, MB, true, NOISE><<<grid, FTPB, sm, s>>>(l1, img1, m1, parts_pm, partial, B, P, per, Kpl, l1_row, nz); \
+            if (int rc = set_smem(step_encode_fwd_kernel<LPP, MB, true, NOISE, DSEED>, sm)) return rc;               \
+            step_encode_fwd_kernel<LPP, MB, true, NOISE, DSEED><<<grid, FTPB, sm, s>>>(l1, img1, m1, parts_pm, partial, B, P, per, Kpl, l1_row, nz); \
         } else {                                                                                              \
-            if (int rc = set_smem(step_encode_fwd_kernel<LPP, MB, false, NOISE>, sm)) return rc;              \
-            step_encode_fwd_kernel<LPP, MB, false, NOISE><<<grid, FTPB, sm, s>>>(l1, img1, m1, parts_pm, partial, B, P, per, Kpl, l1_row, nz); \
+            if (int rc = set_smem(step_encode_fwd_kernel<LPP, MB, false, NOISE, DSEED>, sm)) return rc;              \
+            step_encode_fwd_kernel<LPP, MB, false, NOISE, DSEED><<<grid, FTPB, sm, s>>>(l1, img1, m1, parts_pm, partial, B, P, per, Kpl, l1_row, nz); \
         }                                                                                                     \
     }
 #define UPS_ENC_FWD(LPP) \
@@ -520,6 +531,16 @@ extern "C" int ups_step_encode_fwd_noise(const float* l1, int l1_row, const floa
     UPS_REQUIRE(sample_offset >= 0, "step_encode_fwd: sample_offset=%lld", sample_offset);
     return encode_fwd_launch<true>(l1, l1_row, img1, m1, parts_pm, pooled, B, P, K, Kpl, ws, ws_bytes,
                                    NoiseArgs{seed, sample_offset, noise_level, 1}, stream);
+}
+
+extern "C" int ups_step_encode_fwd_noise_dseed(const float* l1, int l1_row, const float* img1, float* m1, float* parts_pm,
+                                               float* pooled, int B, int P, int K, int Kpl, void* ws, size_t ws_bytes,
+                                               const unsigned long long* seed, long long sample_offset, float noise_level,
+                                               void* stream) {
+    UPS_REQUIRE(seed, "step_encode_fwd: null seed pointer");
+    UPS_REQUIRE(sample_offset >= 0, "step_encode_fwd: sample_offset=%lld", sample_offset);
+    return encode_fwd_launch<true, true>(l1, l1_row, img1, m1, parts_pm, pooled, B, P, K, Kpl, ws, ws_bytes,
+                                         NoiseArgs{(unsigned long long)(uintptr_t)seed, sample_offset, noise_level, 1}, stream);
 }
 
 extern "C" int ups_step_decode_bwd(const float* g_inj, const float* m0, const float* g_m0, const float* feat,

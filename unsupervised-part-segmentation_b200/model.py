@@ -109,6 +109,46 @@ def decode_conv2d(logits, feature_vectors, V, b):
     return ops.decode_conv(logits, G, b)
 
 
+def _noise_args(noise_seed):
+    """noise_seed (None, an int in [0, 2**64) or a one-element int64 CUDA tensor) -> the ops' (noise, seed, seed_value)."""
+    if noise_seed is None:
+        return ops.NOISE_NONE, None, 0
+    if isinstance(noise_seed, torch.Tensor):
+        return ops.NOISE_DEVICE, noise_seed, 0
+    return ops.NOISE_INT, None, ops._seed_i64(noise_seed)
+
+
+def part_encode(logits1, image1, noise_seed=None, noise_level=1.0, sample_offset=0):
+    """The encode side of the step (model.py:428-430,453-455,478 and the pooling tail of e_alpha, :50-52) in one kernel:
+    m1 = softmax(logits1); mask = ST(hard_max(m1)); parts = mask_parts(image1, mask) folded part-major
+    (nn.apply_partwise, cub/code/nn.py:100-103); pooled = mean over pixels of mask * image1.
+    logits1 [B,h,w,parts], image1 [B,h,w,3] (the warped view 1) -> (m1, parts [parts*B,h,w,3] with row k*B+b,
+    pooled [B,parts,3]).  Differentiable in logits1, and in image1 when it requires grad.
+    noise_seed: l1 are the means of MeanFieldDistribution and the kernel softmaxes the sample
+    logits1 + noise_level * eps (model.py:420-421), eps drawn on the device from the seed (draw 1, pixel
+    (sample_offset + b) * h*w + p, as PartStep.forward).  An int is passed by value; a one-element int64 CUDA tensor is
+    read by the kernel, which is what a captured CUDA graph needs (an int raises during capture)."""
+    bs, h, w, n_parts = logits1.shape
+    ishape = list(image1.shape)
+    assert ishape == [bs, h, w, 3], ishape
+    noise, seed, seed_value = _noise_args(noise_seed)
+    return ops.part_encode(logits1, image1, noise, seed, seed_value, float(noise_level), int(sample_offset))
+
+
+def part_decode(logits0, feature_vectors, noise_seed=None, noise_level=1.0, sample_offset=0):
+    """The decode side of the step (model.py:426,434-436,447,470,482-484) in one kernel: m0 = softmax(logits0);
+    labels = argmax(m0); mask = ST(hard_max(m0)); inj = concat(sum_k unpool_features(feature_vectors, mask), mask).
+    logits0 [B,h,w,parts], feature_vectors [B,parts,F] (e_alpha's output) -> (m0, labels int64 [B,h,w],
+    inj [B,h,w,F+parts]).  Differentiable in logits0 and feature_vectors.  noise_seed, noise_level, sample_offset as in
+    part_encode (draw 0)."""
+    bs, h, w, n_parts = logits0.shape
+    fshape = list(feature_vectors.shape)
+    assert len(fshape) == 3, fshape
+    assert fshape[0] == bs and fshape[1] == n_parts, fshape
+    noise, seed, seed_value = _noise_args(noise_seed)
+    return ops.part_decode(logits0, feature_vectors, noise, seed, seed_value, float(noise_level), int(sample_offset))
+
+
 def parts_conv2d(image, mask, V, b):
     """The appearance encoder's first layer on the masked part images, without the part images:
     `mask_parts(image, mask)` (cub/code/SB_model48i/model.py:176-187, :478) folded part-major by

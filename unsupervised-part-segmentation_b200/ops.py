@@ -4,12 +4,14 @@ PyTorch is plumbing here: it owns device memory and streams and records the auto
 every numeric result comes from the sm_100a kernels in csrc/.  There is no CPU
 implementation: a CPU tensor raises.
 """
+import math
 from typing import Optional, Tuple
 
 import torch
 from torch import Tensor
 
 from . import _cabi as C
+from .step import decode_bwd_tc_ok, kernel_route
 
 
 def _stream(t: Tensor):
@@ -886,3 +888,282 @@ def _draw_rect(centers: Tensor, ph: int, pw: int, H: int, W: int) -> Tensor:
 
 
 draw_rect = _op("draw_rect", _draw_rect, lambda c, ph, pw, H, W: c.new_empty(c.shape[0], H, W, dtype=torch.float32))
+
+
+# ------------------------------------------------------------------ the step's two sides in the reference model's order
+# model.py:426-485 runs the appearance encoder between the sides: part_encode (K2: m1, the part images and their mean pool)
+# feeds e_alpha, whose output feeds part_decode (K3: m0, labels0 and the injected map).  Each side is one op with autograd
+# (K5 / K4 as its backward) on the kernels step.kernel_route picks, the rule PartStep follows, so both produce the same
+# bits.  Outputs and workspaces come from the caching allocator on every call: two forwards may precede their backwards.
+# A padded part count (e.g. 25 on the kernels of 32) returns views [..., :K] of row-pitched buffers, as PartStep does.
+#
+# Noise (the sampled logits of MeanFieldDistribution.sample, model.py:420-421): `noise` = NOISE_NONE, NOISE_INT (the
+# seed is `seed_value`, passed by value) or NOISE_DEVICE (the seed is the one int64 element of `seed`, read by the kernels
+# from device memory, so a captured CUDA graph draws with whatever that tensor holds at replay).  Decode draws 0, encode
+# draws 1: the draws of PartStep.forward(noise_seed=...).
+NOISE_NONE, NOISE_INT, NOISE_DEVICE = 0, 1, 2
+
+
+def _noise_call(name, noise, seed, seed_value, *args):
+    """Call entry point `name` noise-free, or its `_noise` / `_noise_dseed` form: the same arguments with
+    (seed, sample_offset, noise_level) inserted before the stream (`args` ends with those three and the stream)."""
+    *head, offset, level, st = args
+    if noise == NOISE_NONE:
+        C.call(name, *head, st)
+    elif noise == NOISE_INT:
+        C.call(name[:-len("_rows")] + "_noise", *head, seed_value % 2 ** 64, offset, level, st)
+    else:
+        C.call(name[:-len("_rows")] + "_noise_dseed", *head, seed.data_ptr(), offset, level, st)
+
+
+def _softmax_noise(logits, noise, seed, seed_value, draw, pix_offset, level, probs, labels, hard, n_pix, K, st):
+    """The generic kernels' softmax of the logits, or of the sampled logits (the step's draw `draw`)."""
+    if noise == NOISE_NONE:
+        C.call("ups_part_softmax_fwd", logits.data_ptr(), probs.data_ptr(), _ptr(labels), _ptr(hard), n_pix, K, st)
+    elif noise == NOISE_INT:
+        C.call("ups_part_softmax_sampled_philox_fwd", logits.data_ptr(), seed_value % 2 ** 64, draw, pix_offset, level,
+               None, probs.data_ptr(), _ptr(labels), _ptr(hard), n_pix, K, st)
+    else:
+        C.call("ups_part_softmax_sampled_philox_fwd_dseed", logits.data_ptr(), seed.data_ptr(), draw, pix_offset, level,
+               None, probs.data_ptr(), _ptr(labels), _ptr(hard), n_pix, K, st)
+
+
+def _check_noise(noise: int, seed: Optional[Tensor], device):
+    if noise == NOISE_INT and torch.cuda.is_current_stream_capturing():
+        raise C.UpsError("ups_b200: an int noise_seed is frozen into a captured CUDA graph (every replay would draw the "
+                         "same noise); pass the seed as a one-element int64 CUDA tensor")
+    if noise == NOISE_DEVICE:
+        if seed is None or seed.dtype != torch.int64 or seed.numel() != 1 or seed.device != device:
+            raise C.UpsError("ups_b200: a device noise_seed is a one-element int64 tensor on the logits' device")
+        if not seed.is_contiguous():
+            raise C.UpsError("ups_b200: the device noise_seed must be contiguous")
+
+
+def _pitched(t: Tensor, Kp: int, st) -> Tensor:
+    """A [.., K] tensor as the base of a row-pitched [.., Kp] buffer: itself when it already is a view [..., :K] of
+    such a buffer (what the padded forwards return), else a zero-padded copy."""
+    K = t.shape[-1]
+    rows = t.numel() // K if K else 0
+    if (t.stride(-1) == 1 and all(t.stride(i) == Kp * math.prod(t.shape[i + 1:-1]) for i in range(t.dim() - 1))
+            and t.untyped_storage().nbytes() >= (t.storage_offset() + rows * Kp) * t.element_size()):
+        return t
+    t = t.contiguous()
+    out = torch.empty(*t.shape[:-1], Kp, dtype=t.dtype, device=t.device)
+    C.call("ups_copy_rows", t.data_ptr(), K, out.data_ptr(), Kp, t.numel() // K if K else 0, K, Kp - K, 0.0, st)
+    return out
+
+
+def _pad_rows(t: Tensor, n: int, pitch: int, st) -> Tensor:
+    """Contiguous [.., n] -> [.., pitch], the columns n.. zero."""
+    t = t.contiguous()
+    out = torch.empty(*t.shape[:-1], pitch, dtype=t.dtype, device=t.device)
+    C.call("ups_copy_rows", t.data_ptr(), n, out.data_ptr(), pitch, t.numel() // n, n, pitch - n, 0.0, st)
+    return out
+
+
+def _hard_of(probs: Tensor, st) -> Tensor:
+    """ST(hard_max(probs)), bit for bit what the softmax kernels write as `hard`."""
+    K = probs.shape[-1]
+    h = torch.empty_like(probs)
+    C.call("ups_hard_max_fwd", probs.data_ptr(), h.data_ptr(), probs.numel() // K, K, st)
+    C.call("ups_straight_through_fwd", h.data_ptr(), probs.data_ptr(), h.data_ptr(), h.numel(), st)
+    return h
+
+
+def _padded_fake(shape, K, Kp, like):
+    """Fake of a view [..., :n] of a [..., n + Kp - K] buffer (n = shape[-1])."""
+    n = shape[-1]
+    return like.new_empty(*shape[:-1], n + Kp - K)[..., :n]
+
+
+# ---- encode side: K2 forward, K5 backward
+def _part_encode(l1: Tensor, image1: Tensor, noise: int, seed: Optional[Tensor], seed_value: int, noise_level: float,
+                 sample_offset: int) -> Tuple[Tensor, Tensor, Tensor]:
+    l1, img = _f32(l1, "logits1"), _f32(image1, "image1")
+    _check_noise(noise, seed, l1.device)
+    B, H, W, K = l1.shape
+    P = H * W
+    st = _stream(l1)
+    route, Kk = kernel_route(K, None, P)
+    dev = dict(dtype=torch.float32, device=l1.device)
+    parts = torch.empty(K * B, H, W, 3, **dev)
+    if route == "generic":
+        m1, hard = torch.empty_like(l1), torch.empty_like(l1)
+        pooled = torch.empty(B, K, 3, **dev)
+        _softmax_noise(l1, noise, seed, seed_value, 1, sample_offset * P, noise_level, m1, None, hard, B * P, K, st)
+        C.call("ups_mask_parts_fwd", img.data_ptr(), hard.data_ptr(), parts.data_ptr(), B, P, K, 3, 1, st)
+        ws = _ws(C.workspace_bytes(C.OP_POOL, B, P, K, 3), l1)
+        C.call("ups_part_pool_fwd", img.data_ptr(), hard.data_ptr(), pooled.data_ptr(), B, P, K, 3, 0, 1.0 / P,
+               ws.data_ptr(), ws.numel(), st)
+        return m1, parts, pooled
+    m1 = torch.empty(B, H, W, Kk, **dev)
+    pooled = torch.empty(B, Kk, 3, **dev)
+    ws = _ws(C.workspace_bytes(C.OP_STEP, B, P, Kk, 3), l1)
+    _noise_call("ups_step_encode_fwd_rows", noise, seed, seed_value, l1.data_ptr(), K, img.data_ptr(), m1.data_ptr(),
+                parts.data_ptr(), pooled.data_ptr(), B, P, Kk, K, ws.data_ptr(), ws.numel(), sample_offset, noise_level, st)
+    return m1[..., :K], parts, pooled[:, :K]
+
+
+def _part_encode_fake(l1, image1, noise, seed, seed_value, noise_level, sample_offset):
+    B, H, W, K = l1.shape
+    route, Kk = kernel_route(K, None, H * W)
+    return (_padded_fake(l1.shape, K, Kk, l1), l1.new_empty(K * B, H, W, 3), l1.new_empty(B, Kk, 3)[:, :K])
+
+
+def _part_encode_grad(g_parts: Tensor, g_pooled: Optional[Tensor], g_m1: Optional[Tensor], m1: Tensor, image1: Tensor,
+                      want_dimg: bool) -> Tuple[Tensor, Tensor]:
+    g_parts, img = _f32(g_parts, "g_parts"), _f32(image1, "image1")
+    g_pooled = None if g_pooled is None else _f32(g_pooled, "g_pooled")
+    g_m1 = None if g_m1 is None else _f32(g_m1, "g_m1")
+    B, H, W, K = m1.shape
+    P = H * W
+    st = _stream(img)
+    route, Kk = kernel_route(K, None, P)
+    dimg = torch.empty(B, H, W, 3, dtype=torch.float32, device=img.device) if want_dimg else img.new_empty(0)
+    if route == "generic":
+        m1 = _f32(m1, "m1")
+        hard = _hard_of(m1, st)
+        dm, dl1 = torch.empty_like(m1), torch.empty_like(m1)
+        C.call("ups_mask_parts_bwd", g_parts.data_ptr(), img.data_ptr(), hard.data_ptr(), _ptr(dimg) if want_dimg else None,
+               dm.data_ptr(), B, P, K, 3, 1, st)
+        dm2 = None
+        if g_pooled is not None:
+            dm2 = torch.empty_like(m1)
+            dfm = torch.empty_like(dimg) if want_dimg else None
+            C.call("ups_part_pool_bwd", g_pooled.data_ptr(), img.data_ptr(), hard.data_ptr(), _ptr(dfm), dm2.data_ptr(),
+                   B, P, K, 3, 0, 1.0 / P, st)
+            if want_dimg:
+                C.call("ups_axpy", dfm.data_ptr(), dimg.data_ptr(), dimg.numel(), 1.0, st)
+        C.call("ups_part_softmax_bwd2", m1.data_ptr(), dm.data_ptr(), _ptr(dm2), _ptr(g_m1), dl1.data_ptr(), B * P, K, st)
+        return dl1, dimg
+    m1p = _pitched(m1, Kk, st)
+    if g_pooled is not None and Kk != K:
+        g_pooled = _pad_rows(g_pooled.reshape(B, K * 3), K * 3, Kk * 3, st)
+    dl1 = torch.empty(B, H, W, Kk, dtype=torch.float32, device=img.device)
+    C.call("ups_step_encode_bwd_rows", g_parts.data_ptr(), _ptr(g_pooled), img.data_ptr(), m1p.data_ptr(), _ptr(g_m1), K,
+           dl1.data_ptr(), _ptr(dimg) if want_dimg else None, B, P, Kk, K, st)
+    return dl1[..., :K], dimg
+
+
+def _part_encode_grad_fake(g_parts, g_pooled, g_m1, m1, image1, want_dimg):
+    B, H, W, K = m1.shape
+    route, Kk = kernel_route(K, None, H * W)
+    return _padded_fake(m1.shape, K, Kk, m1), (m1.new_empty(B, H, W, 3) if want_dimg else m1.new_empty(0))
+
+
+part_encode_grad = _op("part_encode_grad", _part_encode_grad, _part_encode_grad_fake)
+
+
+def _part_encode_setup(ctx, inputs, output):
+    l1, image1 = inputs[0], inputs[1]
+    ctx.set_materialize_grads(False)
+    ctx.save_for_backward(output[0], image1)
+    ctx.parts_shape = tuple(output[1].shape)
+
+
+def _part_encode_bwd(ctx, g_m1, g_parts, g_pooled):
+    m1, image1 = ctx.saved_tensors
+    want_dimg = ctx.needs_input_grad[1]
+    if g_m1 is None and g_parts is None and g_pooled is None:
+        return (None,) * 7
+    if g_parts is None:
+        g_parts = m1.new_zeros(ctx.parts_shape)
+    dl1, dimg = part_encode_grad(g_parts, g_pooled, g_m1, m1, image1, want_dimg)
+    return dl1, (dimg if want_dimg else None), None, None, None, None, None
+
+
+part_encode = _op("part_encode", _part_encode, _part_encode_fake, _part_encode_bwd, _part_encode_setup)
+
+
+# ---- decode side: K3 forward, K4 backward
+def _part_decode(l0: Tensor, feat: Tensor, noise: int, seed: Optional[Tensor], seed_value: int, noise_level: float,
+                 sample_offset: int) -> Tuple[Tensor, Tensor, Tensor]:
+    l0, feat = _f32(l0, "logits0"), _f32(feat, "feature_vectors")
+    _check_noise(noise, seed, l0.device)
+    B, H, W, K = l0.shape
+    F = feat.shape[-1]
+    P = H * W
+    st = _stream(l0)
+    route, Kk = kernel_route(K, F, P)
+    dev = dict(dtype=torch.float32, device=l0.device)
+    labels = torch.empty(B, H, W, dtype=torch.int64, device=l0.device)
+    if route == "generic":
+        m0, hard = torch.empty_like(l0), torch.empty_like(l0)
+        inj = torch.empty(B, H, W, F + K, **dev)
+        _softmax_noise(l0, noise, seed, seed_value, 0, sample_offset * P, noise_level, m0, labels, hard, B * P, K, st)
+        C.call("ups_part_inject_fwd", feat.data_ptr(), hard.data_ptr(), inj.data_ptr(), B, P, K, F, st)
+        return m0, labels, inj
+    if Kk != K:
+        feat = _pad_rows(feat.reshape(B, K * F), K * F, Kk * F, st)
+    m0 = torch.empty(B, H, W, Kk, **dev)
+    inj = torch.empty(B, H, W, F + Kk, **dev)
+    _noise_call("ups_step_decode_fwd_rows", noise, seed, seed_value, l0.data_ptr(), K, feat.data_ptr(), m0.data_ptr(),
+                labels.data_ptr(), inj.data_ptr(), B, P, Kk, F, sample_offset, noise_level, st)
+    return m0[..., :K], labels, inj[..., :F + K]
+
+
+def _part_decode_fake(l0, feat, noise, seed, seed_value, noise_level, sample_offset):
+    B, H, W, K = l0.shape
+    F = feat.shape[-1]
+    route, Kk = kernel_route(K, F, H * W)
+    return (_padded_fake(l0.shape, K, Kk, l0), l0.new_empty(B, H, W, dtype=torch.int64),
+            _padded_fake((B, H, W, F + K), K, Kk, l0))
+
+
+def _part_decode_grad(g_inj: Tensor, g_m0: Optional[Tensor], m0: Tensor, feat: Tensor) -> Tuple[Tensor, Tensor]:
+    g_inj, feat = _f32(g_inj, "g_inj"), _f32(feat, "feature_vectors")
+    g_m0 = None if g_m0 is None else _f32(g_m0, "g_m0")
+    B, H, W, K = m0.shape
+    F = feat.shape[-1]
+    P = H * W
+    st = _stream(feat)
+    route, Kk = kernel_route(K, F, P)
+    if route == "generic":
+        m0 = _f32(m0, "m0")
+        hard = _hard_of(m0, st)
+        dm, dl0, dfeat = torch.empty_like(m0), torch.empty_like(m0), torch.empty_like(feat)
+        ws = _ws(C.workspace_bytes(C.OP_INJECT_BWD, B, P, K, F), feat)
+        C.call("ups_part_inject_bwd", g_inj.data_ptr(), feat.data_ptr(), hard.data_ptr(), dfeat.data_ptr(), dm.data_ptr(),
+               B, P, K, F, ws.data_ptr(), ws.numel(), st)
+        C.call("ups_part_softmax_bwd2", m0.data_ptr(), dm.data_ptr(), _ptr(g_m0), None, dl0.data_ptr(), B * P, K, st)
+        return dl0, dfeat
+    m0p = _pitched(m0, Kk, st)
+    if Kk != K:
+        g_inj = _pad_rows(g_inj, F + K, F + Kk, st)
+        feat = _pad_rows(feat.reshape(B, K * F), K * F, Kk * F, st)
+    dl0 = torch.empty(B, H, W, Kk, dtype=torch.float32, device=feat.device)
+    dfeat = torch.empty(B, Kk, F, dtype=torch.float32, device=feat.device)
+    ws = _ws(C.workspace_bytes(C.OP_STEP, B, P, Kk, F), feat)
+    C.call("ups_step_decode_bwd_tc_rows" if decode_bwd_tc_ok(Kk, F, P) else "ups_step_decode_bwd_rows",
+           g_inj.data_ptr(), m0p.data_ptr(), _ptr(g_m0), K, feat.data_ptr(), dl0.data_ptr(), dfeat.data_ptr(),
+           B, P, Kk, F, ws.data_ptr(), ws.numel(), st)
+    return dl0[..., :K], dfeat[:, :K]
+
+
+def _part_decode_grad_fake(g_inj, g_m0, m0, feat):
+    B, H, W, K = m0.shape
+    F = feat.shape[-1]
+    route, Kk = kernel_route(K, F, H * W)
+    return _padded_fake(m0.shape, K, Kk, m0), m0.new_empty(B, Kk, F)[:, :K]
+
+
+part_decode_grad = _op("part_decode_grad", _part_decode_grad, _part_decode_grad_fake)
+
+
+def _part_decode_setup(ctx, inputs, output):
+    ctx.set_materialize_grads(False)
+    ctx.save_for_backward(output[0], inputs[1])
+    ctx.inj_shape = tuple(output[2].shape)
+
+
+def _part_decode_bwd(ctx, g_m0, g_labels, g_inj):
+    m0, feat = ctx.saved_tensors
+    if g_m0 is None and g_inj is None:
+        return (None,) * 7
+    if g_inj is None:
+        g_inj = m0.new_zeros(ctx.inj_shape)
+    dl0, dfeat = part_decode_grad(g_inj, g_m0, m0, feat)
+    return dl0, dfeat, None, None, None, None, None
+
+
+part_decode = _op("part_decode", _part_decode, _part_decode_fake, _part_decode_bwd, _part_decode_setup)

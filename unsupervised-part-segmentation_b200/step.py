@@ -40,6 +40,28 @@ def _call_rows(name, noise, *args):
         C.call(name[:-len("_rows")] + "_noise", *args[:-1], *noise, args[-1])
 
 
+def kernel_route(K, F, P, first_conv=0, encoder_conv=0):
+    """The kernels that run a step side of K parts (F feature channels, None for the encode side, which has none) on
+    samples of P pixels: ("fused", K) for the fused kernels (K in {8,16,32}); ("padded", Kp) for a part count below 32
+    that is not a power of two, run on the fused kernels of the next power of two Kp with -inf logits in the padding
+    parts; ("generic", K) for everything else (the stand-alone softmax / mask_parts / pool / inject kernels).  The one
+    rule that PartStep and the ups::part_encode / ups::part_decode ops both follow.  UPS_PAD_K=0 keeps padded part
+    counts on the generic kernels."""
+    f_ok = F is None or F in (16, 32, 64)
+    if K in (8, 16, 32) and f_ok and P % 32 == 0:
+        return "fused", K
+    if (not first_conv and not encoder_conv and 1 <= K < 32 and f_ok and P % 32 == 0
+            and os.environ.get("UPS_PAD_K", "1") != "0"):
+        return "padded", 8 if K <= 8 else 16 if K <= 16 else 32
+    return "generic", K
+
+
+def decode_bwd_tc_ok(K, F, P):
+    """Whether K4 (the decode side's backward on the fused kernels) can run as the persistent TMA + tcgen05/TMEM
+    pipeline; otherwise it runs on the CUDA cores."""
+    return K in (16, 32) and F == 64 and P % 128 == 0
+
+
 def _on_device(fn):
     """Run a PartStep method with the step's device current: the C ABI launches on the device that is current on
     the calling thread, on the stream it is given, so both must be the device that owns the step's buffers."""
@@ -72,22 +94,22 @@ class PartStep:
             raise C.UpsError("PartStep needs a CUDA device: there is no CPU path")
         if self.device.index is None:
             self.device = torch.device("cuda", torch.cuda.current_device())
-        self.fused = K in (8, 16, 32) and F in (16, 32, 64) and self.P % 32 == 0
+        route, Kr = kernel_route(K, F, self.P, first_conv, encoder_conv)
+        self.fused = route == "fused"
         # A part count that is not a power of two (the reference ships n_parts = 25, train_cub_subset_tps.yaml:132) runs on
         # the fused kernels of the next power of two Kp: logits padded with -inf, everything else with zeros.  exp_canon
         # maps -inf to exactly 0 and the canonical K-way sum is a pair tree over the zero-padded terms, so
         # probabilities, masks and labels are bit-identical to the K-part evaluation; padding planes of the part images
-        # are neither written nor read (csrc: *_planes entry points).  UPS_PAD_K=0 keeps the generic kernels.
+        # are neither written nor read (csrc: *_planes entry points).
         self.Kp = 0
-        if (not self.fused and _planes is None and not first_conv and not encoder_conv and 1 <= K < 32 and F in (16, 32, 64)
-                and self.P % 32 == 0 and os.environ.get("UPS_PAD_K", "1") != "0"):
-            self.Kp = 8 if K <= 8 else 16 if K <= 16 else 32
+        if route == "padded" and _planes is None:
+            self.Kp = Kr
             self._inner = PartStep(B, S, self.Kp, F, n_views=V, use_tps=use_tps, views_grad=views_grad, device=self.device,
                                    decode_bwd=decode_bwd, sample_offset=sample_offset, _planes=K)
             self._init_padded()
             return
         # K4 variant: "tc" = persistent TMA + tcgen05/TMEM pipeline, "simt" = CUDA-core kernel
-        tc_ok = self.fused and K in (16, 32) and F == 64 and self.P % 128 == 0
+        tc_ok = self.fused and decode_bwd_tc_ok(K, F, self.P)
         assert decode_bwd in ("auto", "tc", "simt")
         if decode_bwd == "tc" and not tc_ok:
             raise C.UpsError("decode_bwd='tc' needs K in {16,32}, F == 64 and H*W % 128 == 0")
