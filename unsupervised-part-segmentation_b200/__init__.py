@@ -11,7 +11,7 @@ from .nn import (softmax, spatial_softmax, hard_max, straight_through_estimator,
                  probs_to_mu_sigma, mumford_shah, mumford_shah_sums, edge_set, MeanFieldDistribution, mask2rgb)
 from .model import (mask_parts, encode_parts, unpool_features, inject_features, make_tps,  # noqa: F401
                     categorical_kl, weak_cross_entropy, images_from_uint8, inject_conv2d, decode_conv2d,
-                    parts_conv2d)
+                    parts_conv2d, encode_conv2d)
 from .pooling import pool_features, pool_unpool_block, get_features, part_mean_pool  # noqa: F401
 from .tps import tps_parameters, make_input_tps_param, ThinPlateSpline  # noqa: F401
 

@@ -93,11 +93,21 @@ def inject_conv2d(feature_vectors, mask, V, b):
     return ops.inject_conv_apply(mask, G, b)
 
 
-def decode_conv2d(logits, feature_vectors, V, b):
+def _noise_args(noise_seed):
+    """noise_seed (None, an int in [0, 2**64) or a one-element int64 CUDA tensor) -> the ops' (noise, seed, seed_value)."""
+    if noise_seed is None:
+        return ops.NOISE_NONE, None, 0
+    if isinstance(noise_seed, torch.Tensor):
+        return ops.NOISE_DEVICE, noise_seed, 0
+    return ops.NOISE_INT, None, ops._seed_i64(noise_seed)
+
+
+def decode_conv2d(logits, feature_vectors, V, b, noise_seed=None, noise_level=1.0, sample_offset=0):
     """The decode side of the step with the first decoder layer folded in (model.py:426,434-436,447,470-473,482-485):
     m0 = softmax(logits); labels = argmax(m0); mask = ST(hard_max(m0)); h = inject_conv2d(feature_vectors, mask, V, b).
     Returns (m0, labels int64, mask, h); the backward runs the conv backward, the straight-through estimator and the
-    softmax backward in one kernel."""
+    softmax backward in one kernel.  noise_seed, noise_level, sample_offset as in part_decode (draw 0): logits are the
+    means and the softmax runs on the sample logits + noise_level * eps."""
     bs, h, w, n_parts = logits.shape
     fshape = list(feature_vectors.shape)
     assert len(fshape) == 3, fshape
@@ -106,16 +116,30 @@ def decode_conv2d(logits, feature_vectors, V, b):
     assert vshape[:3] == [3, 3, fshape[2] + n_parts], vshape
     assert list(b.shape) == [vshape[3]], b.shape
     G = ops.inject_conv_table(feature_vectors, V.reshape(9, vshape[2], vshape[3]))
-    return ops.decode_conv(logits, G, b)
-
-
-def _noise_args(noise_seed):
-    """noise_seed (None, an int in [0, 2**64) or a one-element int64 CUDA tensor) -> the ops' (noise, seed, seed_value)."""
     if noise_seed is None:
-        return ops.NOISE_NONE, None, 0
-    if isinstance(noise_seed, torch.Tensor):
-        return ops.NOISE_DEVICE, noise_seed, 0
-    return ops.NOISE_INT, None, ops._seed_i64(noise_seed)
+        return ops.decode_conv(logits, G, b)
+    noise, seed, seed_value = _noise_args(noise_seed)
+    return ops.decode_conv(logits, G, b, noise, seed, seed_value, float(noise_level), int(sample_offset))
+
+
+def encode_conv2d(logits1, image1, V, b, noise_seed=None, noise_level=1.0, sample_offset=0):
+    """The encode side of the step with the appearance encoder's first layer folded in (model.py:428-430,453-455,478 and
+    encoder_model's `nn.conv2d(x, config[0])`, model.py:40; cub/code/nn.py:617-664): m1 = softmax(logits1);
+    mask = ST(hard_max(m1)); e0 = parts_conv2d(image1, mask, V, b), without the part images.
+    logits1 [B,h,w,parts], image1 [B,h,w,3] (the warped view 1), V [3,3,3,Ce] (TensorFlow HWIO), b [Ce] -> (m1, mask,
+    e0 [parts*B,h,w,Ce] with row k*B+b, what the rest of `e_alpha` consumes inside apply_partwise).  Differentiable in
+    logits1, V and b: the backward runs the conv backward, the straight-through estimator and the softmax backward in
+    one call.  The image gets no gradient (the reference's inputs are placeholders): asking for one raises.
+    noise_seed, noise_level, sample_offset as in part_encode (draw 1)."""
+    bs, h, w, n_parts = logits1.shape
+    ishape = list(image1.shape)
+    assert ishape == [bs, h, w, 3], ishape
+    vshape = list(V.shape)
+    assert vshape[:3] == [3, 3, 3], vshape
+    assert list(b.shape) == [vshape[3]], b.shape
+    noise, seed, seed_value = _noise_args(noise_seed)
+    return ops.encode_conv(logits1, image1, V.reshape(9, 3, vshape[3]), b, noise, seed, seed_value, float(noise_level),
+                           int(sample_offset))
 
 
 def part_encode(logits1, image1, noise_seed=None, noise_level=1.0, sample_offset=0):

@@ -815,28 +815,6 @@ inject_conv_apply = _op("inject_conv_apply", _inject_conv_apply,
                         lambda ctx, inputs, output: ctx.save_for_backward(inputs[0], inputs[1]))
 
 
-def _decode_conv(logits: Tensor, G: Tensor, bias: Tensor) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
-    """softmax -> labels -> ST(hard_max) -> first decoder conv, the decode side of the step with the conv folded in."""
-    probs, labels, hard = _part_softmax_full(logits)
-    return probs, labels, hard, _inject_conv_apply(hard, G, bias)
-
-
-def _decode_conv_bwd(ctx, g_probs, g_labels, g_hard, g_out):
-    probs, hard, G = ctx.saved_tensors
-    g_extra = g_probs if g_hard is None else (g_hard if g_probs is None else g_probs + g_hard)
-    if g_out is None:
-        return (None if g_extra is None else part_softmax_grad(probs, g_extra)), None, None
-    dlogits, dG, db = inject_conv_apply_grad(g_out, hard, G, probs, g_extra)
-    return dlogits, dG, db
-
-
-decode_conv = _op(
-    "decode_conv", _decode_conv,
-    lambda x, G, b: (torch.empty_like(x), x.new_empty(x.shape[:-1], dtype=torch.int64), torch.empty_like(x),
-                     x.new_empty(*x.shape[:-1], G.shape[-1])),
-    _decode_conv_bwd, lambda ctx, inputs, output: ctx.save_for_backward(output[0], output[2], inputs[1]))
-
-
 # ------------------------------------------------------------------ encoder first conv on the masked part images (N4)
 def _parts_conv(image: Tensor, mask: Tensor, V: Tensor, bias: Tensor) -> Tensor:
     image, mask, V, bias = _f32(image, "image"), _f32(mask, "mask"), _f32(V, "V"), _f32(bias, "b")
@@ -1167,3 +1145,113 @@ def _part_decode_bwd(ctx, g_m0, g_labels, g_inj):
 
 
 part_decode = _op("part_decode", _part_decode, _part_decode_fake, _part_decode_bwd, _part_decode_setup)
+
+
+# ------------------------------------------------------------------ the two sides with their first convolutions folded in
+# (N4) in the reference model's order: encode_conv ends the encode side in e_alpha's first layer (e0, the part images are
+# never formed), decode_conv ends the decode side in dd's first layer (h0, from the table G = inject_conv_table(feat, V),
+# the injected map is never formed).  The softmax runs on the generic kernel with the step's draw (encode 1, decode 0),
+# as PartStep(first_conv=Co, encoder_conv=Ce) does, so both produce the same bits.  Outputs and workspaces are fresh on
+# every call.  The backward of the sample with respect to the mean is the identity: the backwards ignore the noise.
+def _decode_conv(logits: Tensor, G: Tensor, bias: Tensor, noise: int = NOISE_NONE, seed: Optional[Tensor] = None,
+                 seed_value: int = 0, noise_level: float = 1.0,
+                 sample_offset: int = 0) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+    """softmax -> labels -> ST(hard_max) -> first decoder conv, the decode side of the step with the conv folded in."""
+    x = _f32(logits, "logits")
+    _check_noise(noise, seed, x.device)
+    B, H, W, K = x.shape
+    probs, hard = torch.empty_like(x), torch.empty_like(x)
+    labels = torch.empty(x.shape[:-1], dtype=torch.int64, device=x.device)
+    _softmax_noise(x, noise, seed, seed_value, 0, sample_offset * H * W, noise_level, probs, labels, hard, B * H * W, K,
+                   _stream(x))
+    return probs, labels, hard, _inject_conv_apply(hard, G, bias)
+
+
+def _decode_conv_bwd(ctx, g_probs, g_labels, g_hard, g_out):
+    probs, hard, G = ctx.saved_tensors
+    g_extra = g_probs if g_hard is None else (g_hard if g_probs is None else g_probs + g_hard)
+    if g_out is None:
+        return (None if g_extra is None else part_softmax_grad(probs, g_extra)), None, None, None, None, None, None, None
+    dlogits, dG, db = inject_conv_apply_grad(g_out, hard, G, probs, g_extra)
+    return dlogits, dG, db, None, None, None, None, None
+
+
+def _decode_conv_setup(ctx, inputs, output):
+    # an output the loss does not use gets no cotangent (not a zero tensor that the backward would add to g_probs)
+    ctx.set_materialize_grads(False)
+    ctx.save_for_backward(output[0], output[2], inputs[1])
+
+
+decode_conv = _op(
+    "decode_conv", _decode_conv,
+    lambda x, G, b, noise=0, seed=None, seed_value=0, noise_level=1.0, sample_offset=0: (
+        torch.empty_like(x), x.new_empty(x.shape[:-1], dtype=torch.int64), torch.empty_like(x),
+        x.new_empty(*x.shape[:-1], G.shape[-1])),
+    _decode_conv_bwd, _decode_conv_setup)
+
+
+def _encode_conv(l1: Tensor, image1: Tensor, V: Tensor, bias: Tensor, noise: int, seed: Optional[Tensor],
+                 seed_value: int, noise_level: float, sample_offset: int) -> Tuple[Tensor, Tensor, Tensor]:
+    """softmax -> ST(hard_max) -> first encoder conv on the masked part images, the encode side with the conv folded in.
+    V [9,3,Ce] -> (m1, mask1, e0 [K*B,H,W,Ce] part-major)."""
+    l1, img = _f32(l1, "logits1"), _f32(image1, "image1")
+    V, bias = _f32(V, "V"), _f32(bias, "b")
+    _check_noise(noise, seed, l1.device)
+    B, H, W, K = l1.shape
+    Co = V.shape[-1]
+    st = _stream(l1)
+    m1, hard = torch.empty_like(l1), torch.empty_like(l1)
+    e0 = torch.empty(K * B, H, W, Co, dtype=torch.float32, device=l1.device)
+    _softmax_noise(l1, noise, seed, seed_value, 1, sample_offset * H * W, noise_level, m1, None, hard, B * H * W, K, st)
+    C.call("ups_parts_conv_fwd", img.data_ptr(), hard.data_ptr(), V.data_ptr(), bias.data_ptr(), e0.data_ptr(),
+           B, H, W, K, img.shape[-1], Co, st)
+    return m1, hard, e0
+
+
+def _encode_conv_fake(l1, image1, V, bias, noise, seed, seed_value, noise_level, sample_offset):
+    B, H, W, K = l1.shape
+    return torch.empty_like(l1), torch.empty_like(l1), l1.new_empty(K * B, H, W, V.shape[-1])
+
+
+def _encode_conv_grad(g_e0: Tensor, g_extra: Optional[Tensor], image1: Tensor, hard: Tensor, V: Tensor,
+                      m1: Tensor) -> Tuple[Tensor, Tensor, Tensor]:
+    """One ups_parts_conv_bwd: the conv backward, then (+ g_extra) the straight-through estimator and the softmax
+    backward -> (dl1, dV [9,3,Ce], db [Ce])."""
+    g_e0, img, hard, V, m1 = _f32(g_e0, "g_e0"), _f32(image1, "image1"), _f32(hard), _f32(V), _f32(m1)
+    g_extra = None if g_extra is None else _f32(g_extra, "g_extra")
+    B, H, W, K = m1.shape
+    Co = V.shape[-1]
+    dl1, dV = torch.empty_like(m1), torch.empty_like(V)
+    db = torch.empty(Co, dtype=torch.float32, device=m1.device)
+    ws = _ws(C.parts_conv_bwd_workspace_bytes(B, H, W, K, Co), m1)
+    C.call("ups_parts_conv_bwd", g_e0.data_ptr(), img.data_ptr(), hard.data_ptr(), V.data_ptr(), m1.data_ptr(),
+           _ptr(g_extra), dl1.data_ptr(), dV.data_ptr(), db.data_ptr(), B, H, W, K, img.shape[-1], Co, ws.data_ptr(),
+           ws.numel(), _stream(g_e0))
+    return dl1, dV, db
+
+
+encode_conv_grad = _op("encode_conv_grad", _encode_conv_grad,
+                       lambda g, e, i, h, v, m: (torch.empty_like(m), torch.empty_like(v), v.new_empty(v.shape[-1])))
+
+
+def _encode_conv_setup(ctx, inputs, output):
+    ctx.set_materialize_grads(False)
+    ctx.save_for_backward(output[0], output[1], inputs[1], inputs[2])
+    ctx.e0_shape = tuple(output[2].shape)
+
+
+def _encode_conv_bwd(ctx, g_m1, g_mask1, g_e0):
+    if ctx.needs_input_grad[1]:
+        raise C.UpsError("ups::encode_conv: no gradient with respect to the image (the reference's inputs are "
+                         "placeholders)")
+    m1, hard, image1, V = ctx.saved_tensors
+    g_extra = g_m1 if g_mask1 is None else (g_mask1 if g_m1 is None else g_m1 + g_mask1)
+    if g_extra is None and g_e0 is None:
+        return (None,) * 9
+    if g_e0 is None:
+        g_e0 = m1.new_zeros(ctx.e0_shape)
+    dl1, dV, db = encode_conv_grad(g_e0, g_extra, image1, hard, V, m1)
+    return dl1, None, dV, db, None, None, None, None, None
+
+
+encode_conv = _op("encode_conv", _encode_conv, _encode_conv_fake, _encode_conv_bwd, _encode_conv_setup)
