@@ -11,7 +11,9 @@ import torch
 from torch import Tensor
 
 from . import _cabi as C
-from .step import decode_bwd_tc_ok, kernel_route
+from .step import (_ptr, _seed_i64, decode_bwd, decode_bwd_tc_ok, decode_fwd, encode_bwd, encode_fwd, inject_conv_bwd,
+                   inject_conv_fwd, inject_conv_table_bwd, inject_conv_table_fwd, kernel_route, part_softmax_fwd,
+                   parts_conv_bwd, parts_conv_fwd)
 
 
 def _stream(t: Tensor):
@@ -26,10 +28,6 @@ def _f32(t: Tensor, name="tensor") -> Tensor:
     if t.dtype != torch.float32:
         raise C.UpsError(f"ups_b200: {name} must be float32, got {t.dtype}")
     return t.contiguous()
-
-
-def _ptr(t: Optional[Tensor]):
-    return None if t is None else t.data_ptr()
 
 
 def _ws(nbytes: int, like: Tensor) -> Tensor:
@@ -670,14 +668,7 @@ part_softmax_sampled = _op(
 # ------------------------------------------------------------------ the logit noise drawn on the device
 # The draw is a pure function of (seed, draw, global pixel, part) (csrc/canon_math.cuh): ups_normal_philox_fwd writes it,
 # ups_part_softmax_sampled_philox_fwd and the step's `_noise` kernels generate the same values in registers.  Seeds are
-# unsigned 64-bit; the op schemas carry them as the int64 with the same bits.
-def _seed_i64(seed: int) -> int:
-    seed = int(seed)
-    if not 0 <= seed < 2 ** 64:
-        raise ValueError(f"seed must be in [0, 2**64), got {seed}")
-    return seed - 2 ** 64 if seed >= 2 ** 63 else seed
-
-
+# unsigned 64-bit; the op schemas carry them as the int64 with the same bits (step._seed_i64).
 def _normal_philox(seed: int, draw: int, pix_offset: int, n_pix: int, K: int, device: torch.device) -> Tensor:
     out = torch.empty(n_pix, K, dtype=torch.float32, device=device)
     if not out.is_cuda:
@@ -756,20 +747,15 @@ mask2rgb = _op("mask2rgb", _mask2rgb, lambda m, t, h: m.new_empty(*m.shape[:-1],
 # ------------------------------------------------------------------ decoder first conv on the part assignment (N4)
 def _inject_conv_table(feat: Tensor, V: Tensor) -> Tensor:
     feat, V = _f32(feat, "feature_vectors"), _f32(V, "V")
-    B, K, F = feat.shape
-    Co = V.shape[-1]
-    G = torch.empty(B, 9, K, Co, dtype=torch.float32, device=feat.device)
-    C.call("ups_inject_conv_table_fwd", feat.data_ptr(), V.data_ptr(), G.data_ptr(), B, K, F, Co, _stream(feat))
+    G = torch.empty(feat.shape[0], 9, feat.shape[1], V.shape[-1], dtype=torch.float32, device=feat.device)
+    inject_conv_table_fwd(feat, V, G, _stream(feat))
     return G
 
 
 def _inject_conv_table_grad(dG: Tensor, feat: Tensor, V: Tensor) -> Tuple[Tensor, Tensor]:
     dG, feat, V = _f32(dG), _f32(feat), _f32(V)
-    B, K, F = feat.shape
-    Co = V.shape[-1]
     dfeat, dV = torch.empty_like(feat), torch.empty_like(V)
-    C.call("ups_inject_conv_table_bwd", dG.data_ptr(), feat.data_ptr(), V.data_ptr(), dfeat.data_ptr(), dV.data_ptr(),
-           B, K, F, Co, _stream(dG))
+    inject_conv_table_bwd(dG, feat, V, dfeat, dV, _stream(dG))
     return dfeat, dV
 
 
@@ -783,11 +769,8 @@ inject_conv_table = _op("inject_conv_table", _inject_conv_table,
 
 def _inject_conv_apply(mask: Tensor, G: Tensor, bias: Tensor) -> Tensor:
     mask, G, bias = _f32(mask, "mask"), _f32(G, "G"), _f32(bias, "b")
-    B, H, W, K = mask.shape
-    Co = G.shape[-1]
-    out = torch.empty(B, H, W, Co, dtype=torch.float32, device=mask.device)
-    C.call("ups_inject_conv_fwd", mask.data_ptr(), G.data_ptr(), bias.data_ptr(), out.data_ptr(), B, H, W, K, Co,
-           _stream(mask))
+    out = torch.empty(*mask.shape[:-1], G.shape[-1], dtype=torch.float32, device=mask.device)
+    inject_conv_fwd(mask, G, bias, out, _stream(mask))
     return out
 
 
@@ -801,8 +784,7 @@ def _inject_conv_apply_grad(g_out: Tensor, mask: Tensor, G: Tensor, probs: Optio
     dmask, dG = torch.empty_like(mask), torch.empty_like(G)
     db = torch.empty(Co, dtype=torch.float32, device=mask.device)
     ws = _ws(C.inject_conv_workspace_bytes(B, H, W, K, Co), mask)
-    C.call("ups_inject_conv_bwd", g_out.data_ptr(), mask.data_ptr(), G.data_ptr(), _ptr(probs), _ptr(g_extra),
-           dmask.data_ptr(), dG.data_ptr(), db.data_ptr(), B, H, W, K, Co, ws.data_ptr(), ws.numel(), _stream(g_out))
+    inject_conv_bwd(g_out, mask, G, probs, g_extra, dmask, dG, db, ws, _stream(g_out))
     return dmask, dG, db
 
 
@@ -819,22 +801,25 @@ inject_conv_apply = _op("inject_conv_apply", _inject_conv_apply,
 def _parts_conv(image: Tensor, mask: Tensor, V: Tensor, bias: Tensor) -> Tensor:
     image, mask, V, bias = _f32(image, "image"), _f32(mask, "mask"), _f32(V, "V"), _f32(bias, "b")
     B, H, W, K = mask.shape
-    Cin, Co = image.shape[-1], V.shape[-1]
-    out = torch.empty(K * B, H, W, Co, dtype=torch.float32, device=image.device)
-    C.call("ups_parts_conv_fwd", image.data_ptr(), mask.data_ptr(), V.data_ptr(), bias.data_ptr(), out.data_ptr(),
-           B, H, W, K, Cin, Co, _stream(image))
+    out = torch.empty(K * B, H, W, V.shape[-1], dtype=torch.float32, device=image.device)
+    parts_conv_fwd(image, mask, V, bias, out, _stream(image))
     return out
 
 
 def _parts_conv_grad(g_out: Tensor, image: Tensor, mask: Tensor, V: Tensor) -> Tuple[Tensor, Tensor, Tensor]:
+    return _parts_conv_backward(g_out, image, mask, V, None, None)
+
+
+def _parts_conv_backward(g_out, image, mask, V, probs, g_extra):
+    """One ups_parts_conv_bwd on fresh outputs: the conv backward -> (dmask, dV, db); given probs, (+ g_extra) the
+    straight-through estimator and the softmax backward as well -> (dlogits, dV, db)."""
     g_out, image, mask, V = _f32(g_out), _f32(image), _f32(mask), _f32(V)
     B, H, W, K = mask.shape
-    Cin, Co = image.shape[-1], V.shape[-1]
+    Co = V.shape[-1]
     dmask, dV = torch.empty_like(mask), torch.empty_like(V)
     db = torch.empty(Co, dtype=torch.float32, device=mask.device)
     ws = _ws(C.parts_conv_bwd_workspace_bytes(B, H, W, K, Co), mask)
-    C.call("ups_parts_conv_bwd", g_out.data_ptr(), image.data_ptr(), mask.data_ptr(), V.data_ptr(), None, None,
-           dmask.data_ptr(), dV.data_ptr(), db.data_ptr(), B, H, W, K, Cin, Co, ws.data_ptr(), ws.numel(), _stream(g_out))
+    parts_conv_bwd(g_out, image, mask, V, probs, g_extra, dmask, dV, db, ws, _stream(g_out))
     return dmask, dV, db
 
 
@@ -882,31 +867,9 @@ draw_rect = _op("draw_rect", _draw_rect, lambda c, ph, pw, H, W: c.new_empty(c.s
 NOISE_NONE, NOISE_INT, NOISE_DEVICE = 0, 1, 2
 
 
-def _noise_call(name, noise, seed, seed_value, *args):
-    """Call entry point `name` noise-free, or its `_noise` / `_noise_dseed` form: the same arguments with
-    (seed, sample_offset, noise_level) inserted before the stream (`args` ends with those three and the stream)."""
-    *head, offset, level, st = args
-    if noise == NOISE_NONE:
-        C.call(name, *head, st)
-    elif noise == NOISE_INT:
-        C.call(name[:-len("_rows")] + "_noise", *head, seed_value % 2 ** 64, offset, level, st)
-    else:
-        C.call(name[:-len("_rows")] + "_noise_dseed", *head, seed.data_ptr(), offset, level, st)
-
-
-def _softmax_noise(logits, noise, seed, seed_value, draw, pix_offset, level, probs, labels, hard, n_pix, K, st):
-    """The generic kernels' softmax of the logits, or of the sampled logits (the step's draw `draw`)."""
-    if noise == NOISE_NONE:
-        C.call("ups_part_softmax_fwd", logits.data_ptr(), probs.data_ptr(), _ptr(labels), _ptr(hard), n_pix, K, st)
-    elif noise == NOISE_INT:
-        C.call("ups_part_softmax_sampled_philox_fwd", logits.data_ptr(), seed_value % 2 ** 64, draw, pix_offset, level,
-               None, probs.data_ptr(), _ptr(labels), _ptr(hard), n_pix, K, st)
-    else:
-        C.call("ups_part_softmax_sampled_philox_fwd_dseed", logits.data_ptr(), seed.data_ptr(), draw, pix_offset, level,
-               None, probs.data_ptr(), _ptr(labels), _ptr(hard), n_pix, K, st)
-
-
-def _check_noise(noise: int, seed: Optional[Tensor], device):
+def _check_noise(noise: int, seed: Optional[Tensor], seed_value: int, noise_level: float, sample_offset: int, device):
+    """The noise arguments, checked, as the step launchers' noise value (step.py): None or (seed, sample_offset,
+    noise_level), the seed an int or the device tensor."""
     if noise == NOISE_INT and torch.cuda.is_current_stream_capturing():
         raise C.UpsError("ups_b200: an int noise_seed is frozen into a captured CUDA graph (every replay would draw the "
                          "same noise); pass the seed as a one-element int64 CUDA tensor")
@@ -915,6 +878,7 @@ def _check_noise(noise: int, seed: Optional[Tensor], device):
             raise C.UpsError("ups_b200: a device noise_seed is a one-element int64 tensor on the logits' device")
         if not seed.is_contiguous():
             raise C.UpsError("ups_b200: the device noise_seed must be contiguous")
+    return None if noise == NOISE_NONE else (seed_value if noise == NOISE_INT else seed, sample_offset, noise_level)
 
 
 def _pitched(t: Tensor, Kp: int, st) -> Tensor:
@@ -958,27 +922,16 @@ def _padded_fake(shape, K, Kp, like):
 def _part_encode(l1: Tensor, image1: Tensor, noise: int, seed: Optional[Tensor], seed_value: int, noise_level: float,
                  sample_offset: int) -> Tuple[Tensor, Tensor, Tensor]:
     l1, img = _f32(l1, "logits1"), _f32(image1, "image1")
-    _check_noise(noise, seed, l1.device)
+    nz = _check_noise(noise, seed, seed_value, noise_level, sample_offset, l1.device)
     B, H, W, K = l1.shape
     P = H * W
-    st = _stream(l1)
     route, Kk = kernel_route(K, None, P)
     dev = dict(dtype=torch.float32, device=l1.device)
     parts = torch.empty(K * B, H, W, 3, **dev)
-    if route == "generic":
-        m1, hard = torch.empty_like(l1), torch.empty_like(l1)
-        pooled = torch.empty(B, K, 3, **dev)
-        _softmax_noise(l1, noise, seed, seed_value, 1, sample_offset * P, noise_level, m1, None, hard, B * P, K, st)
-        C.call("ups_mask_parts_fwd", img.data_ptr(), hard.data_ptr(), parts.data_ptr(), B, P, K, 3, 1, st)
-        ws = _ws(C.workspace_bytes(C.OP_POOL, B, P, K, 3), l1)
-        C.call("ups_part_pool_fwd", img.data_ptr(), hard.data_ptr(), pooled.data_ptr(), B, P, K, 3, 0, 1.0 / P,
-               ws.data_ptr(), ws.numel(), st)
-        return m1, parts, pooled
-    m1 = torch.empty(B, H, W, Kk, **dev)
-    pooled = torch.empty(B, Kk, 3, **dev)
-    ws = _ws(C.workspace_bytes(C.OP_STEP, B, P, Kk, 3), l1)
-    _noise_call("ups_step_encode_fwd_rows", noise, seed, seed_value, l1.data_ptr(), K, img.data_ptr(), m1.data_ptr(),
-                parts.data_ptr(), pooled.data_ptr(), B, P, Kk, K, ws.data_ptr(), ws.numel(), sample_offset, noise_level, st)
+    m1, pooled = torch.empty(B, H, W, Kk, **dev), torch.empty(B, Kk, 3, **dev)
+    hard = torch.empty_like(l1) if route == "generic" else None
+    ws = _ws(C.workspace_bytes(C.OP_POOL if route == "generic" else C.OP_STEP, B, P, Kk, 3), l1)
+    encode_fwd(route, nz, l1, img, m1, parts, pooled, hard, ws, B, P, Kk, K, K, _stream(l1))
     return m1[..., :K], parts, pooled[:, :K]
 
 
@@ -998,28 +951,21 @@ def _part_encode_grad(g_parts: Tensor, g_pooled: Optional[Tensor], g_m1: Optiona
     st = _stream(img)
     route, Kk = kernel_route(K, None, P)
     dimg = torch.empty(B, H, W, 3, dtype=torch.float32, device=img.device) if want_dimg else img.new_empty(0)
+    hard = dm = dm2 = dfm = None
     if route == "generic":
         m1 = _f32(m1, "m1")
         hard = _hard_of(m1, st)
-        dm, dl1 = torch.empty_like(m1), torch.empty_like(m1)
-        C.call("ups_mask_parts_bwd", g_parts.data_ptr(), img.data_ptr(), hard.data_ptr(), _ptr(dimg) if want_dimg else None,
-               dm.data_ptr(), B, P, K, 3, 1, st)
-        dm2 = None
+        dm = torch.empty_like(m1)
         if g_pooled is not None:
             dm2 = torch.empty_like(m1)
             dfm = torch.empty_like(dimg) if want_dimg else None
-            C.call("ups_part_pool_bwd", g_pooled.data_ptr(), img.data_ptr(), hard.data_ptr(), _ptr(dfm), dm2.data_ptr(),
-                   B, P, K, 3, 0, 1.0 / P, st)
-            if want_dimg:
-                C.call("ups_axpy", dfm.data_ptr(), dimg.data_ptr(), dimg.numel(), 1.0, st)
-        C.call("ups_part_softmax_bwd2", m1.data_ptr(), dm.data_ptr(), _ptr(dm2), _ptr(g_m1), dl1.data_ptr(), B * P, K, st)
-        return dl1, dimg
-    m1p = _pitched(m1, Kk, st)
-    if g_pooled is not None and Kk != K:
-        g_pooled = _pad_rows(g_pooled.reshape(B, K * 3), K * 3, Kk * 3, st)
+    else:
+        m1 = _pitched(m1, Kk, st)
+        if g_pooled is not None and Kk != K:
+            g_pooled = _pad_rows(g_pooled.reshape(B, K * 3), K * 3, Kk * 3, st)
     dl1 = torch.empty(B, H, W, Kk, dtype=torch.float32, device=img.device)
-    C.call("ups_step_encode_bwd_rows", g_parts.data_ptr(), _ptr(g_pooled), img.data_ptr(), m1p.data_ptr(), _ptr(g_m1), K,
-           dl1.data_ptr(), _ptr(dimg) if want_dimg else None, B, P, Kk, K, st)
+    encode_bwd(route, g_parts, g_pooled, g_m1, img, m1, hard, dl1, dimg if want_dimg else None, dm, dm2, dfm, B, P, Kk, K,
+               K, st)
     return dl1[..., :K], dimg
 
 
@@ -1057,7 +1003,7 @@ part_encode = _op("part_encode", _part_encode, _part_encode_fake, _part_encode_b
 def _part_decode(l0: Tensor, feat: Tensor, noise: int, seed: Optional[Tensor], seed_value: int, noise_level: float,
                  sample_offset: int) -> Tuple[Tensor, Tensor, Tensor]:
     l0, feat = _f32(l0, "logits0"), _f32(feat, "feature_vectors")
-    _check_noise(noise, seed, l0.device)
+    nz = _check_noise(noise, seed, seed_value, noise_level, sample_offset, l0.device)
     B, H, W, K = l0.shape
     F = feat.shape[-1]
     P = H * W
@@ -1065,18 +1011,11 @@ def _part_decode(l0: Tensor, feat: Tensor, noise: int, seed: Optional[Tensor], s
     route, Kk = kernel_route(K, F, P)
     dev = dict(dtype=torch.float32, device=l0.device)
     labels = torch.empty(B, H, W, dtype=torch.int64, device=l0.device)
-    if route == "generic":
-        m0, hard = torch.empty_like(l0), torch.empty_like(l0)
-        inj = torch.empty(B, H, W, F + K, **dev)
-        _softmax_noise(l0, noise, seed, seed_value, 0, sample_offset * P, noise_level, m0, labels, hard, B * P, K, st)
-        C.call("ups_part_inject_fwd", feat.data_ptr(), hard.data_ptr(), inj.data_ptr(), B, P, K, F, st)
-        return m0, labels, inj
     if Kk != K:
         feat = _pad_rows(feat.reshape(B, K * F), K * F, Kk * F, st)
-    m0 = torch.empty(B, H, W, Kk, **dev)
-    inj = torch.empty(B, H, W, F + Kk, **dev)
-    _noise_call("ups_step_decode_fwd_rows", noise, seed, seed_value, l0.data_ptr(), K, feat.data_ptr(), m0.data_ptr(),
-                labels.data_ptr(), inj.data_ptr(), B, P, Kk, F, sample_offset, noise_level, st)
+    m0, inj = torch.empty(B, H, W, Kk, **dev), torch.empty(B, H, W, F + Kk, **dev)
+    hard = torch.empty_like(l0) if route == "generic" else None
+    decode_fwd(route, nz, l0, feat, m0, labels, inj, hard, B, P, Kk, F, K, st)
     return m0[..., :K], labels, inj[..., :F + K]
 
 
@@ -1096,25 +1035,20 @@ def _part_decode_grad(g_inj: Tensor, g_m0: Optional[Tensor], m0: Tensor, feat: T
     P = H * W
     st = _stream(feat)
     route, Kk = kernel_route(K, F, P)
+    hard = dm = None
     if route == "generic":
         m0 = _f32(m0, "m0")
-        hard = _hard_of(m0, st)
-        dm, dl0, dfeat = torch.empty_like(m0), torch.empty_like(m0), torch.empty_like(feat)
+        hard, dm = _hard_of(m0, st), torch.empty_like(m0)
         ws = _ws(C.workspace_bytes(C.OP_INJECT_BWD, B, P, K, F), feat)
-        C.call("ups_part_inject_bwd", g_inj.data_ptr(), feat.data_ptr(), hard.data_ptr(), dfeat.data_ptr(), dm.data_ptr(),
-               B, P, K, F, ws.data_ptr(), ws.numel(), st)
-        C.call("ups_part_softmax_bwd2", m0.data_ptr(), dm.data_ptr(), _ptr(g_m0), None, dl0.data_ptr(), B * P, K, st)
-        return dl0, dfeat
-    m0p = _pitched(m0, Kk, st)
-    if Kk != K:
-        g_inj = _pad_rows(g_inj, F + K, F + Kk, st)
-        feat = _pad_rows(feat.reshape(B, K * F), K * F, Kk * F, st)
+    else:
+        m0 = _pitched(m0, Kk, st)
+        if Kk != K:
+            g_inj = _pad_rows(g_inj, F + K, F + Kk, st)
+            feat = _pad_rows(feat.reshape(B, K * F), K * F, Kk * F, st)
+        ws = _ws(C.workspace_bytes(C.OP_STEP, B, P, Kk, F), feat)
     dl0 = torch.empty(B, H, W, Kk, dtype=torch.float32, device=feat.device)
     dfeat = torch.empty(B, Kk, F, dtype=torch.float32, device=feat.device)
-    ws = _ws(C.workspace_bytes(C.OP_STEP, B, P, Kk, F), feat)
-    C.call("ups_step_decode_bwd_tc_rows" if decode_bwd_tc_ok(Kk, F, P) else "ups_step_decode_bwd_rows",
-           g_inj.data_ptr(), m0p.data_ptr(), _ptr(g_m0), K, feat.data_ptr(), dl0.data_ptr(), dfeat.data_ptr(),
-           B, P, Kk, F, ws.data_ptr(), ws.numel(), st)
+    decode_bwd(route, decode_bwd_tc_ok(Kk, F, P), g_inj, g_m0, m0, hard, feat, dl0, dfeat, dm, ws, B, P, Kk, F, K, st)
     return dl0[..., :K], dfeat[:, :K]
 
 
@@ -1158,12 +1092,11 @@ def _decode_conv(logits: Tensor, G: Tensor, bias: Tensor, noise: int = NOISE_NON
                  sample_offset: int = 0) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
     """softmax -> labels -> ST(hard_max) -> first decoder conv, the decode side of the step with the conv folded in."""
     x = _f32(logits, "logits")
-    _check_noise(noise, seed, x.device)
+    nz = _check_noise(noise, seed, seed_value, noise_level, sample_offset, x.device)
     B, H, W, K = x.shape
     probs, hard = torch.empty_like(x), torch.empty_like(x)
     labels = torch.empty(x.shape[:-1], dtype=torch.int64, device=x.device)
-    _softmax_noise(x, noise, seed, seed_value, 0, sample_offset * H * W, noise_level, probs, labels, hard, B * H * W, K,
-                   _stream(x))
+    part_softmax_fwd(nz, 0, x, probs, labels, hard, B, H * W, K, _stream(x))
     return probs, labels, hard, _inject_conv_apply(hard, G, bias)
 
 
@@ -1196,16 +1129,11 @@ def _encode_conv(l1: Tensor, image1: Tensor, V: Tensor, bias: Tensor, noise: int
     V [9,3,Ce] -> (m1, mask1, e0 [K*B,H,W,Ce] part-major)."""
     l1, img = _f32(l1, "logits1"), _f32(image1, "image1")
     V, bias = _f32(V, "V"), _f32(bias, "b")
-    _check_noise(noise, seed, l1.device)
+    nz = _check_noise(noise, seed, seed_value, noise_level, sample_offset, l1.device)
     B, H, W, K = l1.shape
-    Co = V.shape[-1]
-    st = _stream(l1)
     m1, hard = torch.empty_like(l1), torch.empty_like(l1)
-    e0 = torch.empty(K * B, H, W, Co, dtype=torch.float32, device=l1.device)
-    _softmax_noise(l1, noise, seed, seed_value, 1, sample_offset * H * W, noise_level, m1, None, hard, B * H * W, K, st)
-    C.call("ups_parts_conv_fwd", img.data_ptr(), hard.data_ptr(), V.data_ptr(), bias.data_ptr(), e0.data_ptr(),
-           B, H, W, K, img.shape[-1], Co, st)
-    return m1, hard, e0
+    part_softmax_fwd(nz, 1, l1, m1, None, hard, B, H * W, K, _stream(l1))
+    return m1, hard, _parts_conv(img, hard, V, bias)
 
 
 def _encode_conv_fake(l1, image1, V, bias, noise, seed, seed_value, noise_level, sample_offset):
@@ -1217,17 +1145,8 @@ def _encode_conv_grad(g_e0: Tensor, g_extra: Optional[Tensor], image1: Tensor, h
                       m1: Tensor) -> Tuple[Tensor, Tensor, Tensor]:
     """One ups_parts_conv_bwd: the conv backward, then (+ g_extra) the straight-through estimator and the softmax
     backward -> (dl1, dV [9,3,Ce], db [Ce])."""
-    g_e0, img, hard, V, m1 = _f32(g_e0, "g_e0"), _f32(image1, "image1"), _f32(hard), _f32(V), _f32(m1)
     g_extra = None if g_extra is None else _f32(g_extra, "g_extra")
-    B, H, W, K = m1.shape
-    Co = V.shape[-1]
-    dl1, dV = torch.empty_like(m1), torch.empty_like(V)
-    db = torch.empty(Co, dtype=torch.float32, device=m1.device)
-    ws = _ws(C.parts_conv_bwd_workspace_bytes(B, H, W, K, Co), m1)
-    C.call("ups_parts_conv_bwd", g_e0.data_ptr(), img.data_ptr(), hard.data_ptr(), V.data_ptr(), m1.data_ptr(),
-           _ptr(g_extra), dl1.data_ptr(), dV.data_ptr(), db.data_ptr(), B, H, W, K, img.shape[-1], Co, ws.data_ptr(),
-           ws.numel(), _stream(g_e0))
-    return dl1, dV, db
+    return _parts_conv_backward(g_e0, image1, hard, V, _f32(m1), g_extra)
 
 
 encode_conv_grad = _op("encode_conv_grad", _encode_conv_grad,

@@ -29,17 +29,6 @@ import torch
 from . import _cabi as C
 
 
-def _call_rows(name, noise, *args):
-    """Call the `_rows` entry point `name`, or, with noise = (seed, sample_offset, noise_level), its `_noise` form: the same
-    kernel reading l0 / l1 as means and adding the draw in registers (the same bytes; arguments of the `_rows` form, then
-    the three noise arguments, then the stream)."""
-    if noise is None:
-        C.call(name, *args)
-    else:
-        assert name.endswith("_rows"), name
-        C.call(name[:-len("_rows")] + "_noise", *args[:-1], *noise, args[-1])
-
-
 def kernel_route(K, F, P, first_conv=0, encoder_conv=0):
     """The kernels that run a step side of K parts (F feature channels, None for the encode side, which has none) on
     samples of P pixels: ("fused", K) for the fused kernels (K in {8,16,32}); ("padded", Kp) for a part count below 32
@@ -60,6 +49,139 @@ def decode_bwd_tc_ok(K, F, P):
     """Whether K4 (the decode side's backward on the fused kernels) can run as the persistent TMA + tcgen05/TMEM
     pipeline; otherwise it runs on the CUDA cores."""
     return K in (16, 32) and F == 64 and P % 128 == 0
+
+
+# ------------------------------------------------------------------ the launch sequence of each step side
+# Written once, called by PartStep with its persistent buffers and by the ups::part_* / ups::*_conv ops with fresh ones.
+# A launcher allocates nothing: outputs, scratch and workspaces, and the padded copies of a padded part count, come from
+# the caller.  `route` is kernel_route's: the fused kernels of K parts ("fused", "padded": logits and cotangents read in
+# rows of `row` floats, `planes` part planes written) or the generic ones ("generic", through the hard mask `hard`).
+# `noise` is None (the noise-free step) or (seed, sample_offset, noise_level): the logits are the means and the kernels
+# add noise_level * eps, eps drawn from (seed, draw, global pixel (sample_offset + b) * P + p, part); decode draws 0,
+# encode draws 1.  The seed is an int passed by value, or a one-element int64 CUDA tensor that the `_dseed` entry points
+# read on the device (a captured CUDA graph then draws with whatever that tensor holds at replay).
+def _ptr(t):
+    return None if t is None else t.data_ptr()
+
+
+def _seed_i64(seed):
+    """An unsigned 64-bit seed as the int64 with the same bits (what the op schemas carry); out of range raises."""
+    seed = int(seed)
+    if not 0 <= seed < 2 ** 64:
+        raise ValueError(f"seed must be in [0, 2**64), got {seed}")
+    return seed - 2 ** 64 if seed >= 2 ** 63 else seed
+
+
+def _seed_arg(seed):
+    return seed.data_ptr() if isinstance(seed, torch.Tensor) else seed % 2 ** 64
+
+
+def call_rows(name, noise, *args):
+    """Call the `_rows` entry point `name`, or with noise its `_noise` / `_noise_dseed` form: the same kernel, reading the
+    logits as means, with (seed, sample_offset, noise_level) inserted before the stream."""
+    if noise is None:
+        C.call(name, *args)
+    else:
+        seed, offset, level = noise
+        suffix = "_noise_dseed" if isinstance(seed, torch.Tensor) else "_noise"
+        C.call(name[:-len("_rows")] + suffix, *args[:-1], _seed_arg(seed), offset, level, args[-1])
+
+
+def part_softmax_fwd(noise, draw, logits, probs, labels, hard, B, P, K, st):
+    """The generic softmax of the logits (probs [, labels] [, hard = ST(hard_max)]), or of the sampled logits."""
+    if noise is None:
+        C.call("ups_part_softmax_fwd", logits.data_ptr(), probs.data_ptr(), _ptr(labels), _ptr(hard), B * P, K, st)
+        return
+    seed, offset, level = noise
+    C.call("ups_part_softmax_sampled_philox_fwd_dseed" if isinstance(seed, torch.Tensor) else
+           "ups_part_softmax_sampled_philox_fwd", logits.data_ptr(), _seed_arg(seed), draw, offset * P, level, None,
+           probs.data_ptr(), _ptr(labels), _ptr(hard), B * P, K, st)
+
+
+def encode_fwd(route, noise, l1, img1, m1, parts, pooled, hard, ws, B, P, K, row, planes, st):
+    """K2 (m1, the part images, their mean pool), or softmax -> mask_parts -> part_pool."""
+    if route != "generic":
+        call_rows("ups_step_encode_fwd_rows", noise, l1.data_ptr(), row, img1.data_ptr(), m1.data_ptr(), parts.data_ptr(),
+                  pooled.data_ptr(), B, P, K, planes, ws.data_ptr(), ws.numel(), st)
+        return
+    part_softmax_fwd(noise, 1, l1, m1, None, hard, B, P, K, st)
+    C.call("ups_mask_parts_fwd", img1.data_ptr(), hard.data_ptr(), parts.data_ptr(), B, P, K, 3, 1, st)
+    C.call("ups_part_pool_fwd", img1.data_ptr(), hard.data_ptr(), pooled.data_ptr(), B, P, K, 3, 0, 1.0 / P,
+           ws.data_ptr(), ws.numel(), st)
+
+
+def encode_bwd(route, g_parts, g_pooled, g_m1, img1, m1, hard, dl1, dimg1, dm, dm2, dfm, B, P, K, row, planes, st):
+    """K5 (dl1 [, dimg1]), or mask_parts_bwd [+ part_pool_bwd into dm2 (its image cotangent dfm added to dimg1)] ->
+    softmax_bwd2 of dm + dm2 + g_m1.  An undefined cotangent (None) or dimg1 = None reaches the kernels as a null pointer."""
+    if route != "generic":
+        C.call("ups_step_encode_bwd_rows", g_parts.data_ptr(), _ptr(g_pooled), img1.data_ptr(), m1.data_ptr(), _ptr(g_m1),
+               row, dl1.data_ptr(), _ptr(dimg1), B, P, K, planes, st)
+        return
+    C.call("ups_mask_parts_bwd", g_parts.data_ptr(), img1.data_ptr(), hard.data_ptr(), _ptr(dimg1), dm.data_ptr(),
+           B, P, K, 3, 1, st)
+    if g_pooled is None:
+        dm2 = None
+    else:
+        C.call("ups_part_pool_bwd", g_pooled.data_ptr(), img1.data_ptr(), hard.data_ptr(),
+               _ptr(dfm if dimg1 is not None else None), dm2.data_ptr(), B, P, K, 3, 0, 1.0 / P, st)
+        if dimg1 is not None:
+            C.call("ups_axpy", dfm.data_ptr(), dimg1.data_ptr(), dimg1.numel(), 1.0, st)
+    C.call("ups_part_softmax_bwd2", m1.data_ptr(), dm.data_ptr(), _ptr(dm2), _ptr(g_m1), dl1.data_ptr(), B * P, K, st)
+
+
+def decode_fwd(route, noise, l0, feat, m0, labels0, inj, hard, B, P, K, F, row, st):
+    """K3 (m0, labels0, the injected map), or softmax -> part_inject."""
+    if route != "generic":
+        call_rows("ups_step_decode_fwd_rows", noise, l0.data_ptr(), row, feat.data_ptr(), m0.data_ptr(), labels0.data_ptr(),
+                  inj.data_ptr(), B, P, K, F, st)
+        return
+    part_softmax_fwd(noise, 0, l0, m0, labels0, hard, B, P, K, st)
+    C.call("ups_part_inject_fwd", feat.data_ptr(), hard.data_ptr(), inj.data_ptr(), B, P, K, F, st)
+
+
+def decode_bwd(route, tc, g_inj, g_m0, m0, hard, feat, dl0, dfeat, dm, ws, B, P, K, F, row, st):
+    """K4 (dl0, dfeat) on tcgen05 (tc) or on the CUDA cores, or part_inject_bwd -> softmax_bwd2 of dm + g_m0."""
+    if route != "generic":
+        C.call("ups_step_decode_bwd_tc_rows" if tc else "ups_step_decode_bwd_rows", g_inj.data_ptr(), m0.data_ptr(),
+               _ptr(g_m0), row, feat.data_ptr(), dl0.data_ptr(), dfeat.data_ptr(), B, P, K, F, ws.data_ptr(), ws.numel(), st)
+        return
+    C.call("ups_part_inject_bwd", g_inj.data_ptr(), feat.data_ptr(), hard.data_ptr(), dfeat.data_ptr(), dm.data_ptr(),
+           B, P, K, F, ws.data_ptr(), ws.numel(), st)
+    C.call("ups_part_softmax_bwd2", m0.data_ptr(), dm.data_ptr(), _ptr(g_m0), None, dl0.data_ptr(), B * P, K, st)
+
+
+# The first convolutions folded into the sides (SURVEY 8f N4).  Shapes: feat [B,K,F], V [..,Co], G / dG [B,9,K,Co],
+# masks [B,H,W,K], img [B,H,W,Cin].
+def inject_conv_table_fwd(feat, V, G, st):
+    B, K, F = feat.shape
+    C.call("ups_inject_conv_table_fwd", feat.data_ptr(), V.data_ptr(), G.data_ptr(), B, K, F, V.shape[-1], st)
+
+
+def inject_conv_table_bwd(dG, feat, V, dfeat, dV, st):
+    B, K, F = feat.shape
+    C.call("ups_inject_conv_table_bwd", dG.data_ptr(), feat.data_ptr(), V.data_ptr(), dfeat.data_ptr(), dV.data_ptr(),
+           B, K, F, V.shape[-1], st)
+
+
+def inject_conv_fwd(mask, G, bias, out, st):
+    C.call("ups_inject_conv_fwd", mask.data_ptr(), G.data_ptr(), bias.data_ptr(), out.data_ptr(), *mask.shape, G.shape[-1],
+           st)
+
+
+def inject_conv_bwd(g_out, mask, G, probs, g_extra, dmask, dG, db, ws, st):
+    C.call("ups_inject_conv_bwd", g_out.data_ptr(), mask.data_ptr(), G.data_ptr(), _ptr(probs), _ptr(g_extra),
+           dmask.data_ptr(), dG.data_ptr(), db.data_ptr(), *mask.shape, G.shape[-1], ws.data_ptr(), ws.numel(), st)
+
+
+def parts_conv_fwd(img, mask, V, bias, out, st):
+    C.call("ups_parts_conv_fwd", img.data_ptr(), mask.data_ptr(), V.data_ptr(), bias.data_ptr(), out.data_ptr(),
+           *mask.shape, img.shape[-1], V.shape[-1], st)
+
+
+def parts_conv_bwd(g_out, img, mask, V, probs, g_extra, dmask, dV, db, ws, st):
+    C.call("ups_parts_conv_bwd", g_out.data_ptr(), img.data_ptr(), mask.data_ptr(), V.data_ptr(), _ptr(probs),
+           _ptr(g_extra), dmask.data_ptr(), dV.data_ptr(), db.data_ptr(), *mask.shape, img.shape[-1], V.shape[-1],
+           ws.data_ptr(), ws.numel(), st)
 
 
 def _on_device(fn):
@@ -94,15 +216,15 @@ class PartStep:
             raise C.UpsError("PartStep needs a CUDA device: there is no CPU path")
         if self.device.index is None:
             self.device = torch.device("cuda", torch.cuda.current_device())
-        route, Kr = kernel_route(K, F, self.P, first_conv, encoder_conv)
-        self.fused = route == "fused"
+        self.route, Kr = kernel_route(K, F, self.P, first_conv, encoder_conv)
+        self.fused = self.route == "fused"
         # A part count that is not a power of two (the reference ships n_parts = 25, train_cub_subset_tps.yaml:132) runs on
         # the fused kernels of the next power of two Kp: logits padded with -inf, everything else with zeros.  exp_canon
         # maps -inf to exactly 0 and the canonical K-way sum is a pair tree over the zero-padded terms, so
         # probabilities, masks and labels are bit-identical to the K-part evaluation; padding planes of the part images
         # are neither written nor read (csrc: *_planes entry points).
         self.Kp = 0
-        if route == "padded" and _planes is None:
+        if self.route == "padded" and _planes is None:
             self.Kp = Kr
             self._inner = PartStep(B, S, self.Kp, F, n_views=V, use_tps=use_tps, views_grad=views_grad, device=self.device,
                                    decode_bwd=decode_bwd, sample_offset=sample_offset, _planes=K)
@@ -154,6 +276,7 @@ class PartStep:
         if self.views_grad:
             self.dimg1 = e(B, S, S, 3, **f32)
             self.dviews = e(max(V, 2), B, S, S, 3, **f32)
+        self.mh0 = self.mh1 = self.dm = self.dm2 = self.dfm = None   # the generic kernels' masks and scratch
         if not self.fused:
             self.mh0, self.mh1 = e(B, S, S, K, **f32), e(B, S, S, K, **f32)
             self.dm = e(B, S, S, K, **f32)
@@ -175,24 +298,8 @@ class PartStep:
         return torch.cuda.current_stream(self.device).cuda_stream
 
     def _noise(self, noise_seed, noise_level):
-        """(seed, sample_offset, noise_level) for the `_noise` entry points, or None (the noise-free step)."""
-        if noise_seed is None:
-            return None
-        seed = int(noise_seed)
-        if not 0 <= seed < 2 ** 64:
-            raise ValueError(f"noise_seed must be in [0, 2**64), got {noise_seed}")
-        return (seed, self.sample_offset, float(noise_level))
-
-    def _softmax_fwd(self, logits, draw, probs, labels, hard, nz, st):
-        """ups_part_softmax_fwd on the logits, or with noise nz on the means (the draw of side `draw` made in registers)."""
-        p = lambda t: None if t is None else t.data_ptr()  # noqa: E731
-        n = self.B * self.P
-        if nz is None:
-            C.call("ups_part_softmax_fwd", logits.data_ptr(), probs.data_ptr(), p(labels), p(hard), n, self.K, st)
-        else:
-            seed, offset, level = nz
-            C.call("ups_part_softmax_sampled_philox_fwd", logits.data_ptr(), seed, draw, offset * self.P, level, None,
-                   probs.data_ptr(), p(labels), p(hard), n, self.K, st)
+        """The launchers' noise value of forward(noise_seed=, noise_level=): None, or (seed, sample_offset, noise_level)."""
+        return None if noise_seed is None else (_seed_i64(noise_seed), self.sample_offset, float(noise_level))
 
     # ------------------------------------------------------------------ padded part count (K -> Kp)
     def _init_padded(self):
@@ -281,18 +388,6 @@ class PartStep:
         return out
 
     # ------------------------------------------------------------------ forward
-    def _decode_fwd(self, l0, feat, conv_V, conv_b, st, l0_row=None, nz=None):
-        """decode side on stream `st`: K3, or with first_conv softmax -> table -> 3x3 conv on the assignment"""
-        B, S, K, F, P = self.B, self.S, self.K, self.F, self.P
-        if not self.Co:
-            _call_rows("ups_step_decode_fwd_rows", nz, l0.data_ptr(), l0_row or K, feat.data_ptr(), self.m0.data_ptr(),
-                       self.labels0.data_ptr(), self.inj.data_ptr(), B, P, K, F, st)
-            return
-        self._softmax_fwd(l0, 0, self.m0, self.labels0, self.mh0c, nz, st)
-        C.call("ups_inject_conv_table_fwd", feat.data_ptr(), conv_V.data_ptr(), self.G.data_ptr(), B, K, F, self.Co, st)
-        C.call("ups_inject_conv_fwd", self.mh0c.data_ptr(), self.G.data_ptr(), conv_b.data_ptr(), self.h0.data_ptr(),
-               B, S, S, K, self.Co, st)
-
     def forward(self, views, coord, t_vector, l0, l1, feat, conv_V=None, conv_b=None, enc_V=None, enc_b=None, rows=None,
                 noise_seed=None, noise_level=1.0):
         """views [V,B,S,S,3] (view0, view1[, view0_target]), fp32 in [-1, 1] or the dataset's uint8
@@ -334,15 +429,14 @@ class PartStep:
         C.call("ups_tps_solve", coord.data_ptr(), t_vector.data_ptr(), self.T.data_ptr(), 2 * B, st)
         if self.before_params is not None:
             self.before_params()     # data-parallel wrapper: wait for the averaged gradients (the TPS solve needs none)
-        _call_rows("ups_step_warp_decode_fwd_rows", nz, views.data_ptr(), views[2].data_ptr() if V > 2 else None,
-                   coord.data_ptr(), self.T.data_ptr(), self.warped.data_ptr(), self.warped[2].data_ptr() if V > 2 else None,
-                   2 * B, B if V > 2 else 0, S, l0.data_ptr(), r0, feat.data_ptr(), self.m0.data_ptr(),
-                   self.labels0.data_ptr(), self.inj.data_ptr(), B, K, F, st)
+        call_rows("ups_step_warp_decode_fwd_rows", nz, views.data_ptr(), views[2].data_ptr() if V > 2 else None,
+                  coord.data_ptr(), self.T.data_ptr(), self.warped.data_ptr(), self.warped[2].data_ptr() if V > 2 else None,
+                  2 * B, B if V > 2 else 0, S, l0.data_ptr(), r0, feat.data_ptr(), self.m0.data_ptr(),
+                  self.labels0.data_ptr(), self.inj.data_ptr(), B, K, F, st)
         self._warped, self._coord = self.warped, coord
         img1 = self.warped[1]
         self._img1, self._feat = img1, feat
-        _call_rows("ups_step_encode_fwd_rows", nz, l1.data_ptr(), r1, img1.data_ptr(), self.m1.data_ptr(),
-                   self.parts.data_ptr(), self.pooled.data_ptr(), B, P, K, self.Kpl, self.ws.data_ptr(), self.ws.numel(), st)
+        encode_fwd(self.route, nz, l1, img1, self.m1, self.parts, self.pooled, None, self.ws, B, P, K, r1, self.Kpl, st)
         return dict(warped=self.warped, m0=self.m0, m1=self.m1, labels0=self.labels0, parts=self.parts,
                     pooled=self.pooled, inj=self.inj)
 
@@ -416,22 +510,17 @@ class PartStep:
             assert tuple(enc_V.shape) == (3, 3, 3, self.Ce) and tuple(enc_b.shape) == (self.Ce,)
             assert enc_V.is_contiguous() and enc_b.is_contiguous()
             self._enc_V = enc_V
-            self._softmax_fwd(l1, 1, self.m1, None, self.mh1c, nz, st)
-            C.call("ups_parts_conv_fwd", img1.data_ptr(), self.mh1c.data_ptr(), enc_V.data_ptr(), enc_b.data_ptr(),
-                   self.e0.data_ptr(), B, S, S, K, 3, self.Ce, st)
-        elif self.fused:
-            _call_rows("ups_step_encode_fwd_rows", nz, l1.data_ptr(), r1, img1.data_ptr(), self.m1.data_ptr(),
-                       self.parts.data_ptr(), self.pooled.data_ptr(), B, P, K, self.Kpl, self.ws.data_ptr(), self.ws.numel(), st)
+            part_softmax_fwd(nz, 1, l1, self.m1, None, self.mh1c, B, P, K, st)
+            parts_conv_fwd(img1, self.mh1c, enc_V, enc_b, self.e0, st)
         else:
-            self._softmax_fwd(l1, 1, self.m1, None, self.mh1, nz, st)
-            C.call("ups_mask_parts_fwd", img1.data_ptr(), self.mh1.data_ptr(), self.parts.data_ptr(), B, P, K, 3, 1, st)
-            C.call("ups_part_pool_fwd", img1.data_ptr(), self.mh1.data_ptr(), self.pooled.data_ptr(), B, P, K, 3, 0,
-                   1.0 / P, self.ws.data_ptr(), self.ws.numel(), st)
-        if self.fused or self.Co:
-            self._decode_fwd(l0, feat, conv_V, conv_b, st, r0, nz)
+            encode_fwd(self.route, nz, l1, img1, self.m1, self.parts, self.pooled, self.mh1, self.ws, B, P, K, r1, self.Kpl,
+                       st)
+        if self.Co:
+            part_softmax_fwd(nz, 0, l0, self.m0, self.labels0, self.mh0c, B, P, K, st)
+            inject_conv_table_fwd(feat, conv_V, self.G, st)
+            inject_conv_fwd(self.mh0c, self.G, conv_b, self.h0, st)
         else:
-            self._softmax_fwd(l0, 0, self.m0, self.labels0, self.mh0, nz, st)
-            C.call("ups_part_inject_fwd", feat.data_ptr(), self.mh0.data_ptr(), self.inj.data_ptr(), B, P, K, F, st)
+            decode_fwd(self.route, nz, l0, feat, self.m0, self.labels0, self.inj, self.mh0, B, P, K, F, r0, st)
         out = dict(warped=warped, m0=self.m0, m1=self.m1, labels0=self.labels0)
         if self.Ce:
             out["e0"] = self.e0
@@ -464,24 +553,13 @@ class PartStep:
         B, S, K, F, P = self.B, self.S, self.K, self.F, self.P
         st = self._stream()
         feat = self._feat
-        p = lambda t: None if t is None else t.data_ptr()  # noqa: E731
         if self.Co:
             assert tuple(g_inj.shape) == (B, S, S, self.Co), list(g_inj.shape)
-            C.call("ups_inject_conv_bwd", g_inj.data_ptr(), self.mh0c.data_ptr(), self.G.data_ptr(), self.m0.data_ptr(),
-                   p(g_m0), self.dl0.data_ptr(), self.dG.data_ptr(), self.db.data_ptr(), B, S, S, K, self.Co,
-                   self.ws_ic.data_ptr(), self.ws_ic.numel(), st)
-            C.call("ups_inject_conv_table_bwd", self.dG.data_ptr(), feat.data_ptr(), self._conv_V.data_ptr(),
-                   self.dfeat.data_ptr(), self.dV.data_ptr(), B, K, F, self.Co, st)
-        elif self.fused:
-            C.call("ups_step_decode_bwd_tc_rows" if self.decode_bwd == "tc" else "ups_step_decode_bwd_rows",
-                   g_inj.data_ptr(), self.m0.data_ptr(), p(g_m0), gm_row or K, feat.data_ptr(),
-                   self.dl0.data_ptr(), self.dfeat.data_ptr(), B, P, K, F, self.ws.data_ptr(), self.ws.numel(), st)
+            inject_conv_bwd(g_inj, self.mh0c, self.G, self.m0, g_m0, self.dl0, self.dG, self.db, self.ws_ic, st)
+            inject_conv_table_bwd(self.dG, feat, self._conv_V, self.dfeat, self.dV, st)
         else:
-            # dm0 = inject-bwd (+ g_m0, accumulated by the kernel) -> softmax-bwd
-            C.call("ups_part_inject_bwd", g_inj.data_ptr(), feat.data_ptr(), self.mh0.data_ptr(),
-                   self.dfeat.data_ptr(), self.dm.data_ptr(), B, P, K, F, self.ws.data_ptr(), self.ws.numel(), st)
-            C.call("ups_part_softmax_bwd2", self.m0.data_ptr(), self.dm.data_ptr(), p(g_m0), None, self.dl0.data_ptr(),
-                   B * P, K, st)
+            decode_bwd(self.route, self.decode_bwd == "tc", g_inj, g_m0, self.m0, self.mh0, feat, self.dl0, self.dfeat,
+                       self.dm, self.ws, B, P, K, F, gm_row or K, st)
         out = dict(dl0=self.dl0, dfeat=self.dfeat)
         if self.Co:
             out["dV"], out["db"] = self.dV, self.db
@@ -493,28 +571,12 @@ class PartStep:
         B, S, K, P, V = self.B, self.S, self.K, self.P, self.V
         st = self._stream()
         img1 = self._img1
-        p = lambda t: None if t is None else t.data_ptr()  # noqa: E731
-        want_dimg = self.views_grad
         if self.Ce:
             assert tuple(g_parts.shape) == (K * B, S, S, self.Ce), list(g_parts.shape)      # g_e0 in the place of g_parts
-            C.call("ups_parts_conv_bwd", g_parts.data_ptr(), img1.data_ptr(), self.mh1c.data_ptr(), self._enc_V.data_ptr(),
-                   self.m1.data_ptr(), p(g_m1), self.dl1.data_ptr(), self.dVe.data_ptr(), self.dbe.data_ptr(), B, S, S, K, 3,
-                   self.Ce, self.ws_pc.data_ptr(), self.ws_pc.numel(), st)
+            parts_conv_bwd(g_parts, img1, self.mh1c, self._enc_V, self.m1, g_m1, self.dl1, self.dVe, self.dbe, self.ws_pc, st)
             return dict(dl1=self.dl1, dVe=self.dVe, dbe=self.dbe)
-        if self.fused:
-            C.call("ups_step_encode_bwd_rows", g_parts.data_ptr(), p(g_pooled), img1.data_ptr(), self.m1.data_ptr(),
-                   p(g_m1), gm_row or K, self.dl1.data_ptr(), self.dimg1.data_ptr() if want_dimg else None, B, P, K, self.Kpl, st)
-        else:
-            C.call("ups_mask_parts_bwd", g_parts.data_ptr(), img1.data_ptr(), self.mh1.data_ptr(),
-                   self.dimg1.data_ptr() if want_dimg else None, self.dm.data_ptr(), B, P, K, 3, 1, st)
-            if g_pooled is not None:
-                C.call("ups_part_pool_bwd", g_pooled.data_ptr(), img1.data_ptr(), self.mh1.data_ptr(),
-                       self.dfm.data_ptr() if want_dimg else None, self.dm2.data_ptr(), B, P, K, 3, 0, 1.0 / P, st)
-                if want_dimg:
-                    C.call("ups_axpy", self.dfm.data_ptr(), self.dimg1.data_ptr(), self.dimg1.numel(), 1.0, st)
-            # dl1 = softmax-bwd(m1, dm + dm2 + g_m1): the three cotangents are summed inside the kernel
-            C.call("ups_part_softmax_bwd2", self.m1.data_ptr(), self.dm.data_ptr(),
-                   self.dm2.data_ptr() if g_pooled is not None else None, p(g_m1), self.dl1.data_ptr(), B * P, K, st)
+        encode_bwd(self.route, g_parts, g_pooled, g_m1, img1, self.m1, self.mh1, self.dl1,
+                   self.dimg1 if self.views_grad else None, self.dm, self.dm2, self.dfm, B, P, K, gm_row or K, self.Kpl, st)
         out = dict(dl1=self.dl1)
         if self.views_grad:
             if self.use_tps:
@@ -523,13 +585,13 @@ class PartStep:
                 if gw is not None:
                     assert gw.is_contiguous() and tuple(gw.shape) == (max(V, 2), B, S, S, 3), list(gw.shape)
                 pair = V > 2 and gw is not None
-                C.call("ups_tps_warp_bwd_sum", p(gw), gw[2].data_ptr() if pair else None, self.dimg1.data_ptr(), B, B,
+                C.call("ups_tps_warp_bwd_sum", _ptr(gw), gw[2].data_ptr() if pair else None, self.dimg1.data_ptr(), B, B,
                        coord.data_ptr(), self.T.data_ptr(), self.dviews.data_ptr(),
                        self.dviews[2].data_ptr() if pair else None, 2 * B, B, S, S, 3, S, S, st)
                 if V > 2 and gw is None:
                     C.call("ups_views_cotangent", None, None, self.dviews[2].data_ptr(), 1, 0, B * P * 3, st)   # zeros
             else:
-                C.call("ups_views_cotangent", p(g_warped), self.dimg1.data_ptr(), self.dviews.data_ptr(), max(V, 2), 1,
+                C.call("ups_views_cotangent", _ptr(g_warped), self.dimg1.data_ptr(), self.dviews.data_ptr(), max(V, 2), 1,
                        B * P * 3, st)
             out["dviews"] = self.dviews
         return out
