@@ -95,6 +95,27 @@ int ups_tps_warp_pair_fwd(const float* U, const float* U2, const float* coord, c
 int ups_tps_warp_pair_bwd(const float* g_out, const float* g_out2, const float* coord, const float* T, float* dU,
                           float* dU2, int N, int N2, int H, int W, int C, int out_h, int out_w, void* stream);
 
+/* tps_parameters (transformations.py:17-39) drawn on the device from a seed, make_input_tps_param and the solve, in one
+ * launch.  The draw is defined in csrc/canon_math.cuh ("the TPS parameters"): the fields of view v, global sample g are
+ * a pure function of (seed, v, g) (Philox4x32-10, counter (g lo, g hi, j, 2 + v); draws 0 and 1 of a seed are the logit
+ * noise), uniforms in [0, 1) as tf.random_uniform.  Row r = v * n_per_view + s (n_views = 1 or 2) is view v of global
+ * sample sample_offset + s.  The ten scalars (fp32, formed from tps_parameters' arguments in double and rounded once):
+ * coord_lo, coord_w = -0.2, 0.4; vec_lo, vec_w = -tps_scal, 2 tps_scal; off_lo, off_w = -off_scal, 2 off_scal;
+ * scal_lo, scal_w = scal (1 - scal_var), 2 scal scal_var; rescal; rot_turn = rot_scal / (2 pi) in [0, 1/2].
+ * Raw outputs coord, vector [N,8,2], offset, offset_2 [N,1,2], t_scal [N,2], rot_mat [N,2,2] may each be NULL;
+ * t_vector [N,8,2] and T [N,2,11] are bit for bit what ups_tps_input_param + ups_tps_solve give on the raw fields.
+ * _dseed: `seed` points to one device word holding the seed, read once by the kernel (a captured CUDA graph draws with
+ * the value the word holds at replay). */
+int ups_tps_draw_solve(unsigned long long seed, long long sample_offset, int n_per_view, int n_views, float coord_lo,
+                       float coord_w, float vec_lo, float vec_w, float off_lo, float off_w, float scal_lo, float scal_w,
+                       float rescal, float rot_turn, float* coord, float* vector, float* offset, float* offset_2,
+                       float* t_scal, float* rot_mat, float* t_vector, float* T, void* stream);
+int ups_tps_draw_solve_dseed(const unsigned long long* seed, long long sample_offset, int n_per_view, int n_views,
+                             float coord_lo, float coord_w, float vec_lo, float vec_w, float off_lo, float off_w,
+                             float scal_lo, float scal_w, float rescal, float rot_turn, float* coord, float* vector,
+                             float* offset, float* offset_2, float* t_scal, float* rot_mat, float* t_vector, float* T,
+                             void* stream);
+
 /* ---- part-map softmax / hard max / straight-through / argmax ------------------------ */
 /* nn.softmax(x, spatial=False) — cub/code/nn.py:58-62, fused with the consumers at
  * cub/code/SB_model48i/model.py:426-473: probs, optional int64 argmax labels (first index),

@@ -33,6 +33,26 @@ void ups_host_normal_philox(unsigned long long seed, int draw, long long pix_off
         }
 }
 
+// the TPS parameters (canon_math.cuh::tps_fields).  s = the ten TpsDrawScalars in their declared order.
+// From given words x [n, 39] (lets tests pick words such as u = 0 and u = 1 - 2^-24):
+void ups_host_tps_fields(const uint32_t* x, const float* s, float* coord, float* vector, float* offset, float* offset_2,
+                         float* t_scal, float* rot, long long n) {
+    const ups::TpsDrawScalars sc{s[0], s[1], s[2], s[3], s[4], s[5], s[6], s[7], s[8], s[9]};
+    for (long long i = 0; i < n; ++i)
+        ups::tps_fields(sc, x + i * ups::TPS_DRAW_WORDS, coord + i * 16, vector + i * 16, offset + i * 2, offset_2 + i * 2,
+                        t_scal + i * 2, rot + i * 4);
+}
+// drawn for view v, global samples g_offset .. g_offset + n - 1 (one view of ups_tps_draw_solve on the host)
+void ups_host_tps_draw(unsigned long long seed, int v, unsigned long long g_offset, long long n, const float* s, float* coord,
+                       float* vector, float* offset, float* offset_2, float* t_scal, float* rot) {
+    const ups::TpsDrawScalars sc{s[0], s[1], s[2], s[3], s[4], s[5], s[6], s[7], s[8], s[9]};
+    uint32_t x[4 * ups::TPS_DRAW_CALLS];
+    for (long long i = 0; i < n; ++i) {
+        for (int j = 0; j < ups::TPS_DRAW_CALLS; ++j) ups::tps_words4(seed, v, g_offset + (unsigned long long)i, (uint32_t)j, x + 4 * j);
+        ups::tps_fields(sc, x, coord + i * 16, vector + i * 16, offset + i * 2, offset_2 + i * 2, t_scal + i * 2, rot + i * 4);
+    }
+}
+
 void ups_host_softmax(const float* x, float* p, long long* labels, float* hard, long long n_pix, int K) {
     std::vector<float> e(ups::KMAX * 2);
     for (long long i = 0; i < n_pix; ++i) {

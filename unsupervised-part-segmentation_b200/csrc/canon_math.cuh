@@ -323,4 +323,78 @@ UPS_HD void normal4_philox(unsigned long long seed, uint32_t draw, unsigned long
 
 UPS_HD float sampled_logit(float mean, float noise_level, float z) { return UPS_FADD(mean, UPS_FMUL(noise_level, z)); }
 
+// ---------------------------------------------------------------- the Philox draws of one seed
+// Every device draw under one seed uses Philox4x32-10 with key = seed and a counter whose last word names the draw, so
+// that no two draws ever share a counter:
+//   0  the logit noise of l0 (decode side)      1  the logit noise of l1 (encode side)
+//   2  the TPS parameters of view 0             3  the TPS parameters of view 1
+constexpr uint32_t DRAW_LOGITS0 = 0, DRAW_LOGITS1 = 1, DRAW_TPS_VIEW0 = 2, DRAW_TPS_VIEW1 = 3;
+
+// ---------------------------------------------------------------- the TPS parameters (oracle/tps_draw.py)
+// tps_parameters (transformations.py:17-39) draws its fields with tf.random_uniform, in [lo, hi).  Here the fields of one
+// sample are a pure function of (seed, view v, global sample g):
+//   x[4j .. 4j+3] = Philox4x32-10(counter = (g lo, g hi, j, DRAW_TPS_VIEW0 + v), key = (seed lo, seed hi)),  j = 0 .. 9
+//   u(x)          = (x >> 8) * 2^-24                        in [0, 1), exact in fp32
+//   U(lo, w)      = fl(lo + fl(u * w))                      lo and w = hi - lo formed in double, rounded to fp32 once
+// Word order (39 of the 40 words are used):
+//   0 .. 15   coord [8,2] row-major: fl(base + U(-0.2, 0.2)), base = the fp32 control points of transformations.py:18-19
+//   16 .. 31  vector [8,2] row-major: U(-tps_scal, tps_scal)
+//   32, 33    offset: U(-off_scal, off_scal)              34, 35  offset_2: the same range
+//   36, 37    t_scal: fl(U(scal (1 - scal_var), scal (1 + scal_var)) * rescal)
+//   38        rotation, as a signed fraction of a turn: t = fl(rot_turn * fl(2u - 1)), rot_turn = fl(rot_scal / (2 pi));
+//             (s, c) = sincos2pi_canon(|t|), s negated when t < 0;  rot_mat [2,2] = [[c, -s], [s, c]]
+// The value does not depend on the batch size, the launch geometry or how the batch is split.
+constexpr int TPS_DRAW_CALLS = 10, TPS_DRAW_WORDS = 39;
+constexpr int TPS_W_COORD = 0, TPS_W_VECTOR = 16, TPS_W_OFFSET = 32, TPS_W_OFFSET2 = 34, TPS_W_TSCAL = 36, TPS_W_ROT = 38;
+
+struct TpsDrawScalars {
+    float coord_lo, coord_w, vec_lo, vec_w, off_lo, off_w, scal_lo, scal_w, rescal, rot_turn;
+};
+
+UPS_HD float tps_base(int i) {   // transformations.py:18-19, [8,2] row-major
+    const float b[16] = {-0.5f, -0.5f, 0.5f, -0.5f, -0.5f, 0.5f, 0.5f, 0.5f, 0.2f, -0.2f, -0.2f, 0.2f, 0.2f, 0.2f, -0.2f, -0.2f};
+    return b[i];
+}
+
+UPS_HD float uniform24_half_open(uint32_t x) { return UPS_FMUL((float)(x >> 8), 5.9604644775390625e-8f); }
+
+// the field of word w < TPS_W_ROT; the rotation word is tps_rotation's
+UPS_HD float tps_field(const TpsDrawScalars& s, int w, uint32_t x) {
+    const float u = uniform24_half_open(x);
+    if (w < TPS_W_VECTOR) return UPS_FADD(tps_base(w - TPS_W_COORD), UPS_FADD(s.coord_lo, UPS_FMUL(u, s.coord_w)));
+    if (w < TPS_W_OFFSET) return UPS_FADD(s.vec_lo, UPS_FMUL(u, s.vec_w));
+    if (w < TPS_W_TSCAL) return UPS_FADD(s.off_lo, UPS_FMUL(u, s.off_w));
+    return UPS_FMUL(UPS_FADD(s.scal_lo, UPS_FMUL(u, s.scal_w)), s.rescal);
+}
+
+// rot [2,2] row-major from the rotation word
+UPS_HD void tps_rotation(float rot_turn, uint32_t x, float* rot) {
+    const float t = UPS_FMUL(rot_turn, UPS_FSUB(UPS_FMUL(2.0f, uniform24_half_open(x)), 1.0f));
+    float s, c;
+    sincos2pi_canon(fabsf(t), s, c);
+    s = t < 0.0f ? -s : s;
+    rot[0] = c; rot[1] = -s; rot[2] = s; rot[3] = c;
+}
+
+// all fields of one sample from its words x[0 .. 38], in the reference's layouts (coord / vector [8,2], offset /
+// offset_2 [2], t_scal [2], rot [2,2])
+UPS_HD void tps_fields(const TpsDrawScalars& s, const uint32_t* x, float* coord, float* vector, float* offset,
+                       float* offset_2, float* t_scal, float* rot) {
+    for (int i = 0; i < 16; ++i) coord[i] = tps_field(s, TPS_W_COORD + i, x[TPS_W_COORD + i]);
+    for (int i = 0; i < 16; ++i) vector[i] = tps_field(s, TPS_W_VECTOR + i, x[TPS_W_VECTOR + i]);
+    for (int i = 0; i < 2; ++i) {
+        offset[i] = tps_field(s, TPS_W_OFFSET + i, x[TPS_W_OFFSET + i]);
+        offset_2[i] = tps_field(s, TPS_W_OFFSET2 + i, x[TPS_W_OFFSET2 + i]);
+        t_scal[i] = tps_field(s, TPS_W_TSCAL + i, x[TPS_W_TSCAL + i]);
+    }
+    tps_rotation(s.rot_turn, x[TPS_W_ROT], rot);
+}
+
+// words 4j .. 4j+3 of the draw of view v, global sample g
+UPS_HD void tps_words4(unsigned long long seed, int v, unsigned long long g, uint32_t j, uint32_t* x) {
+    uint32_t c0 = (uint32_t)g, c1 = (uint32_t)(g >> 32), c2 = j, c3 = DRAW_TPS_VIEW0 + (uint32_t)v;
+    philox4x32_10(c0, c1, c2, c3, (uint32_t)seed, (uint32_t)(seed >> 32));
+    x[0] = c0; x[1] = c1; x[2] = c2; x[3] = c3;
+}
+
 }  // namespace ups

@@ -36,16 +36,12 @@ __global__ void tps_input_param_kernel(const float* __restrict__ coord, const fl
 // the result is bit-identical to the sequential form (tests/test_canon_host.py pins that form).
 constexpr int SOLVE_WARPS = 4;
 
-__global__ void __launch_bounds__(SOLVE_WARPS * 32) tps_solve_kernel(const float* __restrict__ coord,
-                                                                     const float* __restrict__ vector,
-                                                                     float* __restrict__ T, int N) {
+// The solve of sample b by its warp: qx / qy = the flipped control points (every lane holds all 8), vec_at(k) = element
+// k of the sample's vector [8,2] (called by lanes 0..7 for k = 2 lane, 2 lane + 1).
+template <typename VecAt>
+__device__ __forceinline__ void tps_solve_warp(const float (&qx)[8], const float (&qy)[8], VecAt vec_at,
+                                               float* __restrict__ T, int b, int lane) {
     constexpr unsigned FULLM = 0xffffffffu;
-    const int lane = threadIdx.x & 31;
-    const int b = blockIdx.x * SOLVE_WARPS + (threadIdx.x >> 5);
-    if (b >= N) return;  // warp-uniform
-    float qx[8], qy[8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) { qx[i] = __ldg(coord + b * 16 + 2 * i + 1); qy[i] = __ldg(coord + b * 16 + 2 * i); }
     double row[13];
 #pragma unroll
     for (int j = 0; j < 13; ++j) row[j] = 0.0;
@@ -62,8 +58,8 @@ __global__ void __launch_bounds__(SOLVE_WARPS * 32) tps_solve_kernel(const float
             const float d2 = __fadd_rn(__fadd_rn(__fmul_rn(d0, d0), __fmul_rn(d1, d1)), __fmul_rn(d2_, d2_));
             row[3 + j] = (double)tps_rbf(d2);
         }
-        row[11] = (double)__fadd_rn(mx, __ldg(vector + b * 16 + 2 * lane + 1));
-        row[12] = (double)__fadd_rn(my, __ldg(vector + b * 16 + 2 * lane));
+        row[11] = (double)__fadd_rn(mx, vec_at(2 * lane + 1));
+        row[12] = (double)__fadd_rn(my, vec_at(2 * lane));
     } else if (lane < 11) {
 #pragma unroll
         for (int j = 0; j < 8; ++j) row[3 + j] = (lane == 8) ? 1.0 : (lane == 9 ? (double)qx[j] : (double)qy[j]);
@@ -97,6 +93,70 @@ __global__ void __launch_bounds__(SOLVE_WARPS * 32) tps_solve_kernel(const float
         T[b * 22 + pos] = (float)__ddiv_rn(row[11], d);
         T[b * 22 + 11 + pos] = (float)__ddiv_rn(row[12], d);
     }
+}
+
+__global__ void __launch_bounds__(SOLVE_WARPS * 32) tps_solve_kernel(const float* __restrict__ coord,
+                                                                     const float* __restrict__ vector,
+                                                                     float* __restrict__ T, int N) {
+    const int lane = threadIdx.x & 31;
+    const int b = blockIdx.x * SOLVE_WARPS + (threadIdx.x >> 5);
+    if (b >= N) return;  // warp-uniform
+    float qx[8], qy[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) { qx[i] = __ldg(coord + b * 16 + 2 * i + 1); qy[i] = __ldg(coord + b * 16 + 2 * i); }
+    tps_solve_warp(qx, qy, [&](int k) { return __ldg(vector + b * 16 + k); }, T, b, lane);
+}
+
+// ------------------------------------------------------------------ a1 + a2 + a3(ii): draw, make_input_tps_param, solve
+// One warp per row r = v * n_per_view + s (view v, global sample sample_offset + s).  Lanes 0..9 make one Philox call
+// each (words 4 lane .. 4 lane + 3, canon_math.cuh "the TPS parameters"); every lane then gathers the 39 words, forms the
+// fields with tps_fields and t_vector with tps_input_param, and the warp runs tps_solve_warp, the body of
+// tps_solve_kernel.  coord / t_vector / T are bit for bit what ups_tps_input_param + ups_tps_solve give on the fields.
+// DSEED: `seed` is the address of the seed (resolve_seed).  Each raw output may be null.
+// a[i] of a register array, without local memory
+template <int N>
+__device__ __forceinline__ float pick(const float (&a)[N], int i) {
+    float r = a[0];
+#pragma unroll
+    for (int k = 1; k < N; ++k) if (k == i) r = a[k];
+    return r;
+}
+
+template <bool DSEED>
+__global__ void __launch_bounds__(SOLVE_WARPS * 32) tps_draw_solve_kernel(
+    unsigned long long seed, long long sample_offset, int n_per_view, int N, TpsDrawScalars sc, float* __restrict__ coord,
+    float* __restrict__ vector, float* __restrict__ offset, float* __restrict__ offset_2, float* __restrict__ t_scal,
+    float* __restrict__ rot_mat, float* __restrict__ t_vector, float* __restrict__ T) {
+    constexpr unsigned FULLM = 0xffffffffu;
+    if (DSEED) seed = *reinterpret_cast<const unsigned long long*>(seed);
+    const int lane = threadIdx.x & 31;
+    const int b = blockIdx.x * SOLVE_WARPS + (threadIdx.x >> 5);
+    if (b >= N) return;  // warp-uniform
+    const int v = b / n_per_view;
+    const unsigned long long g = (unsigned long long)(sample_offset + (b - v * n_per_view));
+    uint32_t own[4];
+    tps_words4(seed, v, g, (uint32_t)(lane < TPS_DRAW_CALLS ? lane : 0), own);
+    uint32_t x[TPS_DRAW_WORDS];
+#pragma unroll
+    for (int w = 0; w < TPS_DRAW_WORDS; ++w) x[w] = __shfl_sync(FULLM, own[w & 3], w >> 2);
+    float c[16], vec[16], o[2], o2[2], ts[2], rot[4], tv[16];
+    tps_fields(sc, x, c, vec, o, o2, ts, rot);
+    tps_input_param(c, vec, o, o2, ts, rot, tv);
+    if (lane < 16) {
+        if (coord) coord[b * 16 + lane] = pick(c, lane);
+        if (vector) vector[b * 16 + lane] = pick(vec, lane);
+        t_vector[b * 16 + lane] = pick(tv, lane);
+    }
+    if (lane < 2) {
+        if (offset) offset[b * 2 + lane] = pick(o, lane);
+        if (offset_2) offset_2[b * 2 + lane] = pick(o2, lane);
+        if (t_scal) t_scal[b * 2 + lane] = pick(ts, lane);
+    }
+    if (lane < 4 && rot_mat) rot_mat[b * 4 + lane] = pick(rot, lane);
+    float qx[8], qy[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) { qx[i] = c[2 * i + 1]; qy[i] = c[2 * i]; }
+    tps_solve_warp(qx, qy, [&](int k) { return pick(tv, k); }, T, b, lane);
 }
 
 // K1 as its own kernel.  MINB = resident CTAs per SM asked of ptxas: besides capping registers, an explicit value
@@ -268,6 +328,43 @@ extern "C" int ups_tps_solve(const float* coord, const float* vector, float* T, 
     if (N == 0) return UPS_OK;
     tps_solve_kernel<<<(unsigned)cdiv(N, SOLVE_WARPS), SOLVE_WARPS * 32, 0, as_stream(stream)>>>(coord, vector, T, N);
     return after_launch("tps_solve_kernel");
+}
+
+template <bool DSEED>
+static int tps_draw_solve_launch(unsigned long long seed, long long sample_offset, int n_per_view, int n_views,
+                                 const TpsDrawScalars& sc, float* coord, float* vector, float* offset, float* offset_2,
+                                 float* t_scal, float* rot_mat, float* t_vector, float* T, void* stream) {
+    UPS_REQUIRE(t_vector && T, "tps_draw_solve: null pointer");
+    UPS_REQUIRE(n_per_view >= 0 && (n_views == 1 || n_views == 2) && sample_offset >= 0,
+                "tps_draw_solve: n_per_view=%d n_views=%d sample_offset=%lld", n_per_view, n_views, sample_offset);
+    UPS_REQUIRE((long long)n_per_view * n_views * 16 < (1ll << 31), "tps_draw_solve: n_per_view=%d too large", n_per_view);
+    UPS_REQUIRE(sc.rot_turn >= 0.0f && sc.rot_turn <= 0.5f, "tps_draw_solve: rot_turn=%g outside [0, 1/2]", (double)sc.rot_turn);
+    const int N = n_per_view * n_views;
+    if (N == 0) return UPS_OK;
+    tps_draw_solve_kernel<DSEED><<<(unsigned)cdiv(N, SOLVE_WARPS), SOLVE_WARPS * 32, 0, as_stream(stream)>>>(
+        seed, sample_offset, n_per_view, N, sc, coord, vector, offset, offset_2, t_scal, rot_mat, t_vector, T);
+    return after_launch("tps_draw_solve_kernel");
+}
+
+extern "C" int ups_tps_draw_solve(unsigned long long seed, long long sample_offset, int n_per_view, int n_views,
+                                  float coord_lo, float coord_w, float vec_lo, float vec_w, float off_lo, float off_w,
+                                  float scal_lo, float scal_w, float rescal, float rot_turn, float* coord, float* vector,
+                                  float* offset, float* offset_2, float* t_scal, float* rot_mat, float* t_vector, float* T,
+                                  void* stream) {
+    const TpsDrawScalars sc{coord_lo, coord_w, vec_lo, vec_w, off_lo, off_w, scal_lo, scal_w, rescal, rot_turn};
+    return tps_draw_solve_launch<false>(seed, sample_offset, n_per_view, n_views, sc, coord, vector, offset, offset_2,
+                                        t_scal, rot_mat, t_vector, T, stream);
+}
+
+extern "C" int ups_tps_draw_solve_dseed(const unsigned long long* seed, long long sample_offset, int n_per_view, int n_views,
+                                        float coord_lo, float coord_w, float vec_lo, float vec_w, float off_lo, float off_w,
+                                        float scal_lo, float scal_w, float rescal, float rot_turn, float* coord,
+                                        float* vector, float* offset, float* offset_2, float* t_scal, float* rot_mat,
+                                        float* t_vector, float* T, void* stream) {
+    UPS_REQUIRE(seed, "tps_draw_solve: null seed pointer");
+    const TpsDrawScalars sc{coord_lo, coord_w, vec_lo, vec_w, off_lo, off_w, scal_lo, scal_w, rescal, rot_turn};
+    return tps_draw_solve_launch<true>((unsigned long long)(uintptr_t)seed, sample_offset, n_per_view, n_views, sc, coord,
+                                       vector, offset, offset_2, t_scal, rot_mat, t_vector, T, stream);
 }
 
 static int check_warp_args(const void* U, const void* coord, const void* T, const void* move, const void* scal,

@@ -285,7 +285,7 @@ class DataParallelPartStep:
 
     def __init__(self, per_gpu_batch, spatial_size, n_parts, local_app_size=64, n_views=3, use_tps=True,
                  views_grad=False, n_grad_params=33_300_000, device="cuda", decode_bwd="auto", allreduce="auto",
-                 allreduce_ctas=0, seed=0, reducer=None, standin="auto", main_bucket="auto"):
+                 allreduce_ctas=0, seed=0, reducer=None, standin="auto", main_bucket="auto", tps_parameters=None):
         from .step import PartStep
         self.rank = dist.get_rank() if dist.is_initialized() else 0
         self.world = dist.get_world_size() if dist.is_initialized() else 1
@@ -307,7 +307,8 @@ class DataParallelPartStep:
         # rank r holds samples [r*B, (r+1)*B) of the global batch: with the same noise seed on every rank, the N ranks draw
         # exactly the logit noise that one GPU draws over the global batch (PartStep.forward(noise_seed=...))
         self.step = PartStep(per_gpu_batch, spatial_size, n_parts, local_app_size, n_views, use_tps, views_grad, device,
-                             decode_bwd=decode_bwd, sample_offset=self.rank * int(per_gpu_batch))
+                             decode_bwd=decode_bwd, sample_offset=self.rank * int(per_gpu_batch),
+                             tps_parameters=tps_parameters)
         dev = self.step.device
         K, F = self.step.K, self.step.F
         self.mod = StandInModules(K, F, dev, seed)
@@ -331,8 +332,10 @@ class DataParallelPartStep:
         self._ev = torch.cuda.Event()
 
     # ---------------------------------------------------------------- forward
-    def forward(self, views, coord, t_vector, l0, l1, feat, conv_V=None, conv_b=None, noise_seed=None, noise_level=1.0):
-        """PartStep.forward on this rank's shard; pass the same noise_seed on every rank."""
+    def forward(self, views, coord, t_vector, l0, l1, feat, conv_V=None, conv_b=None, noise_seed=None, noise_level=1.0,
+                tps_seed=None):
+        """PartStep.forward on this rank's shard; pass the same noise_seed (and tps_seed) on every rank: the N ranks
+        then draw the logit noise and the warp that one GPU draws over the global batch."""
         # the parameters (hence the averaged gradients of the previous step) are needed from the first kernel that consumes
         # logits or features; the 11x11 TPS solves in front of it depend on the batch's warp parameters only
         inner = self.step._inner if self.step.Kp else self.step
@@ -341,7 +344,7 @@ class DataParallelPartStep:
         else:
             self.reducer.wait()
         return self.step.forward(views, coord, t_vector, l0, l1, feat, conv_V, conv_b, noise_seed=noise_seed,
-                                 noise_level=noise_level)
+                                 noise_level=noise_level, tps_seed=tps_seed)
 
     def wait_grads(self):
         """The current stream waits until both buckets hold the mean over ranks (times 1/grad_scale for NCCL)."""

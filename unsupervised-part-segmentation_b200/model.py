@@ -97,9 +97,7 @@ def _noise_args(noise_seed):
     """noise_seed (None, an int in [0, 2**64) or a one-element int64 CUDA tensor) -> the ops' (noise, seed, seed_value)."""
     if noise_seed is None:
         return ops.NOISE_NONE, None, 0
-    if isinstance(noise_seed, torch.Tensor):
-        return ops.NOISE_DEVICE, noise_seed, 0
-    return ops.NOISE_INT, None, ops._seed_i64(noise_seed)
+    return _tps.seed_args(noise_seed)
 
 
 def decode_conv2d(logits, feature_vectors, V, b, noise_seed=None, noise_level=1.0, sample_offset=0):
@@ -197,19 +195,35 @@ def images_from_uint8(images):
     return ops.views_u8_to_f32(images)
 
 
-def make_tps(views, tps_parameters, generator=None):
+def make_tps(views, tps_parameters, generator=None, seed=None, sample_offset=0):
     """TrainModel.make_tps — cub/code/SB_model48i/model.py:282-311 (3 views; the target view
-    re-uses the first-half parameters) / pennaction/code/SB_model48i/model.py:281-303 (2 views)."""
+    re-uses the first-half parameters) / pennaction/code/SB_model48i/model.py:281-303 (2 views).
+
+    seed (an int in [0, 2**64), or a one-element int64 CUDA tensor): the warp parameters are drawn on the device
+    (tps.tps_parameters(..., seed=, views=2)): one ups::tps_draw call gives coord, t_vector and the solved system of
+    the 2B rows [view 0 | view 1] of global samples sample_offset .. + B - 1, with no host work and no host-to-device
+    copy, so the whole function can be captured in a CUDA graph with a tensor seed (an int seed raises during
+    capture).  seed=None draws on the host from `generator`, as before."""
     bs = views[0].shape[0]
     img_batch = torch.cat(list(views[:2]), dim=0)
     bs_doubled = img_batch.shape[0]
-    tps_param_dict = _tps.tps_parameters(bs_doubled, generator=generator, device=img_batch.device,
-                                         **tps_parameters)
-    coord, vector = _tps.make_input_tps_param(tps_param_dict)
-    t_images, t_mesh = _tps.ThinPlateSpline(img_batch, coord, vector, img_batch.shape[1], img_batch.shape[-1])
+    if seed is not None:
+        if generator is not None:
+            raise ValueError("make_tps: pass a seed (device draw) or a generator (host draw), not both")
+        out = _tps.draw(seed, bs, 2, sample_offset, img_batch.device, **tps_parameters)
+        coord, vector, T = out[0], out[6], out[7]
+        t_images, _ = ops.tps_warp(img_batch, coord, T, img_batch.shape[1], None, None)
+    else:
+        tps_param_dict = _tps.tps_parameters(bs_doubled, generator=generator, device=img_batch.device,
+                                             **tps_parameters)
+        coord, vector = _tps.make_input_tps_param(tps_param_dict)
+        t_images, t_mesh = _tps.ThinPlateSpline(img_batch, coord, vector, img_batch.shape[1], img_batch.shape[-1])
     augmented_views = list(torch.split(t_images, bs, dim=0))
     if len(views) > 2:
-        t_images, t_mesh = _tps.ThinPlateSpline(views[2], coord[:bs], vector[:bs], views[2].shape[1],
-                                                views[2].shape[-1])
+        if seed is not None:
+            t_images, _ = ops.tps_warp(views[2], coord[:bs], T[:bs], views[2].shape[1], None, None)
+        else:
+            t_images, t_mesh = _tps.ThinPlateSpline(views[2], coord[:bs], vector[:bs], views[2].shape[1],
+                                                    views[2].shape[-1])
         augmented_views.append(t_images)
     return augmented_views

@@ -867,17 +867,18 @@ draw_rect = _op("draw_rect", _draw_rect, lambda c, ph, pw, H, W: c.new_empty(c.s
 NOISE_NONE, NOISE_INT, NOISE_DEVICE = 0, 1, 2
 
 
-def _check_noise(noise: int, seed: Optional[Tensor], seed_value: int, noise_level: float, sample_offset: int, device):
+def _check_noise(noise: int, seed: Optional[Tensor], seed_value: int, noise_level: float, sample_offset: int, device,
+                 name="noise_seed", draws="noise", where="the logits' device"):
     """The noise arguments, checked, as the step launchers' noise value (step.py): None or (seed, sample_offset,
-    noise_level), the seed an int or the device tensor."""
+    noise_level), the seed an int or the device tensor.  name / draws / where word the errors for other seeded draws."""
     if noise == NOISE_INT and torch.cuda.is_current_stream_capturing():
-        raise C.UpsError("ups_b200: an int noise_seed is frozen into a captured CUDA graph (every replay would draw the "
-                         "same noise); pass the seed as a one-element int64 CUDA tensor")
+        raise C.UpsError(f"ups_b200: an int {name} is frozen into a captured CUDA graph (every replay would draw the "
+                         f"same {draws}); pass the seed as a one-element int64 CUDA tensor")
     if noise == NOISE_DEVICE:
         if seed is None or seed.dtype != torch.int64 or seed.numel() != 1 or seed.device != device:
-            raise C.UpsError("ups_b200: a device noise_seed is a one-element int64 tensor on the logits' device")
+            raise C.UpsError(f"ups_b200: a device {name} is a one-element int64 tensor on {where}")
         if not seed.is_contiguous():
-            raise C.UpsError("ups_b200: the device noise_seed must be contiguous")
+            raise C.UpsError(f"ups_b200: the device {name} must be contiguous")
     return None if noise == NOISE_NONE else (seed_value if noise == NOISE_INT else seed, sample_offset, noise_level)
 
 
@@ -1174,3 +1175,40 @@ def _encode_conv_bwd(ctx, g_m1, g_mask1, g_e0):
 
 
 encode_conv = _op("encode_conv", _encode_conv, _encode_conv_fake, _encode_conv_bwd, _encode_conv_setup)
+
+
+# ------------------------------------------------------------------ the TPS parameters drawn on the device
+# tps_parameters + make_input_tps_param + the solve in one launch (ups_tps_draw_solve, csrc/canon_math.cuh "the TPS
+# parameters"): the rows are [view 0 | view 1] (views = 2) of global samples sample_offset .. + n_per_view - 1, or view 0
+# alone (views = 1).  The seed follows the NOISE_INT / NOISE_DEVICE convention; `scalars` are the ten values of
+# tps.draw_scalars (rounded to fp32 by the call).  Returns (coord, vector, offset, offset_2, t_scal, rot_mat, t_vector,
+# T).  No gradient: the warp parameters are data (tps.ThinPlateSpline).
+def _tps_draw(noise: int, seed: Optional[Tensor], seed_value: int, sample_offset: int, n_per_view: int, views: int,
+              scalars: list[float], device: torch.device) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor, Tensor,
+                                                                   Tensor]:
+    if noise not in (NOISE_INT, NOISE_DEVICE):
+        raise C.UpsError("ups_b200: tps_draw needs a seed (NOISE_INT or NOISE_DEVICE)")
+    device = torch.device(device)
+    if device.type != "cuda":
+        raise C.UpsError("ups_b200: tps_draw needs a CUDA device (no CPU fallback exists)")
+    if device.index is None:
+        device = torch.device("cuda", torch.cuda.current_device())
+    nz = _check_noise(noise, seed, seed_value, 0.0, sample_offset, device, "tps seed", "warp", "the output device")
+    if sample_offset < 0 or n_per_view < 0 or views not in (1, 2) or len(scalars) != 10:
+        raise C.UpsError(f"ups_b200: tps_draw: sample_offset={sample_offset} n_per_view={n_per_view} views={views} "
+                         f"{len(scalars)} scalars")
+    out = _tps_draw_fake(noise, seed, seed_value, sample_offset, n_per_view, views, scalars, device)
+    s = nz[0]
+    C.call("ups_tps_draw_solve_dseed" if isinstance(s, Tensor) else "ups_tps_draw_solve",
+           s.data_ptr() if isinstance(s, Tensor) else s % 2 ** 64, sample_offset, n_per_view, views, *scalars,
+           *[t.data_ptr() for t in out], _stream(out[0]))
+    return out
+
+
+def _tps_draw_fake(noise, seed, seed_value, sample_offset, n_per_view, views, scalars, device):
+    N = n_per_view * views
+    shapes = ((N, 8, 2), (N, 8, 2), (N, 1, 2), (N, 1, 2), (N, 2), (N, 2, 2), (N, 8, 2), (N, 2, 11))
+    return tuple(torch.empty(sh, dtype=torch.float32, device=device) for sh in shapes)
+
+
+tps_draw = _op("tps_draw", _tps_draw, _tps_draw_fake)

@@ -199,7 +199,7 @@ def _on_device(fn):
 class PartStep:
     def __init__(self, batch_size, spatial_size, n_parts, local_app_size=64, n_views=3, use_tps=True,
                  views_grad=False, device="cuda", decode_bwd="auto", first_conv=0, encoder_conv=0, sample_offset=0,
-                 _planes=None):
+                 tps_parameters=None, _planes=None):
         B, S, K, F, V = int(batch_size), int(spatial_size), int(n_parts), int(local_app_size), int(n_views)
         # sample_offset: global index of this step's first sample in the noise draw (forward(noise_seed=...)): a rank of a
         # data-parallel run that holds samples [o, o + B) of the global batch draws exactly what one GPU draws for them
@@ -210,6 +210,11 @@ class PartStep:
         # _planes (internal): part planes that really exist when this step runs a padded part count (see below)
         self.Kpl = K if _planes is None else int(_planes)
         self.use_tps = bool(use_tps) and V >= 2
+        # tps_parameters: the ranges (tps.tps_parameters' keyword arguments) that forward(tps_seed=...) draws the warp from
+        from . import configs
+        from .tps import draw_scalars
+        self.tps_parameters = dict(configs.CUB_TPS if tps_parameters is None else tps_parameters)
+        self._tps_scalars = draw_scalars(**self.tps_parameters)
         self.views_grad = bool(views_grad)
         self.device = torch.device(device)
         if self.device.type != "cuda":
@@ -227,7 +232,8 @@ class PartStep:
         if self.route == "padded" and _planes is None:
             self.Kp = Kr
             self._inner = PartStep(B, S, self.Kp, F, n_views=V, use_tps=use_tps, views_grad=views_grad, device=self.device,
-                                   decode_bwd=decode_bwd, sample_offset=sample_offset, _planes=K)
+                                   decode_bwd=decode_bwd, sample_offset=sample_offset,
+                                   tps_parameters=self.tps_parameters, _planes=K)
             self._init_padded()
             return
         # K4 variant: "tc" = persistent TMA + tcgen05/TMEM pipeline, "simt" = CUDA-core kernel
@@ -239,6 +245,8 @@ class PartStep:
         f32 = dict(dtype=torch.float32, device=self.device)
         e = torch.empty
         self.T = e(2 * B, 2, 11, **f32)
+        # the warp parameters forward(tps_seed=...) draws (tps_drawn())
+        self._tps_coord, self._tps_tv = e(2 * B, 8, 2, **f32), e(2 * B, 8, 2, **f32)
         self.warped = e(max(V, 2), B, S, S, 3, **f32) if self.use_tps else None
         self.m0, self.m1 = e(B, S, S, K, **f32), e(B, S, S, K, **f32)
         self.labels0 = e(B, S, S, dtype=torch.int64, device=self.device)
@@ -297,6 +305,47 @@ class PartStep:
     def _stream(self):
         return torch.cuda.current_stream(self.device).cuda_stream
 
+    def _check_tps(self, coord, t_vector, tps_seed):
+        """forward's warp arguments: given coord and t_vector, or tps_seed alone."""
+        if tps_seed is None:
+            if self.use_tps and (coord is None or t_vector is None):
+                raise ValueError("PartStep.forward: pass coord and t_vector, or tps_seed to draw them on the device")
+            return
+        if coord is not None or t_vector is not None:
+            raise ValueError("PartStep.forward: pass coord and t_vector, or tps_seed, not both")
+        if not self.use_tps:
+            raise ValueError("PartStep.forward: tps_seed needs a step with use_tps")
+        if isinstance(tps_seed, torch.Tensor):
+            if tps_seed.dtype != torch.int64 or tps_seed.numel() != 1 or tps_seed.device != self.device \
+                    or not tps_seed.is_contiguous():
+                raise C.UpsError("PartStep: a device tps_seed is a contiguous one-element int64 tensor on the step's device")
+        else:
+            _seed_i64(tps_seed)
+            if torch.cuda.is_current_stream_capturing():
+                raise C.UpsError("PartStep: an int tps_seed is frozen into a captured CUDA graph (every replay would draw "
+                                 "the same warp); pass the seed as a one-element int64 CUDA tensor")
+
+    def _tps_solve(self, coord, t_vector, tps_seed, st):
+        """The 11x11 systems of the 2B warps into self.T: of the given coord / t_vector, or of the warp drawn from
+        tps_seed (view v of global sample sample_offset + b in row v * B + b) into the step's own buffers, in the same
+        one launch.  Returns the coord the warp uses."""
+        B = self.B
+        if tps_seed is None:
+            assert tuple(coord.shape) == (2 * B, 8, 2) and tuple(t_vector.shape) == (2 * B, 8, 2)
+            C.call("ups_tps_solve", coord.data_ptr(), t_vector.data_ptr(), self.T.data_ptr(), 2 * B, st)
+            return coord
+        C.call("ups_tps_draw_solve_dseed" if isinstance(tps_seed, torch.Tensor) else "ups_tps_draw_solve",
+               _seed_arg(tps_seed), self.sample_offset, B, 2, *self._tps_scalars, self._tps_coord.data_ptr(), None, None,
+               None, None, None, self._tps_tv.data_ptr(), self.T.data_ptr(), st)
+        return self._tps_coord
+
+    def tps_drawn(self):
+        """The warp the last forward(tps_seed=...) drew: dict(coord, t_vector) [2B,8,2], views of the step's buffers.
+        forward(views, coord, t_vector, ...) with copies of them computes the same bits."""
+        if self.Kp:
+            return self._inner.tps_drawn()
+        return dict(coord=self._tps_coord, t_vector=self._tps_tv)
+
     def _noise(self, noise_seed, noise_level):
         """The launchers' noise value of forward(noise_seed=, noise_level=): None, or (seed, sample_offset, noise_level)."""
         return None if noise_seed is None else (_seed_i64(noise_seed), self.sample_offset, float(noise_level))
@@ -349,7 +398,7 @@ class PartStep:
                buf.shape[-1] - n_cols, fill, st)
 
     @_on_device
-    def _forward_padded(self, views, coord, t_vector, l0, l1, feat, noise_seed=None, noise_level=1.0):
+    def _forward_padded(self, views, coord, t_vector, l0, l1, feat, noise_seed=None, noise_level=1.0, tps_seed=None):
         B, S, K, F, P, Kp = self.B, self.S, self.K, self.F, self.P, self.Kp
         st = self._stream()
         assert feat.is_contiguous()
@@ -361,7 +410,7 @@ class PartStep:
         # feat [B,K,F] -> [B,Kp,F]: per sample the first K*F floats of the padded block (the rest stays zero)
         C.call("ups_copy_rows", feat.data_ptr(), K * F, self._featp.data_ptr(), Kp * F, B, K * F, 0, 0.0, st)
         o = self._inner.forward(views, coord, t_vector, a0, a1, self._featp, rows=dict(l0=n0, l1=n1), noise_seed=noise_seed,
-                                noise_level=noise_level)
+                                noise_level=noise_level, tps_seed=tps_seed)
         self._feat, self._img1 = feat, self._inner._img1
         return dict(warped=o["warped"], m0=self.m0, m1=self.m1, labels0=self.labels0, parts=self.parts, pooled=self.pooled,
                     inj=self.inj)
@@ -389,7 +438,7 @@ class PartStep:
 
     # ------------------------------------------------------------------ forward
     def forward(self, views, coord, t_vector, l0, l1, feat, conv_V=None, conv_b=None, enc_V=None, enc_b=None, rows=None,
-                noise_seed=None, noise_level=1.0):
+                noise_seed=None, noise_level=1.0, tps_seed=None):
         """views [V,B,S,S,3] (view0, view1[, view0_target]), fp32 in [-1, 1] or the dataset's uint8
         (normalised on the device exactly as cub/code/data/data.py:134 does on the host); coord,
         t_vector [2B,8,2] from make_input_tps_param; l0, l1 [B,S,S,K]; feat [B,K,F].  Returns a dict
@@ -408,25 +457,32 @@ class PartStep:
         On the fused path K1 (TPS warp) and K3 (decode side) are independent and run as ONE launch with interleaved
         CTAs (ups_step_warp_decode_fwd): the warp's arithmetic hides under the decode side's memory stream.
         forward_warp / forward_parts are the same step as two calls (K1 | K2, K3) for callers that have the views
-        before the logits."""
+        before the logits.
+
+        tps_seed (an int in [0, 2**64), or a one-element int64 CUDA tensor read by the kernel, which a captured CUDA graph
+        needs; pass coord = t_vector = None): the warp parameters are drawn on the device instead, from the ranges of
+        the constructor's tps_parameters, as tps.tps_parameters(2B, seed=tps_seed, sample_offset=sample_offset, views=2)
+        draws them.  The draw runs in the launch that otherwise solves the given warp, so the step issues as many
+        launches as with given coord; tps_drawn() returns the drawn coord / t_vector."""
+        self._check_tps(coord, t_vector, tps_seed)
         if self.Kp:
-            return self._forward_padded(views, coord, t_vector, l0, l1, feat, noise_seed, noise_level)
+            return self._forward_padded(views, coord, t_vector, l0, l1, feat, noise_seed, noise_level, tps_seed)
         # rows (internal, padded part counts): row lengths of l0 / l1 when they are read in place ({"l0": 25, "l1": 25})
         if self.fuse_fwd:
-            return self._forward_fused(views, coord, t_vector, l0, l1, feat, rows, self._noise(noise_seed, noise_level))
-        self.forward_warp(views, coord, t_vector)
+            return self._forward_fused(views, coord, t_vector, l0, l1, feat, rows, self._noise(noise_seed, noise_level),
+                                       tps_seed)
+        self.forward_warp(views, coord, t_vector, tps_seed)
         return self.forward_parts(l0, l1, feat, conv_V, conv_b, enc_V, enc_b, rows, noise_seed, noise_level)
 
     @_on_device
-    def _forward_fused(self, views, coord, t_vector, l0, l1, feat, rows=None, nz=None):
+    def _forward_fused(self, views, coord, t_vector, l0, l1, feat, rows=None, nz=None, tps_seed=None):
         B, S, K, F, P, V = self.B, self.S, self.K, self.F, self.P, self.V
         st = self._stream()
         views = self._ingest(views, st)
         r0, r1 = (rows or {}).get("l0", K), (rows or {}).get("l1", K)
         assert l0.is_contiguous() and l1.is_contiguous() and feat.is_contiguous()
         assert tuple(l0.shape) == (B, S, S, r0) and tuple(l1.shape) == (B, S, S, r1) and tuple(feat.shape) == (B, K, F)
-        assert tuple(coord.shape) == (2 * B, 8, 2) and tuple(t_vector.shape) == (2 * B, 8, 2)
-        C.call("ups_tps_solve", coord.data_ptr(), t_vector.data_ptr(), self.T.data_ptr(), 2 * B, st)
+        coord = self._tps_solve(coord, t_vector, tps_seed, st)
         if self.before_params is not None:
             self.before_params()     # data-parallel wrapper: wait for the averaged gradients (the TPS solve needs none)
         call_rows("ups_step_warp_decode_fwd_rows", nz, views.data_ptr(), views[2].data_ptr() if V > 2 else None,
@@ -465,14 +521,14 @@ class PartStep:
         return views
 
     @_on_device
-    def forward_warp(self, views, coord, t_vector):
-        """K1: the TPS equivariance warp of the views (model.py:282-311).  Returns the warped views [V,B,S,S,3]."""
+    def forward_warp(self, views, coord, t_vector, tps_seed=None):
+        """K1: the TPS equivariance warp of the views (model.py:282-311).  Returns the warped views [V,B,S,S,3].
+        tps_seed: draw the warp on the device (see forward)."""
         B, S, V = self.B, self.S, self.V
         st = self._stream()
         views = self._ingest(views, st)
         if self.use_tps:
-            assert tuple(coord.shape) == (2 * B, 8, 2) and tuple(t_vector.shape) == (2 * B, 8, 2)
-            C.call("ups_tps_solve", coord.data_ptr(), t_vector.data_ptr(), self.T.data_ptr(), 2 * B, st)
+            coord = self._tps_solve(coord, t_vector, tps_seed, st)
             if V > 2:  # the target view shares view0's warp (model.py:306-309): one launch, shared grid
                 C.call("ups_tps_warp_pair_fwd", views.data_ptr(), views[2].data_ptr(), coord.data_ptr(),
                        self.T.data_ptr(), self.warped.data_ptr(), self.warped[2].data_ptr(), 2 * B, B, S, S, 3, S, S, st)
